@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload decode64k|compress128k]
                     [--corpus log|tick|random|mixed] [--chunk BYTES] [--level 1..3] [--bytes N] [--dictionary BYTES]
-                    [--no-extras] [--no-cpu-baseline]
+                    [--no-extras] [--no-cpu-baseline] [--dump-outputs DIR]
 
 One process per GPU (under torchrun for N > 1: RANK/LOCAL_RANK/WORLD_SIZE from the env).  Frames are independent,
 so ranks shard the work with no data-path collective ("scaling": "weak": every rank processes --bytes of its own
@@ -31,6 +31,13 @@ The other BASELINE.json configs are the same two workloads with other shapes: --
                 libzstd 1.5.5's own decoder beside it as `cpu_baseline_libzstd`; compress: libzstd 1.5.5 (the reference
                 has no compressor) — all host cores in every case
 `--impl reference` times that CPU baseline alone, rank 0 only, as the reference arm.
+
+--dump-outputs DIR writes what the device-resident arm returned to its caller in the last timed step (rank 0), so that two
+builds can be compared output for output on identical inputs (the corpus and libzstd's frames are deterministic):
+  result.npy     float64, the result code of every item (bytes written, or the error code)
+  dst.npy        float32, one row of dst_stride bytes per sampled item: its destination bytes, zero past its result
+  dst_items.npy  float64, the sampled items: np.random.default_rng(0).permutation(n)[:k] sorted, k = as many rows as fit
+                 in 32 MiB
 """
 import argparse
 import ctypes
@@ -44,6 +51,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True          # the tree may be read-only: no __pycache__ next to the imported modules
 
 CHUNK = {"decode64k": 65536, "compress128k": 131072}
 METRIC = {"decode64k": "decompress_GBps_uncompressed", "compress128k": "compress_GBps_uncompressed"}
@@ -64,7 +72,13 @@ def parse_args():
                     "(ZDICT) on the head of the corpus, decoded through zstdb200_load_dictionary (SURVEY 8f-3)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the compress block, the pageable / single-call / single-context measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as .npy files to DIR (see the docstring)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the GPU path (--impl ours)")
+    return args
 
 
 def recorded_traffic(workload_key, kernel):
@@ -286,9 +300,29 @@ class Gpu:
             self.dist.barrier()
 
 
-def measure(g, args, w, steps, warmup, sampler=None, extras=False):
+DUMP_ROW_BYTES = 32 << 20      # float32 rows of dst.npy; result.npy and dst_items.npy come on top (64 MB in all at most)
+
+
+def dump_outputs(out_dir, w, t_dst, t_res):
+    """--dump-outputs: result codes of every item and the destination bytes of a seeded sample of items (docstring)."""
+    import torch
+    n, stride = w["n"], w["dst_stride"]
+    res = t_res.cpu().numpy().view(np.uint32)
+    k = max(1, min(n, DUMP_ROW_BYTES // (4 * stride)))
+    items = np.sort(np.random.default_rng(0).permutation(n)[:k])
+    rows = t_dst[:n * stride].view(n, stride)[torch.from_numpy(items).to(t_dst.device)].cpu().numpy()
+    written = np.where(res[items] <= stride, res[items], 0)          # an error code writes nothing
+    rows[np.arange(stride)[None, :] >= written[:, None].astype(np.int64)] = 0
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "result.npy"), res.astype(np.float64))
+    np.save(os.path.join(out_dir, "dst.npy"), rows.astype(np.float32))
+    np.save(os.path.join(out_dir, "dst_items.npy"), items.astype(np.float64))
+
+
+def measure(g, args, w, steps, warmup, sampler=None, extras=False, dump=None):
     """One workload on this rank's GPU: device-resident pipeline (CUDA events, max over ranks), per-kernel times, and the
-    host-buffer C-ABI call from pinned memory.  extras: also pageable caller memory and the single-item call (decode)."""
+    host-buffer C-ABI call from pinned memory.  extras: also pageable caller memory and the single-item call (decode).
+    dump: a directory for the outputs of the last timed step (dump_outputs)."""
     torch, ctx, lib, dev = g.torch, g.ctx, g.lib, g.dev
     n, total, decode, level = w["n"], w["total"], w["kind"] == "decode64k", w["level"]
     src_bytes = int(w["src_off"][-1])
@@ -353,6 +387,8 @@ def measure(g, args, w, steps, warmup, sampler=None, extras=False):
     g.barrier()
     ms = g.max_over_ranks(ev0.elapsed_time(ev1))
     launches = ctx.kernel_launches - l0
+    if dump:
+        dump_outputs(dump, w, t_dst, t_res)
 
     # per-kernel device times (CUDA events between the kernels, separate synchronised runs)
     kms = {}
@@ -476,12 +512,15 @@ def main():
     g = Gpu(args)
     world = g.world
     w = prepare(args, g.rank)
+    if args.dump_outputs and 8 * w["n"] > (12 << 20):
+        raise SystemExit(f"--dump-outputs: the result codes of {w['n']} items do not fit the dump's 64 MB; use a larger --chunk")
     decode = w["kind"] == "decode64k"
     if w.get("dictionary"):
         g.ctx.load_dictionary(w["dictionary"])
         args.no_cpu_baseline = True          # the all-core oracle arm has no dictionary entry point
     sampler = ClockSampler(g.local)
-    m = measure(g, args, w, args.steps, args.warmup, sampler=sampler, extras=not args.no_extras)
+    m = measure(g, args, w, args.steps, args.warmup, sampler=sampler, extras=not args.no_extras,
+                dump=args.dump_outputs if g.rank == 0 else None)
     sampler.stop_flag = True      # clocks are sampled through both timed regions (device-resident and host-buffer)
     sampler.join()
     n, total, src_bytes, ms, kms = m["n"], m["total"], m["src_bytes"], m["ms"], m["kernel_ms"]
