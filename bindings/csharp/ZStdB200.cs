@@ -25,6 +25,8 @@ namespace EPAM.Deltix.ZStd
         [DllImport(Lib)] internal static extern UIntPtr zstdb200_compress_bound(UIntPtr srcSize);
         [DllImport(Lib)] internal static extern uint zstdb200_compress(IntPtr ctx, int level, int checksum, void* dst, uint dstCapacity, void* src, uint srcSize);
         [DllImport(Lib)] internal static extern int zstdb200_compress_batch(IntPtr ctx, int level, int checksum, void** src, uint* srcSize, void** dst, uint* dstCap, uint* result, UIntPtr n);
+        [DllImport(Lib)] internal static extern uint zstdb200_compress_using_dict(IntPtr ctx, int level, int checksum, void* dst, uint dstCapacity, void* src, uint srcSize);
+        [DllImport(Lib)] internal static extern int zstdb200_compress_batch_using_dict(IntPtr ctx, int level, int checksum, void** src, uint* srcSize, void** dst, uint* dstCap, uint* result, UIntPtr n);
         [DllImport(Lib)] internal static extern IntPtr zstdb200_host_alloc(UIntPtr bytes);
         [DllImport(Lib)] internal static extern void zstdb200_host_free(IntPtr p);
         [DllImport(Lib)] internal static extern IntPtr zstdb200_version();
@@ -134,6 +136,20 @@ namespace EPAM.Deltix.ZStd
             IntPtr c = Native.Ctx();
             int cs = checksum ? 1 : 0;
             Native.Batch(srcs, dsts, results, (sp, ss, dp, dc, r, n) => Native.zstdb200_compress_batch(c, level, cs, sp, ss, dp, dc, r, n));
+        }
+
+        // with the dictionary of this thread's context (ZStdDecompress.UseDictionary): frames name its id and decode with it.
+        // Without one the single-item call returns GENERIC and the batched call throws.
+        public static uint CompressUsingDict(byte[] dst, byte[] src, int level = 3, bool checksum = true)
+        {
+            fixed (byte* d = dst, s = src)
+                return Native.zstdb200_compress_using_dict(Native.Ctx(), level, checksum ? 1 : 0, d, (uint)dst.Length, s, (uint)src.Length);
+        }
+        public static void CompressUsingDict(IReadOnlyList<ArraySegment<byte>> srcs, IReadOnlyList<ArraySegment<byte>> dsts, uint[] results, int level = 3, bool checksum = true)
+        {
+            IntPtr c = Native.Ctx();
+            int cs = checksum ? 1 : 0;
+            Native.Batch(srcs, dsts, results, (sp, ss, dp, dc, r, n) => Native.zstdb200_compress_batch_using_dict(c, level, cs, sp, ss, dp, dc, r, n));
         }
     }
 

@@ -101,6 +101,21 @@ int zstdb200_compress_batch_device(zstdb200_ctx* ctx, int device_index, int leve
                                    void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap,
                                    uint32_t* result, size_t n, void* stream);
 
+/* The same three calls with the context's dictionary (the one zstdb200_load_dictionary loaded; same arguments and contracts as
+ * the call each mirrors).  Frames name the dictionary's id in their header (a raw-content dictionary has id 0 and none is
+ * written), match against its content and start from its repeat offsets; they decode with that dictionary
+ * (zstdb200_decompress*, libzstd's ZSTD_decompress_usingDict).  With no dictionary loaded the call fails at batch level
+ * (non-zero, or GENERIC for zstdb200_compress_using_dict; zstdb200_last_error says why); when the dictionary's entropy
+ * section is malformed every item gets dictionary_corrupted.  The calls without _using_dict ignore a loaded dictionary. */
+uint32_t zstdb200_compress_using_dict(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize);
+int zstdb200_compress_batch_using_dict(zstdb200_ctx* ctx, int level, int checksum,
+                                       const void* const* src, const uint32_t* srcSize,
+                                       void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n);
+int zstdb200_compress_batch_device_using_dict(zstdb200_ctx* ctx, int device_index, int level, int checksum,
+                                              const void* src_base, const uint64_t* src_off, const uint32_t* src_size,
+                                              void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap,
+                                              uint32_t* result, size_t n, void* stream);
+
 /* Pinned host memory for src/dst buffers (lets the batch calls DMA straight from/to caller memory). */
 void* zstdb200_host_alloc(size_t bytes);
 void zstdb200_host_free(void* p);

@@ -37,6 +37,11 @@ ABI = {
     "zstdb200_compress_batch": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _vpp, _u32p, _vpp, _u32p, _u32p, _c.c_size_t]),
     "zstdb200_compress_batch_device": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_void_p, _c.c_void_p,
                                                   _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p]),
+    "zstdb200_compress_using_dict": (_c.c_uint32, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p, _c.c_uint32, _c.c_void_p, _c.c_uint32]),
+    "zstdb200_compress_batch_using_dict": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _vpp, _u32p, _vpp, _u32p, _u32p, _c.c_size_t]),
+    "zstdb200_compress_batch_device_using_dict": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_void_p,
+                                                             _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p,
+                                                             _c.c_size_t, _c.c_void_p]),
     "zstdb200_host_alloc": (_c.c_void_p, [_c.c_size_t]),
     "zstdb200_host_free": (None, [_c.c_void_p]),
     "zstdb200_max_items": (_c.c_size_t, [_c.c_void_p]),
@@ -170,7 +175,7 @@ class Context:
 
     def load_dictionary(self, dictionary):
         """ZSTD_decompress_usingDict (ZStdDecompress.cs:2162-2167, :2366-2475): later decompress calls start every data frame
-        from this dictionary; None / b"" removes it."""
+        from this dictionary, and the *_using_dict compress calls compress against it; None / b"" removes it."""
         d = bytes(dictionary) if dictionary else b""
         rc = self._lib.zstdb200_load_dictionary(self._h, d if d else None, len(d))
         if rc != 0:
@@ -182,6 +187,10 @@ class Context:
 
     def compress_batch(self, srcs, dsts, level=3, checksum=True):
         return self._batch(self._lib.zstdb200_compress_batch, (int(level), 1 if checksum else 0), srcs, dsts)
+
+    def compress_batch_using_dict(self, srcs, dsts, level=3, checksum=True):
+        """compress_batch with the dictionary of load_dictionary (raises when none is loaded)."""
+        return self._batch(self._lib.zstdb200_compress_batch_using_dict, (int(level), 1 if checksum else 0), srcs, dsts)
 
     # ---- device-pointer batches (raw addresses, e.g. torch .data_ptr()) -----------------------
     def decompress_batch_device(self, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0, device_index=0):
@@ -211,6 +220,13 @@ class Context:
         if rc != 0:
             raise RuntimeError("zstdb200_compress_batch_device failed: " + self.last_error())
 
+    def compress_batch_device_using_dict(self, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n,
+                                         stream=0, device_index=0):
+        """compress_batch_device with the dictionary of load_dictionary (raises when none is loaded)."""
+        rc = self._lib.zstdb200_compress_batch_device_using_dict(self._h, device_index, int(level), 1 if checksum else 0, src_base, src_off,
+                                                                 src_size, dst_base, dst_off, dst_cap, result, n, stream)
+        if rc != 0:
+            raise RuntimeError("zstdb200_compress_batch_device_using_dict failed: " + self.last_error())
 
     def compress_batch_device_timed(self, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0,
                                     device_index=0):
@@ -333,3 +349,15 @@ class ZStdCompress:
     @staticmethod
     def CompressBatch(srcs, dsts, level=3, checksum=True, ctx=None):
         return (ctx or default_context()).compress_batch(srcs, dsts, level, checksum)
+
+    @staticmethod
+    def CompressUsingDict(dst, src, level=3, checksum=True, ctx=None):
+        """Compress with the dictionary loaded into the context (Context.load_dictionary); GENERIC when none is."""
+        dv, sv = _as_u8(dst, writable=True), _as_u8(src)
+        ctx = ctx or default_context()
+        return int(load_library().zstdb200_compress_using_dict(ctx.handle, int(level), 1 if checksum else 0, dv.ctypes.data if dv.size else None,
+                                                               dv.size, sv.ctypes.data if sv.size else None, sv.size))
+
+    @staticmethod
+    def CompressBatchUsingDict(srcs, dsts, level=3, checksum=True, ctx=None):
+        return (ctx or default_context()).compress_batch_using_dict(srcs, dsts, level, checksum)

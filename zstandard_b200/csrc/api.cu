@@ -15,6 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -22,6 +23,7 @@
 #include "../../include/zstdb200.h"
 #include "decode_kernels.cuh"
 #include "encode_kernels.cuh"
+#include "zb_encode.cuh"
 
 using namespace zb;
 
@@ -57,6 +59,7 @@ struct Device {
   BlockUnit* d_units = nullptr; u32* d_parList = nullptr; u32* d_cnt = nullptr;   // block-parallel path of multi-block frames (DecodeArgs::units / par_list / cnt, 2 counters per stream)
   u8* d_hufFull = nullptr; size_t hufFullBytes = 0;   // full Huffman tables of the resident frames (DecodeArgs::huf_full), one region per stream
   u8* d_dict = nullptr; size_t dictCap = 0; DictState* d_dictState = nullptr; bool dictOn = false;   // zstdb200_load_dictionary
+  u8* d_encDict = nullptr; size_t encDictCap = 0;   // the same dictionary prepared for the encoder (EncDict block, zb_encode.cuh)
   EncodeScratch enc;                            // encoder arenas (encode_kernels.cuh)
   // pinned host memory
   u8 *h_src = nullptr, *h_dst = nullptr;
@@ -72,6 +75,7 @@ struct zstdb200_ctx {
   size_t maxBatch = 0, maxItems = 0, srcCap = 0, dstSpan = 0;
   std::string err;
   uint64_t launches = 0;
+  std::vector<uint4> encDict;   // host copy of the encoder's dictionary block (enc_dict_prepare); empty: no dictionary loaded
 };
 
 namespace {
@@ -129,7 +133,7 @@ void free_device(Device& d) {
   cudaFree(d.d_src); cudaFree(d.d_dst); cudaFree(d.d_desc);
   cudaFree(d.d_info); cudaFree(d.d_lit); cudaFree(d.d_seq); cudaFree(d.d_more); cudaFreeHost(d.h_more);
   cudaFree(d.d_units); cudaFree(d.d_parList); cudaFree(d.d_cnt); cudaFree(d.d_hufFull);
-  cudaFree(d.d_dict); cudaFree(d.d_dictState);
+  cudaFree(d.d_dict); cudaFree(d.d_dictState); cudaFree(d.d_encDict);
   encode_free(d.enc);
   cudaFreeHost(d.h_src); cudaFreeHost(d.h_dst); cudaFreeHost(d.h_desc);
   for (auto& s : d.stream) if (s) cudaStreamDestroy(s);
@@ -238,7 +242,14 @@ struct Job {
   // scratch buffer must not reserve that much of the arenas (run_host_batch).  == dstCap unless clamped.
   const uint32_t* effCap;
   uint32_t maxSrc;     // largest srcSize of the call (compress: table sizes of the match stage)
+  bool useDict;        // compress with the context's dictionary (the *_using_dict calls)
 };
+
+// The encoder's dictionary on device d (zstdb200_load_dictionary put it on every device of the context)
+void set_dict(const zstdb200_ctx* ctx, const Device& d, EncodeArgs& a) {
+  const EncDict* h = reinterpret_cast<const EncDict*>(ctx->encDict.data());
+  a.dict = reinterpret_cast<const EncDict*>(d.d_encDict); a.dict_id = h->dictID; a.dict_err = h->err;
+}
 
 // One sub-batch [lo, hi) on one device: slices over NSTREAMS streams, direct DMA where the layout allows.
 // Returns "" or an error description.
@@ -341,6 +352,7 @@ std::string run_subbatch(zstdb200_ctx* ctx, Device& d, const Job& j, size_t lo, 
     } else {
       EncodeArgs ar{d.d_src, d_srcOff + a, d_srcSize + a, d.d_dst, d_dstOff + a, d_dstCap + a, d.d_result + a, (u32)cnt, (u32)a,
                     j.level, j.checksum, j.maxSrc, (u32)(s % nStreams)};
+      if (j.useDict) set_dict(ctx, d, ar);
       e = encode_launch(ar, d.enc, st, &nl);
     }
     *launches += nl;
@@ -483,7 +495,7 @@ int run_host_batch(zstdb200_ctx* ctx, const Job& j0, size_t n, bool clamp = true
     const size_t m = again.size();
     std::vector<const void*> s2(m); std::vector<void*> d2(m); std::vector<uint32_t> ss2(m), dc2(m), r2(m);
     for (size_t k = 0; k < m; k++) { const size_t i = again[k]; s2[k] = j.src[i]; d2[k] = j.dst[i]; ss2[k] = j.srcSize[i]; dc2[k] = j.dstCap[i]; }
-    Job jr{j.op, j.level, j.checksum, s2.data(), ss2.data(), d2.data(), dc2.data(), r2.data(), nullptr, j.maxSrc};
+    Job jr{j.op, j.level, j.checksum, s2.data(), ss2.data(), d2.data(), dc2.data(), r2.data(), nullptr, j.maxSrc, j.useDict};
     if (run_host_batch(ctx, jr, m, false)) return 1;
     for (size_t k = 0; k < m; k++) j.result[again[k]] = r2[k];
   }
@@ -558,6 +570,18 @@ uint64_t zstdb200_get_decompressed_size(const void* src, uint32_t srcSize) {
 int zstdb200_load_dictionary(zstdb200_ctx* ctx, const void* dict, uint32_t dictSize) {
   if (!ctx) return 1;
   ctx->err.clear();
+  // the encoder's preparation, once on the host (the same dict_load the decoder runs in k_dict, then enc_dict_prepare);
+  // every device gets a copy of the block
+  ctx->encDict.clear();
+  if (dict && dictSize) {
+    std::vector<u8> bytes((const u8*)dict, (const u8*)dict + dictSize); bytes.resize((size_t)dictSize + 64, 0);
+    std::unique_ptr<DictState> ds(new DictState());
+    HufBuildWk wk; HufFseScratch fs; u8 slot[260]; s16 norm[64]; u16 next[64];
+    dict_load(bytes.data(), dictSize, *ds, wk, fs, slot, norm, next);
+    ctx->encDict.assign((enc_dict_bytes(ds->err ? 0 : ds->contentSize) + 15) / 16, uint4{});
+    std::vector<u8> tableSymbol(512);
+    enc_dict_prepare(bytes.data(), dictSize, *ds, reinterpret_cast<EncDict*>(ctx->encDict.data()), wk, fs, slot, tableSymbol.data());
+  }
   for (auto& d : ctx->dev) {
     CK(cudaSetDevice(d.id));
     if (!dict || dictSize == 0) { d.dictOn = false; continue; }
@@ -568,6 +592,12 @@ int zstdb200_load_dictionary(zstdb200_ctx* ctx, const void* dict, uint32_t dictS
     if (!d.d_dictState) CK(cudaMalloc(&d.d_dictState, sizeof(DictState)));
     CK(cudaMemcpyAsync(d.d_dict, dict, dictSize, cudaMemcpyHostToDevice, d.stream[0]));
     CK(decode_load_dictionary(d.d_dict, dictSize, d.d_dictState, d.stream[0]));
+    const size_t encBytes = ctx->encDict.size() * sizeof(uint4);
+    if (encBytes > d.encDictCap) {
+      cudaFree(d.d_encDict); d.d_encDict = nullptr; d.encDictCap = 0;
+      CK(cudaMalloc(&d.d_encDict, encBytes)); d.encDictCap = encBytes;
+    }
+    CK(cudaMemcpyAsync(d.d_encDict, ctx->encDict.data(), encBytes, cudaMemcpyHostToDevice, d.stream[0]));
     CK(cudaStreamSynchronize(d.stream[0]));
     d.dictOn = true;
   }
@@ -578,7 +608,7 @@ int zstdb200_decompress_batch(zstdb200_ctx* ctx, const void* const* src, const u
                               void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n) {
   if (!ctx) return 1;
   ctx->err.clear();
-  Job j{Op::Decompress, 0, 0, src, srcSize, dst, dstCap, result, nullptr, 0};
+  Job j{Op::Decompress, 0, 0, src, srcSize, dst, dstCap, result, nullptr, 0, false};
   return run_host_batch(ctx, j, n);
 }
 
@@ -657,42 +687,72 @@ static int device_max_u32(zstdb200_ctx* ctx, Device& d, const uint32_t* d_vals, 
   return 0;
 }
 
-int zstdb200_compress_batch(zstdb200_ctx* ctx, int level, int checksum, const void* const* src, const uint32_t* srcSize,
-                            void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n) {
+// The compress entry points with and without the context's dictionary share these bodies (useDict).
+static int compress_batch(zstdb200_ctx* ctx, int level, int checksum, const void* const* src, const uint32_t* srcSize,
+                          void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n, bool useDict) {
   if (!ctx) return 1;
   ctx->err.clear();
   if (level < 1 || level > 3) { ctx->err = "level must be 1..3"; return 1; }
-  Job j{Op::Compress, level, checksum, src, srcSize, dst, dstCap, result, nullptr, 0};
+  if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
+  Job j{Op::Compress, level, checksum, src, srcSize, dst, dstCap, result, nullptr, 0, useDict};
   return run_host_batch(ctx, j, n);
 }
 
-uint32_t zstdb200_compress(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize) {
+static uint32_t compress_one(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize,
+                             bool useDict) {
   uint32_t r = zerr(ZE_GENERIC);
   const void* s = src; void* d = dst;
   static unsigned char dummy[16];
   if (!s) { s = dummy; srcSize = 0; }
   if (!d) { d = dummy; dstCapacity = 0; }
-  if (zstdb200_compress_batch(ctx, level, checksum, &s, &srcSize, &d, &dstCapacity, &r, 1)) return zerr(ZE_GENERIC);
+  if (compress_batch(ctx, level, checksum, &s, &srcSize, &d, &dstCapacity, &r, 1, useDict)) return zerr(ZE_GENERIC);
   return r;
 }
 
-int zstdb200_compress_batch_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
-                                   const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
-                                   const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream) {
+static int compress_batch_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
+                                 const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
+                                 const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream, bool useDict) {
   if (!ctx) return 1;
   ctx->err.clear();
   if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
   if (level < 1 || level > 3) { ctx->err = "level must be 1..3"; return 1; }
   if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
+  if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
   Device& d = ctx->dev[device_index];
   CK(cudaSetDevice(d.id));
   u32 maxSrc = 0;
   if (device_max_u32(ctx, d, src_size, n, stream ? (cudaStream_t)stream : d.stream[0], &maxSrc)) return 1;
   EncodeArgs a{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result, (u32)n, 0, level, checksum, maxSrc, ENC_EXCLUSIVE};
+  if (useDict) set_dict(ctx, d, a);
   int nl = 0;
   CK(encode_launch(a, d.enc, stream ? (cudaStream_t)stream : d.stream[0], &nl));
   ctx->launches += nl;
   return 0;
+}
+
+int zstdb200_compress_batch(zstdb200_ctx* ctx, int level, int checksum, const void* const* src, const uint32_t* srcSize,
+                            void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n) {
+  return compress_batch(ctx, level, checksum, src, srcSize, dst, dstCap, result, n, false);
+}
+int zstdb200_compress_batch_using_dict(zstdb200_ctx* ctx, int level, int checksum, const void* const* src, const uint32_t* srcSize,
+                                       void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n) {
+  return compress_batch(ctx, level, checksum, src, srcSize, dst, dstCap, result, n, true);
+}
+uint32_t zstdb200_compress(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize) {
+  return compress_one(ctx, level, checksum, dst, dstCapacity, src, srcSize, false);
+}
+uint32_t zstdb200_compress_using_dict(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize) {
+  return compress_one(ctx, level, checksum, dst, dstCapacity, src, srcSize, true);
+}
+int zstdb200_compress_batch_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
+                                   const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
+                                   const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream) {
+  return compress_batch_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, false);
+}
+int zstdb200_compress_batch_device_using_dict(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
+                                              const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
+                                              const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream) {
+  return compress_batch_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, true);
 }
 
 // zstdb200_compress_batch_device with CUDA events between its kernels (see zstdb200_decompress_batch_device_timed).

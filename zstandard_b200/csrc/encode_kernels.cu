@@ -1,6 +1,7 @@
 // encode_kernels.cu — sm_100a kernels of the batched zstd frame encoder.
 //
-//   k_enc_match<DFAST> : warp / block    match finder: 32 consecutive (or strided) positions per step, one per lane;
+//   k_enc_match<DFAST, DICT>             (DICT: also against the context's dictionary, see the kernel)
+//                      : warp / block    match finder: 32 consecutive (or strided) positions per step, one per lane;
 //                                        position hash table(s) of u16 entries in per-warp global scratch (L1 / L2
 //                                        resident; 32 one-warp CTAs per SM) or, for the concurrent slices of a host
 //                                        batch, in shared memory; in-window duplicate
@@ -52,12 +53,6 @@ __device__ __forceinline__ u32 ldu32(const u8* p) {
   const u32 a0 = w[0], a1 = sh ? w[1] : 0;
   return __funnelshift_r(a0, a1, sh);
 }
-__device__ __forceinline__ u32 hash64(u64 v, u32 hlog, u32 mls) {
-  if (mls >= 8) return (u32)((v * 0xCF1BBCDCB7A56463ull) >> (64 - hlog));
-  const u32 lo = (u32)v, hi = (u32)(v >> 32);                   // 5 / 6 bytes: two 32-bit multiplies do (ratio within 0.1 % of the 64-bit hash)
-  return (lo * 2654435761u + (hi & (mls == 6 ? 0xFFFFu : 0xFFu)) * 2246822519u) >> (32 - hlog);
-}
-
 // candidate position from a 16-bit table entry: the most recent position below p with those low 16 bits
 __device__ __forceinline__ bool cand_from_entry(u32 p, u32 e, u32& cand) {
   u32 d = (p - e) & 0xFFFF; if (d == 0) d = 0x10000;
@@ -76,11 +71,32 @@ __device__ __forceinline__ u32 warp_extend(const u8* src, u32 a, u32 off, u32 en
     return n + (u32)__ffs(~m) - 1;
   }
 }
+// the same against a second sequence: number of i >= a with src[i] == ref[i], a + n <= end
+__device__ __forceinline__ u32 warp_extend_ref(const u8* src, const u8* ref, u32 a, u32 end, u32 lane) {
+  u32 n = 0;
+  while (true) {
+    const u32 i = a + n + lane;
+    const bool eq = i < end && src[i] == ref[i];
+    const unsigned m = __ballot_sync(FULLMASK, eq);
+    if (m == FULLMASK) { n += 32; continue; }
+    return n + (u32)__ffs(~m) - 1;
+  }
+}
 
-template <bool DFAST>
+// DICT: the launch compresses with the context's dictionary (EncodeArgs::dict).  Its match tables are looked up by every
+// lane whose position found no match in the chunk's own tables, in libzstd's dictMatchState order: chunk long, dictionary
+// long, chunk short, dictionary short.  A dictionary match ends at the end of the content, its offset reaches back over
+// the chunk into the content, and the first block starts from the dictionary's repeat offsets.
+template <bool DFAST, bool DICT>
 __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc, u32 hlogL, u32 hlogS, u32 mls, u16* gtab) {
   extern __shared__ __align__(16) u16 tabShared[];
   const u32 lane = threadIdx.x, warp = blockIdx.x, nWarps = gridDim.x;
+  const EncDict* const ed = DICT ? a.dict : nullptr;
+  if (DICT && a.dict_err) return;                               // k_enc_entropy reports it for every item
+  const u32* const dtabL = DICT ? enc_dict_table(ed, DFAST ? EDT_LONG : (mls == 6 ? EDT_MLS6 : EDT_MLS5)) : nullptr;
+  const u32* const dtabS = DICT ? enc_dict_table(ed, EDT_MLS5) : nullptr;
+  const u8* const dc = DICT ? enc_dict_content(ed) : nullptr;
+  const u32 dsize = DICT ? ed->contentSize : 0;
   const u32 tw = (1u << hlogL) + (DFAST ? (1u << hlogS) : 0);
   // gtab != nullptr (launches that have the device to themselves): the tables of this warp live in global scratch,
   // kGtabStride bytes per warp, and the launch asks for no shared memory.  This kernel's throughput is its resident warp count (a serial chain per warp with a far
@@ -119,7 +135,7 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
         __syncwarp();
       }
     }
-    u32 rep1 = 1, rep2 = 4;
+    u32 rep1 = DICT ? ed->rep[0] : 1, rep2 = DICT ? ed->rep[1] : 4;   // the decoder starts every frame from the same two
     {
       const u32 bsize = size - bpos < BLOCKSIZE_MAX ? size - bpos : BLOCKSIZE_MAX;
       const u32 bend = bpos + bsize;
@@ -147,7 +163,8 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
           const u32 p = p0 + lane * step;
           const bool act = p < ilimit;
           u32 r2a = 0, r2b = 1;
-          if (fresh && rep2 != 0) { r2a = ldu32(src + p0); r2b = ldu32(src + p0 - rep2); }
+          if (fresh && rep2 != 0 && (!DICT || rep2 <= p0)) { r2a = ldu32(src + p0); r2b = ldu32(src + p0 - rep2); }   // (without a
+                                                                       //  dictionary rep2 is an offset seen in the chunk: always <= p0)
           const u64 v = act ? ldu64(src + p) : 0;
           const u32 hL = act ? hash64(v, hlogL, DFAST ? 8 : mls) : (0x80000000u | lane);
           const u32 eL = act ? tabL[hL] : 0;
@@ -166,6 +183,15 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
           bool okL = false, okS = false;
           if (validL) okL = DFAST ? (ldu64(src + candL) == v) : (ldu32(src + candL) == (u32)v);
           if (DFAST && validS) okS = ldu32(src + candS) == (u32)v;
+          u32 candDL = 0, candDS = 0; bool okDL = false, okDS = false;   // dictionary candidates (content positions)
+          if (DICT && act && !okL) {
+            candDL = dtabL[hash64(v, ENC_DICT_HLOG, DFAST ? 8 : mls)];
+            if (candDL != ENC_DICT_EMPTY) okDL = DFAST ? (ldu64(dc + candDL) == v) : (ldu32(dc + candDL) == (u32)v);
+          }
+          if (DICT && DFAST && act && !okL && !okDL && !okS) {
+            candDS = dtabS[hash64(v, ENC_DICT_HLOG, mls)];
+            if (candDS != ENC_DICT_EMPTY) okDS = ldu32(dc + candDS) == (u32)v;
+          }
           const bool rok = act && rep1 != 0 && rep1 <= p && ldu32(src + p - rep1) == (u32)v;
           if (fresh) {
             fresh = false;
@@ -186,7 +212,7 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
             }
           }
           const unsigned fRep = __ballot_sync(FULLMASK, rok);
-          const unsigned found = __ballot_sync(FULLMASK, okL | okS) | fRep;
+          const unsigned found = __ballot_sync(FULLMASK, okL | okS | okDL | okDS) | fRep;
           if (!found) {                                                // no match in the window: enter every position, move on
             if (act && (mL >> lane) == 1) tabL[hL] = (u16)p;          // the last position of each hash group is the one kept
             if (DFAST && act && (mS >> lane) == 1) tabS[hS] = (u16)p;
@@ -197,14 +223,28 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
           // a repeat-offset match up to 3 positions further on beats a table match here (it is cheaper to code)
           if (!((fRep >> fl) & 1)) { const unsigned nearRep = fRep & (0xEu << fl); if (nearRep) fl = (u32)__ffs(nearRep) - 1; }
           u32 pos = p0 + fl * step;
-          const u32 kind = rok ? 0 : (okL ? 1 : 2);                   // at the winning lane: repeat offset > long/main table > short table
+          // at the winning lane: repeat offset > long/main table > (dictionary long) > short table (> dictionary short)
+          const u32 kind = rok ? 0 : (okL ? 1 : (DICT ? (okDL ? 3 : (okS ? 2 : 4)) : 2));
           const u32 kf = __shfl_sync(FULLMASK, kind, fl);
-          const u32 cf = __shfl_sync(FULLMASK, kind == 1 ? candL : candS, fl);
+          const u32 cf = __shfl_sync(FULLMASK, DICT ? (kind == 1 ? candL : (kind == 3 ? candDL : (kind == 4 ? candDS : candS))) : (kind == 1 ? candL : candS), fl);
           u32 cnd = kf == 0 ? pos - rep1 : cf;
-          const u32 off = pos - cnd;
+          const u32 off = (DICT && kf >= 3) ? pos + (dsize - cnd) : pos - cnd;
           // forward extension and backward catch-up (:pos > anchor && cnd > 0 && equal) from one round of loads
           u32 mlen;
-          {
+          if (DICT && kf >= 3) {
+            // against the dictionary (cnd: content position): ref[i] is the byte src[i] is compared with; forward up to the
+            // end of the content, backward down to its start or the anchor
+            const u8* const ref = dc + cnd - pos;
+            const u32 fend = min(bend, pos + (dsize - cnd));
+            const u32 i = pos + 4 + lane; const bool feq = i < fend && src[i] == ref[i];
+            const u32 maxb = min(pos - anchor, cnd);
+            const bool beq = lane < maxb && src[pos - 1 - lane] == ref[pos - 1 - lane];
+            const unsigned fm = __ballot_sync(FULLMASK, feq), bm = __ballot_sync(FULLMASK, beq);
+            const u32 fwd = fm == FULLMASK ? 32 + warp_extend_ref(src, ref, pos + 36, fend, lane) : (u32)__ffs(~fm) - 1;
+            u32 bwd = bm == FULLMASK ? 32 : (u32)__ffs(~bm) - 1;
+            if (bm == FULLMASK) while (bwd < maxb && src[pos - 1 - bwd] == ref[pos - 1 - bwd]) bwd++;
+            mlen = 4 + fwd + bwd; pos -= bwd;
+          } else {
             const u32 i = pos + 4 + lane; const bool feq = i < bend && src[i] == src[i - off];
             const u32 maxb = min(pos - anchor, cnd);
             const bool beq = lane < maxb && src[pos - 1 - lane] == src[cnd - 1 - lane];
@@ -292,8 +332,8 @@ __device__ __forceinline__ u32 wmax(u32 v) {
   return v;
 }
 
-// literals section; returns bytes written, 0 = no room (mirror of enc_literals)
-__device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWarp& w, u8* tmp, u32 lane) {
+// literals section; returns bytes written, 0 = no room (mirror of enc_literals; ed likewise: the dictionary for the first block)
+__device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWarp& w, u8* tmp, u32 lane, const EncDict* ed) {
   const u32 rawLh = n < 32 ? 1 : (n < 4096 ? 2 : 3);
   auto raw = [&]() -> u32 {
     if (rawLh + n > cap) return 0;
@@ -361,10 +401,14 @@ __device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWar
   hdr = __shfl_sync(FULLMASK, hdr, 0);
   if (!hdr) return raw();
   __syncwarp();
-  u32 csize = hdr;
+  u32 tl = 0;
+  if (ed && lane == 0) tl = huf_dict_better(ed->huf, w.he, hdr, w.hist) ? 1 : 0;
+  const bool treeless = ed && __shfl_sync(FULLMASK, tl, 0);
+  const HufEnc& code = treeless ? ed->huf : w.he;             // the dictionary's code is read from global memory, through L1
+  u32 csize = treeless ? 0 : hdr;
   if (single) {
     u32 sz = 0;
-    if (lane == 0) sz = huf_encode_stream(body + csize, bodyCap - csize, lits, n, w.he);
+    if (lane == 0) sz = huf_encode_stream(body + csize, bodyCap - csize, lits, n, code);
     sz = __shfl_sync(FULLMASK, sz, 0);
     if (!sz) return raw();
     csize += sz;
@@ -372,7 +416,7 @@ __device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWar
     const u32 seg = (n + 3) / 4;
     if (csize + 6 > bodyCap) return raw();
     u32 sz = 0;
-    if (lane < 4) { const u32 from = lane * seg, len = lane < 3 ? seg : n - 3 * seg; sz = huf_encode_stream(tmp + (size_t)lane * kStreamTmp, kStreamTmp, lits + from, len, w.he); }
+    if (lane < 4) { const u32 from = lane * seg, len = lane < 3 ? seg : n - 3 * seg; sz = huf_encode_stream(tmp + (size_t)lane * kStreamTmp, kStreamTmp, lits + from, len, code); }
     const u32 s0 = __shfl_sync(FULLMASK, sz, 0), s1 = __shfl_sync(FULLMASK, sz, 1), s2 = __shfl_sync(FULLMASK, sz, 2), s3 = __shfl_sync(FULLMASK, sz, 3);
     if (!s0 || !s1 || !s2 || !s3 || s0 > 65535 || s1 > 65535 || s2 > 65535 || s3 > 65535) return raw();
     if (csize + 6 + s0 + s1 + s2 + s3 > bodyCap) return raw();
@@ -387,16 +431,19 @@ __device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWar
   const u32 minGain = (n >> 6) + 2;
   if (csize + minGain >= n) return raw();
   if (lane == 0) {
-    if (lhSize == 3) { const u32 v = 2 | ((single ? 0u : 1u) << 2) | (n << 4) | (csize << 14); out[0] = (u8)v; out[1] = (u8)(v >> 8); out[2] = (u8)(v >> 16); }
-    else if (lhSize == 4) { const u32 v = 2 | (2u << 2) | (n << 4) | (csize << 18); out[0] = (u8)v; out[1] = (u8)(v >> 8); out[2] = (u8)(v >> 16); out[3] = (u8)(v >> 24); }
-    else { const u32 v = 2 | (3u << 2) | (n << 4) | (csize << 22); out[0] = (u8)v; out[1] = (u8)(v >> 8); out[2] = (u8)(v >> 16); out[3] = (u8)(v >> 24); out[4] = (u8)(csize >> 10); }
+    const u32 lt = treeless ? 3 : 2;
+    if (lhSize == 3) { const u32 v = lt | ((single ? 0u : 1u) << 2) | (n << 4) | (csize << 14); out[0] = (u8)v; out[1] = (u8)(v >> 8); out[2] = (u8)(v >> 16); }
+    else if (lhSize == 4) { const u32 v = lt | (2u << 2) | (n << 4) | (csize << 18); out[0] = (u8)v; out[1] = (u8)(v >> 8); out[2] = (u8)(v >> 16); out[3] = (u8)(v >> 24); }
+    else { const u32 v = lt | (3u << 2) | (n << 4) | (csize << 22); out[0] = (u8)v; out[1] = (u8)(v >> 8); out[2] = (u8)(v >> 16); out[3] = (u8)(v >> 24); out[4] = (u8)(csize >> 10); }
   }
   __syncwarp();
   return lhSize + csize;
 }
 
-// sequences section; returns bytes written, 0 on failure (mirror of enc_sequences)
-__device__ u32 warp_enc_sequences(u8* out, u32 cap, const SeqStore& st, u8* codes, EntWarp& w, const EntLut& lut, int level, u32 lane) {
+// sequences section; returns bytes written, 0 on failure (mirror of enc_sequences; a repeat-mode table of the dictionary is
+// copied into w.ct with its state table left in global memory)
+__device__ u32 warp_enc_sequences(u8* out, u32 cap, const SeqStore& st, u8* codes, EntWarp& w, const EntLut& lut, int level, u32 lane,
+                                  const EncDict* ed) {
   const u32 nbSeq = st.n;
   if (cap < 4) return 0;
   u32 op = 0;
@@ -419,10 +466,10 @@ __device__ u32 warp_enc_sequences(u8* out, u32 cap, const SeqStore& st, u8* code
     u8* modeByte = out + o2++;
     const SeqKind kLL = seq_kind(KIND_LL), kOF = seq_kind(KIND_OF), kML = seq_kind(KIND_ML);
     u32 mLL = 0, mOF = 0, mML = 0;
-    mLL = enc_seq_table_counts(w.ct[0], w.state[0], w.sym, w.cnt[KIND_LL], llc[nbSeq - 1], nbSeq, kLL, level, out + o2, cap - o2, &used);
+    mLL = enc_seq_table_counts_dict(w.ct[0], w.state[0], w.sym, w.cnt[KIND_LL], llc[nbSeq - 1], nbSeq, kLL, level, out + o2, cap - o2, &used, ed, KIND_LL);
     if (mLL == 0xFF) good = false; else o2 += used;
-    if (good) { mOF = enc_seq_table_counts(w.ct[1], w.state[1], w.sym, w.cnt[KIND_OF], ofc[nbSeq - 1], nbSeq, kOF, level, out + o2, cap - o2, &used); if (mOF == 0xFF) good = false; else o2 += used; }
-    if (good) { mML = enc_seq_table_counts(w.ct[2], w.state[2], w.sym, w.cnt[KIND_ML], mlc[nbSeq - 1], nbSeq, kML, level, out + o2, cap - o2, &used); if (mML == 0xFF) good = false; else o2 += used; }
+    if (good) { mOF = enc_seq_table_counts_dict(w.ct[1], w.state[1], w.sym, w.cnt[KIND_OF], ofc[nbSeq - 1], nbSeq, kOF, level, out + o2, cap - o2, &used, ed, KIND_OF); if (mOF == 0xFF) good = false; else o2 += used; }
+    if (good) { mML = enc_seq_table_counts_dict(w.ct[2], w.state[2], w.sym, w.cnt[KIND_ML], mlc[nbSeq - 1], nbSeq, kML, level, out + o2, cap - o2, &used, ed, KIND_ML); if (mML == 0xFF) good = false; else o2 += used; }
     if (good) { *modeByte = (u8)((mLL << 6) | (mOF << 4) | (mML << 2)); o2w = o2; }
   }
   o2w = __shfl_sync(FULLMASK, o2w, 0);
@@ -526,6 +573,8 @@ __device__ u32 warp_enc_sequences(u8* out, u32 cap, const SeqStore& st, u8* code
   return total;
 }
 
+// DICT: frames name the dictionary (Dictionary_ID field) and a malformed one fails every item
+template <bool DICT>
 __global__ void __launch_bounds__(128) k_enc_entropy(EncodeArgs a, EncodeScratch sc, u32 slot0, u32 nwarps) {
   __shared__ EntWarp sm[4];
   __shared__ EntLut lut;
@@ -543,19 +592,13 @@ __global__ void __launch_bounds__(128) k_enc_entropy(EncodeArgs a, EncodeScratch
     u8* dst = a.dst_base + a.dst_off[f]; const u32 cap = a.dst_cap[f];
     u8* const lits0 = lit_base(a, sc, f); u32* const seqs0 = seq_base(a, sc, f); const BlockMeta* meta = meta_base(a, sc, f);
     // frame header (mirror of encode_frame_with)
-    const u32 fcsCode = size < 256 ? 0 : (size < 65536 + 256 ? 1 : 2);
-    const u32 fhs = 4 + 1 + (fcsCode == 0 ? 1 : (fcsCode == 1 ? 2 : 4));
+    const u32 fhs = enc_frame_header_size(size, DICT ? a.dict_id : 0);
     const u32 tail = a.checksum ? 4 : 0;
     u32 res = 0; bool failed = false;
     if (cap < fhs + 3 + tail) { failed = true; res = zerr(ZE_dstSize_tooSmall); }
+    if (DICT && a.dict_err) { failed = true; res = zerr(a.dict_err); }
     u32 op = fhs;
-    if (!failed && lane == 0) {
-      dst[0] = 0x28; dst[1] = 0xB5; dst[2] = 0x2F; dst[3] = 0xFD;
-      dst[4] = (u8)((fcsCode << 6) | (1u << 5) | (a.checksum ? 4 : 0));
-      if (fcsCode == 0) dst[5] = (u8)size;
-      else if (fcsCode == 1) { const u32 v = size - 256; dst[5] = (u8)v; dst[6] = (u8)(v >> 8); }
-      else { dst[5] = (u8)size; dst[6] = (u8)(size >> 8); dst[7] = (u8)(size >> 16); dst[8] = (u8)(size >> 24); }
-    }
+    if (!failed && lane == 0) enc_frame_header(dst, size, a.checksum, DICT ? a.dict_id : 0);
     u32 pos = 0, blk = 0;
     if (!failed) do {
       const u32 bsize = size - pos < BLOCKSIZE_MAX ? size - pos : BLOCKSIZE_MAX;
@@ -580,9 +623,10 @@ __global__ void __launch_bounds__(128) k_enc_entropy(EncodeArgs a, EncodeScratch
           const u32 avail = cap - op - 3 - tail;
           if (room > avail) room = avail;
           u8* body = dst + op + 3;
-          const u32 l = warp_enc_literals(body, room, st.lits, st.nlits, w, tmp, lane);
+          const EncDict* const edb = DICT && blk == 0 && a.dict->hasEntropy ? a.dict : nullptr;   // (as encode_frame_with)
+          const u32 l = warp_enc_literals(body, room, st.lits, st.nlits, w, tmp, lane, edb);
           if (l) {
-            const u32 sq = warp_enc_sequences(body + l, room - l, st, codes, w, lut, a.level, lane);
+            const u32 sq = warp_enc_sequences(body + l, room - l, st, codes, w, lut, a.level, lane, edb);
             if (sq && l + sq < bsize) { csize = l + sq; compressed = true; }
           }
         }
@@ -656,11 +700,13 @@ static cudaError_t encode_lazy_alloc(EncodeScratch& s) {
   cudaDeviceGetAttribute(&s.sms, cudaDevAttrMultiProcessorCount, dev);
   // as many entropy-stage warps as are resident at once: every warp then takes the same number of frames (+-1)
   int nb = 0;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_enc_entropy, 128, 0) != cudaSuccess || nb < 1) nb = 4;
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_enc_entropy<false>, 128, 0) != cudaSuccess || nb < 1) nb = 4;
   s.entWarps = (u32)(s.sms * nb * 4);
   if (s.entWarps > kSlotsExclusive) s.entWarps = kSlotsExclusive;
-  cudaFuncSetAttribute(k_enc_match<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-  cudaFuncSetAttribute(k_enc_match<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+  cudaFuncSetAttribute(k_enc_match<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(k_enc_match<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+  cudaFuncSetAttribute(k_enc_match<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(k_enc_match<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
   return cudaSuccess;
 }
 
@@ -700,13 +746,20 @@ cudaError_t encode_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st
     if (s.gtab) { gtab = (u16*)s.gtab; grid = (u32)s.sms * wps; if (grid > units) grid = (u32)units; }
   }
   if (marks) cudaEventRecord(marks[0], st);
-  if (dfast) k_enc_match<true><<<grid, 32, gtab ? 0 : smem, st>>>(a, s, hlogL, hlogS, mls, gtab);
-  else k_enc_match<false><<<grid, 32, gtab ? 0 : smem, st>>>(a, s, hlogL, hlogS, mls, gtab);
+  const size_t sm = gtab ? 0 : smem;
+  if (a.dict) {
+    if (dfast) k_enc_match<true, true><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    else k_enc_match<false, true><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+  } else {
+    if (dfast) k_enc_match<true, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    else k_enc_match<false, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+  }
   const u32 slot0 = exclusive ? 0 : (a.stream_slot % ENC_STREAM_PARTS) * kSlotsPerPart;
   const u32 maxSlots = exclusive ? s.entWarps : kSlotsPerPart;
   const u32 slots = a.n < maxSlots ? a.n : maxSlots;
   if (marks) cudaEventRecord(marks[1], st);
-  k_enc_entropy<<<(slots + 3) / 4, 128, 0, st>>>(a, s, slot0, slots);
+  if (a.dict) k_enc_entropy<true><<<(slots + 3) / 4, 128, 0, st>>>(a, s, slot0, slots);
+  else k_enc_entropy<false><<<(slots + 3) / 4, 128, 0, st>>>(a, s, slot0, slots);
   if (marks) cudaEventRecord(marks[2], st);
   if (launches) *launches += 2;
   if (a.checksum) { k_enc_xxh<<<(a.n * 4 + 127) / 128, 128, 0, st>>>(a); if (launches) *launches += 1; }

@@ -5,6 +5,8 @@
 
 namespace zb {
 
+struct EncDict;
+
 // All pointers are device pointers.  Item i: src_base[src_off[i] .. +src_size[i]) -> one zstd frame written at
 // dst_base[dst_off[i] ..] (at most dst_cap[i] bytes); result[i] = frame size or an error code.
 // src_off must be non-decreasing with src_off[i] + src_size[i] <= src_off[i+1] (the match stage's scratch is
@@ -21,6 +23,9 @@ struct EncodeArgs {
   u32 max_src_size;  // largest src_size of the whole call (selects the match stage's table sizes, zb_encode.cuh enc_hlog_*)
   u32 stream_slot;   // partition (0..ENC_STREAM_PARTS-1) of the entropy stage's slot pool for launches that run concurrently
                      // on different streams, or ENC_EXCLUSIVE when the launch has the context to itself
+  const EncDict* dict;   // the context's dictionary prepared for the encoder (zb_encode.cuh enc_dict_prepare), null: none
+  u32 dict_id, dict_err; // its dictID and err, copied by the host (the entropy stage reads them from the parameter bank: no
+                         // registers held across its frame loop)
 };
 
 // Per-device scratch owned by the context (allocated on the first compress call).

@@ -20,6 +20,34 @@ namespace zb {
 ZB_HD u64 rd64u(const u8* p) { return ld64(p); }
 ZB_HD u32 rd32u(const u8* p) { return ld32(p); }
 
+// position hash of the warp-parallel match finder (k_enc_match and its lock-step emulation in tests/hostsim) over the
+// 8 bytes at a position: mls 8 hashes all of them, mls 5 / 6 the first 5 / 6
+ZB_HD u32 hash64(u64 v, u32 hlog, u32 mls) {
+  if (mls >= 8) return (u32)((v * 0xCF1BBCDCB7A56463ull) >> (64 - hlog));
+  const u32 lo = (u32)v, hi = (u32)(v >> 32);                   // 5 / 6 bytes: two 32-bit multiplies do (ratio within 0.1 % of the 64-bit hash)
+  return (lo * 2654435761u + (hi & (mls == 6 ? 0xFFFFu : 0xFFu)) * 2246822519u) >> (32 - hlog);
+}
+
+// Frame header of the encoder (mirrored by k_enc_entropy): single segment, Dictionary_ID field of 1 / 2 / 4 bytes when the
+// id is not 0, content size of 1 / 2 / 4 bytes.  Returns its size; the caller has checked the room.
+ZB_HD u32 enc_frame_header_size(u32 size, u32 dictID) {
+  const u32 fcsCode = size < 256 ? 0 : (size < 65536 + 256 ? 1 : 2);
+  const u32 didBytes = dictID == 0 ? 0 : (dictID < 256 ? 1 : (dictID < 65536 ? 2 : 4));
+  return 4 + 1 + didBytes + (fcsCode == 0 ? 1 : (fcsCode == 1 ? 2 : 4));
+}
+ZB_HD u32 enc_frame_header(u8* dst, u32 size, int checksum, u32 dictID) {
+  const u32 fcsCode = size < 256 ? 0 : (size < 65536 + 256 ? 1 : 2);
+  const u32 didBytes = dictID == 0 ? 0 : (dictID < 256 ? 1 : (dictID < 65536 ? 2 : 4));
+  dst[0] = 0x28; dst[1] = 0xB5; dst[2] = 0x2F; dst[3] = 0xFD;
+  dst[4] = (u8)((fcsCode << 6) | (1u << 5) | (checksum ? 4 : 0) | (didBytes == 4 ? 3 : didBytes));
+  u32 p = 5;
+  for (u32 k = 0; k < didBytes; k++) dst[p++] = (u8)(dictID >> (8 * k));
+  if (fcsCode == 0) dst[p++] = (u8)size;
+  else if (fcsCode == 1) { const u32 v = size - 256; dst[p++] = (u8)v; dst[p++] = (u8)(v >> 8); }
+  else { dst[p++] = (u8)size; dst[p++] = (u8)(size >> 8); dst[p++] = (u8)(size >> 16); dst[p++] = (u8)(size >> 24); }
+  return p;
+}
+
 
 
 // ------------------------------------------------------------------------------------------------
@@ -237,6 +265,24 @@ ZB_HD u32 huf_sort_symbols(u16* order, const u32* count, u32 maxSym) {
   return n;
 }
 
+// Code lengths and canonical values from he.weight[0..maxSym] (0 = unused) of a code of table log tl, matching the decoder's
+// table fill: within a weight, symbols ascending; weights ascending start at rankStart (HufDecompress.cs:151-177):
+// code value = cell index >> (tableLog - nbBits)
+ZB_HD void huf_assign_codes(HufEnc& he, u32 maxSym, u32 tl) {
+  he.tableLog = tl; he.maxSym = maxSym;
+  u32 rankCount[16]; for (u32 i = 0; i < 16; i++) rankCount[i] = 0;
+  for (u32 s = 0; s <= maxSym; s++) rankCount[he.weight[s]]++;
+  u32 rankStart[16]; u32 nextStart = 0;
+  for (u32 wv = 1; wv <= tl; wv++) { rankStart[wv] = nextStart; nextStart += rankCount[wv] << (wv - 1); }
+  for (u32 s = 0; s <= maxSym; s++) {
+    const u32 wv = he.weight[s];
+    he.code[s].nbBits = wv ? (u8)(tl + 1 - wv) : 0;
+    if (!wv) continue;
+    he.code[s].val = (u16)(rankStart[wv] >> (wv - 1));
+    rankStart[wv] += 1u << (wv - 1);
+  }
+}
+
 // sc.order[0..n) holds the used symbols sorted as huf_sort_symbols does
 ZB_HD bool huf_build_sorted(HufEnc& he, const u32* count, u32 n, u32 maxBits, HufBuildScratch& sc) {
   if (n < 2) return false;
@@ -284,20 +330,10 @@ ZB_HD bool huf_build_sorted(HufEnc& he, const u32* count, u32 n, u32 maxBits, Hu
   u32 tl = 0; for (u32 i = 0; i < n; i++) if (depth[i] > tl) tl = depth[i];
   { u64 kraft = 0; for (u32 i = 0; i < n; i++) kraft += 1ull << (tl - depth[i]); if (kraft != (1ull << tl)) return false; }
   for (u32 s = 0; s < 256; s++) { he.code[s].nbBits = 0; he.code[s].val = 0; he.weight[s] = 0; }
-  for (u32 i = 0; i < n; i++) { he.code[order[i]].nbBits = depth[i]; he.weight[order[i]] = (u8)(tl + 1 - depth[i]); }
-  he.tableLog = tl; he.maxSym = order[0];
-  for (u32 i = 0; i < n; i++) if (order[i] > he.maxSym) he.maxSym = order[i];
-  // canonical values matching the decoder's table fill: within a weight, symbols ascending; weights ascending
-  // start at rankStart (HufDecompress.cs:151-177): code value = cell index >> (tableLog - nbBits)
-  u32 rankCount[16]; for (u32 i = 0; i < 16; i++) rankCount[i] = 0;
-  for (u32 s = 0; s <= he.maxSym; s++) rankCount[he.weight[s]]++;
-  u32 rankStart[16]; u32 nextStart = 0;
-  for (u32 wv = 1; wv <= tl; wv++) { rankStart[wv] = nextStart; nextStart += rankCount[wv] << (wv - 1); }
-  for (u32 s = 0; s <= he.maxSym; s++) {
-    const u32 wv = he.weight[s]; if (!wv) continue;
-    he.code[s].val = (u16)(rankStart[wv] >> (wv - 1));
-    rankStart[wv] += 1u << (wv - 1);
-  }
+  for (u32 i = 0; i < n; i++) he.weight[order[i]] = (u8)(tl + 1 - depth[i]);
+  u32 maxSym = order[0];
+  for (u32 i = 0; i < n; i++) if (order[i] > maxSym) maxSym = order[i];
+  huf_assign_codes(he, maxSym, tl);
   return true;
 }
 
@@ -427,5 +463,129 @@ ZB_HD SeqKind seq_kind(int kind) {
 
 
 
+
+// ------------------------------------------------------------------------------------------------
+// encoder-side dictionary (zstdb200_compress*_using_dict): prepared once per zstdb200_load_dictionary on the host,
+// copied to every device as one block  [EncDict][three match tables][content + 64 bytes of read slack]
+// ------------------------------------------------------------------------------------------------
+// Match tables of the dictionary content: 2^ENC_DICT_HLOG u32 content positions each, ENC_DICT_EMPTY where no position
+// hashes.  One table per hash the match stage uses: mls 6 (level 1), mls 5 (level 2, and level 3's short table), the
+// 8-byte long hash (level 3).  They are read-only and shared by every warp, so they can be larger than the per-warp
+// chunk tables, but larger is not better: in a ratio sweep of the lock-step emulation (256 x 4 KiB log messages, 32 KiB
+// trained dictionary, profiles/dict_match_table_sweep.jsonl) 2^12 .. 2^16 entries give 4.715 / 4.695 / 4.685 / 4.678 / 4.675
+// at level 1 and 4.523 .. 4.463 at level 2 (a greedy parse takes the first hit: fewer, more recent dictionary positions
+// leave more to the cheaper in-chunk matches); level 3 is flat (4.686 .. 4.679).  2^12 is also the smallest (48 KB).
+#define ENC_DICT_HLOG 12
+static constexpr u32 ENC_DICT_EMPTY = 0xFFFFFFFFu;
+enum { EDT_MLS6 = 0, EDT_MLS5 = 1, EDT_LONG = 2 };
+struct alignas(16) EncDict {
+  u32 err;               // ZE_dictionary_corrupted when the entropy section is malformed: every item fails with it
+  u32 dictID;            // written into the frame header when not 0 (a raw-content dictionary has id 0)
+  u32 contentSize;       // bytes of content the match tables index (0 when err)
+  u32 rep[3];            // the repeat offsets a frame starts from (1, 4, 8 for a raw-content dictionary)
+  u32 hasEntropy;        // the tables below are the dictionary's (magic 0xEC30A437): what a frame's first block may reuse
+  u32 pad;
+  // Huffman encoding table from the dictionary's weights (the canonical codes huf_fill_table decodes), and the three FSE
+  // compression tables from its normalized counts (KIND_LL, KIND_OF, KIND_ML; seqCt[k].stateTable is set where it is used:
+  // seqState[k] at the address the reader sees)
+  HufEnc huf;
+  FseCTable seqCt[3];
+  s16 seqNorm[3][64];
+  u32 seqMaxSV[3], pad2;
+  u16 seqState[3][512];
+};
+ZB_HD size_t enc_dict_bytes(u32 contentSize) { return sizeof(EncDict) + 3 * ((size_t)4 << ENC_DICT_HLOG) + contentSize + 64; }
+ZB_HD const u32* enc_dict_table(const EncDict* d, int which) { return reinterpret_cast<const u32*>(d + 1) + ((size_t)which << ENC_DICT_HLOG); }
+ZB_HD const u8* enc_dict_content(const EncDict* d) { return reinterpret_cast<const u8*>(d + 1) + 3 * ((size_t)4 << ENC_DICT_HLOG); }
+
+// Fills the block at `out` (enc_dict_bytes(ds.err ? 0 : ds.contentSize) bytes) from the dictionary bytes (size of them, readable
+// 64 bytes further) and what dict_load parsed of them (the decoder's preparation: id, content range, repeat offsets, validity of
+// the entropy section).  An entropy dictionary's Huffman weights and normalized counts are read again (huf_read_weights,
+// read_ncount: dict_load keeps only the decode tables) and turned into encoding tables.  Every content position whose 8 bytes
+// lie inside the content is entered into the match tables in ascending order: the last one of a hash wins.
+// Scratch: tableSymbol 512 bytes, slot 256 bytes.
+ZB_HD void enc_dict_prepare(const u8* dict, u32 size, const DictState& ds, EncDict* out, HufBuildWk& wk, HufFseScratch& fs, u8* slot, u8* tableSymbol) {
+  out->err = ds.err; out->dictID = ds.dictID; out->contentSize = ds.err ? 0 : ds.contentSize;
+  for (int i = 0; i < 3; i++) out->rep[i] = ds.rep[i];
+  out->hasEntropy = !ds.err && ds.hasEntropy; out->pad = 0; out->pad2 = 0;
+  for (u32 s = 0; s < 256; s++) { out->huf.code[s].val = 0; out->huf.code[s].nbBits = 0; out->huf.weight[s] = 0; }
+  out->huf.maxSym = 0; out->huf.tableLog = 0;
+  for (int k = 0; k < 3; k++) {
+    out->seqCt[k] = FseCTable(); out->seqMaxSV[k] = 0;
+    for (u32 s = 0; s < 64; s++) out->seqNorm[k][s] = 0;
+    for (u32 i = 0; i < 512; i++) out->seqState[k][i] = 0;
+  }
+  if (out->hasEntropy) {
+    u32 p = 8, hdr = 0, tl = 0, nbSym = 0;
+    huf_read_weights(dict + p, size - p, wk, fs, slot, &hdr, &tl, &nbSym);      // accepted by dict_load: cannot fail here
+    for (u32 s = 0; s < nbSym; s++) out->huf.weight[s] = wk.weight[s];
+    huf_assign_codes(out->huf, nbSym - 1, tl);
+    p += hdr;
+    const int order[3] = {KIND_OF, KIND_ML, KIND_LL};
+    for (int o = 0; o < 3; o++) {
+      const int kind = order[o];
+      u32 maxSV = kind == KIND_LL ? MaxLL : (kind == KIND_ML ? MaxML : MaxOff), stl = 0, h = 0;
+      read_ncount(out->seqNorm[kind], &maxSV, &stl, dict + p, size - p, &h);
+      fse_build_ctable(out->seqCt[kind], out->seqState[kind], out->seqNorm[kind], maxSV, stl, tableSymbol);
+      out->seqCt[kind].stateTable = nullptr;
+      out->seqMaxSV[kind] = maxSV; p += h;
+    }
+  }
+  u32* const t = const_cast<u32*>(enc_dict_table(out, 0));
+  for (u32 i = 0; i < 3u << ENC_DICT_HLOG; i++) t[i] = ENC_DICT_EMPTY;
+  u8* const content = const_cast<u8*>(enc_dict_content(out));
+  const u32 n = out->contentSize;
+  for (u32 i = 0; i < n; i++) content[i] = dict[ds.contentOff + i];
+  for (u32 i = 0; i < 64; i++) content[n + i] = 0;
+  u32* const t6 = t + ((u32)EDT_MLS6 << ENC_DICT_HLOG); u32* const t5 = t + ((u32)EDT_MLS5 << ENC_DICT_HLOG); u32* const tl = t + ((u32)EDT_LONG << ENC_DICT_HLOG);
+  for (u32 q = 0; q + 8 <= n; q++) {
+    const u64 v = ld64(content + q);
+    t6[hash64(v, ENC_DICT_HLOG, 6)] = q; t5[hash64(v, ENC_DICT_HLOG, 5)] = q; tl[hash64(v, ENC_DICT_HLOG, 8)] = q;
+  }
+}
+
+// Estimated cost in 1/256 bits of coding count[s] symbols s <= maxSym with the FSE table ct (libzstd's ZSTD_fseBitCost per
+// symbol, from the table's deltaNbBits; an RLE table costs nothing).
+ZB_HD u64 fse_cost256(const FseCTable& ct, const u32* count, u32 maxSym) {
+  if (ct.tableLog == 0) return 0;
+  const u32 tableSize = 1u << ct.tableLog;
+  u64 bits = 0;
+  for (u32 s = 0; s <= maxSym; s++) {
+    if (!count[s]) continue;
+    const u32 d = ct.deltaNbBits[s], minNb = d >> 16, threshold = (minNb + 1) << 16;
+    bits += (u64)count[s] * (((minNb + 1) << 8) - (((threshold - (d + tableSize)) << 8) >> ct.tableLog));
+  }
+  return bits;
+}
+
+// enc_seq_table_counts, and for the first block of a frame with an entropy dictionary (ed != null) repeat mode (3) with the
+// dictionary's table when every code present has a non-zero probability there (and is at most its maxSV) and its estimated
+// bits are fewer than those of the mode chosen without it (its table description included).  count[] as for
+// enc_seq_table_counts.
+ZB_HD u32 enc_seq_table_counts_dict(FseCTable& ct, u16* stateTable, u8* symScratch, u32* count, u32 lastCode, u32 nbSeq, const SeqKind& k,
+                                    int level, u8* out, u32 cap, u32* used, const EncDict* ed, int kind) {
+  const u32 cLast = count[lastCode];
+  const u32 m = enc_seq_table_counts(ct, stateTable, symScratch, count, lastCode, nbSeq, k, level, out, cap, used);
+  if (!ed || m == 0xFF) return m;
+  count[lastCode] = cLast;
+  u32 maxSym = k.maxSym; while (maxSym > 0 && !count[maxSym]) maxSym--;
+  if (maxSym > ed->seqMaxSV[kind]) return m;
+  for (u32 s = 0; s <= maxSym; s++) if (count[s] && ed->seqNorm[kind][s] == 0) return m;
+  if (fse_cost256(ed->seqCt[kind], count, maxSym) >= fse_cost256(ct, count, maxSym) + ((u64)*used << 11)) return m;
+  ct = ed->seqCt[kind]; ct.stateTable = const_cast<u16*>(ed->seqState[kind]); *used = 0;
+  return 3;
+}
+
+// Treeless literals (type 3) with the dictionary's Huffman code for the first block of a frame: when every literal present has
+// a code there and the estimated stream bits are fewer than those of the fresh code `he` plus its header of hdrBytes.
+ZB_HD bool huf_dict_better(const HufEnc& dictHuf, const HufEnc& he, u32 hdrBytes, const u32* count) {
+  u64 dictBits = 0, freshBits = (u64)hdrBytes * 8;
+  for (u32 s = 0; s < 256; s++) {
+    if (!count[s]) continue;
+    if (!dictHuf.code[s].nbBits) return false;
+    dictBits += (u64)count[s] * dictHuf.code[s].nbBits; freshBits += (u64)count[s] * he.code[s].nbBits;
+  }
+  return dictBits < freshBits;
+}
 
 }  // namespace zb
