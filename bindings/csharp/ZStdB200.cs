@@ -30,6 +30,7 @@ namespace EPAM.Deltix.ZStd
         [DllImport(Lib)] internal static extern IntPtr zstdb200_host_alloc(UIntPtr bytes);
         [DllImport(Lib)] internal static extern void zstdb200_host_free(IntPtr p);
         [DllImport(Lib)] internal static extern IntPtr zstdb200_version();
+        [DllImport(Lib)] internal static extern uint zstdb200_train_dictionary(IntPtr ctx, void* dictBuffer, uint dictCapacity, void* samples, uint* sampleSizes, UIntPtr nbSamples, TrainParams* parameters);
 
         // one context per thread: a zstdb200_ctx is single-caller (include/zstdb200.h)
         [ThreadStatic] static IntPtr ctx;
@@ -150,6 +151,53 @@ namespace EPAM.Deltix.ZStd
             IntPtr c = Native.Ctx();
             int cs = checksum ? 1 : 0;
             Native.Batch(srcs, dsts, results, (sp, ss, dp, dc, r, n) => Native.zstdb200_compress_batch_using_dict(c, level, cs, sp, ss, dp, dc, r, n));
+        }
+    }
+
+    // zstdb200_train_params (include/zstdb200.h); zero fields take the library's defaults
+    [StructLayout(LayoutKind.Sequential)]
+    public struct TrainParams
+    {
+        public uint K;             // 0 = search {50, 537, 1024, 1511, 1998}
+        public uint D;             // 6 or 8; 0 = 8
+        public uint F;             // 0 = 20; at most 24
+        public uint Accel;         // 1..10; 0 = 1
+        public uint SplitPercent;  // 0 = 75 when searching, 100 with a fixed k
+        public int Level;          // 1..3; 0 = 3
+        public uint DictId;        // 0 = derived from the content
+    }
+
+    public static unsafe class ZStdDictionary
+    {
+        // new: builds a dictionary (magic 0xEC30A437) from sample messages on this thread's context's GPU, as libzstd's fastCover
+        // trainer selects content.  Returns its bytes; parameters (optional) receives the k and d chosen.  Throws on an error
+        // result, with its code in the message.
+        public static byte[] TrainDictionary(IReadOnlyList<ArraySegment<byte>> samples, int capacity, ref TrainParams parameters)
+        {
+            int n = samples.Count;
+            long total = 0;
+            for (int i = 0; i < n; i++) total += samples[i].Count;
+            var blob = new byte[Math.Max(total, 1)];
+            var sizes = new uint[Math.Max(n, 1)];
+            long pos = 0;
+            for (int i = 0; i < n; i++)
+            {
+                if (samples[i].Count > 0) Buffer.BlockCopy(samples[i].Array, samples[i].Offset, blob, (int)pos, samples[i].Count);
+                sizes[i] = (uint)samples[i].Count; pos += samples[i].Count;
+            }
+            var dict = new byte[capacity];
+            uint r;
+            fixed (byte* d = dict, s = blob) fixed (uint* z = sizes) fixed (TrainParams* p = &parameters)
+                r = Native.zstdb200_train_dictionary(Native.Ctx(), d, (uint)capacity, s, z, (UIntPtr)n, p);
+            if (Native.zstdb200_is_error(r) != 0)
+                throw new InvalidOperationException("zstdb200_train_dictionary failed: error " + (uint)(-(int)r) + " " + Marshal.PtrToStringAnsi(Native.zstdb200_last_error(Native.Ctx())));
+            Array.Resize(ref dict, (int)r);
+            return dict;
+        }
+        public static byte[] TrainDictionary(IReadOnlyList<ArraySegment<byte>> samples, int capacity)
+        {
+            var p = new TrainParams();
+            return TrainDictionary(samples, capacity, ref p);
         }
     }
 

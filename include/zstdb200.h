@@ -116,6 +116,30 @@ int zstdb200_compress_batch_device_using_dict(zstdb200_ctx* ctx, int device_inde
                                               void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap,
                                               uint32_t* result, size_t n, void* stream);
 
+/* Dictionary training (no reference counterpart: users of the reference train with libzstd's ZDICT_trainFromBuffer).  Builds
+ * a dictionary with entropy tables (magic 0xEC30A437) from nbSamples samples laid back to back in host memory, as ZDICT takes
+ * them.  The content is selected as libzstd 1.5.5's fastCover trainer selects it (ZDICT_trainFromBuffer_fastCover with a
+ * fixed k; with k = 0 the k search of ZDICT_trainFromBuffer, candidates scored by compressing the test share of the samples
+ * with this library's dictionary encoder at `level`); the entropy tables come from this library's match stage over the first
+ * block of the finalize samples.  Runs on the context's first device, allocates what the sample set needs and frees it before
+ * returning; the context's loaded dictionary is not touched.  Returns the dictionary size or an error code:
+ * dstSize_tooSmall (capacity below 256 or below k; 1998 when searching), srcSize_wrong (fewer than 5 training samples, no
+ * test sample when searching, fewer bytes than max(d, 8)), GENERIC with zstdb200_last_error set (a parameter out of range,
+ * samples totalling 2^32 bytes or more, a test sample larger than max_batch_bytes, a CUDA failure). */
+typedef struct {
+  uint32_t k;             /* segment size; 0 = search k over ZDICT_trainFromBuffer's grid {50, 537, 1024, 1511, 1998}; at most 2048 */
+  uint32_t d;             /* d-mer size, 6 or 8; 0 = 8 */
+  uint32_t f;             /* log2 of the frequency table; 0 = 20; at most 24 */
+  uint32_t accel;         /* 1..10, ZDICT's fastCover acceleration; 0 = 1 */
+  uint32_t split_percent; /* training share of the samples; 0 = 75 when searching, 100 with a fixed k (ZDICT's defaults) */
+  int      level;         /* 1..3: level whose match stage gathers the entropy statistics and scores search candidates; 0 = 3 */
+  uint32_t dict_id;       /* 0 = ZDICT's rule (XXH64 of the selected content, mod 2^31 - 32768, + 32768) */
+} zstdb200_train_params;
+
+uint32_t zstdb200_train_dictionary(zstdb200_ctx* ctx, void* dictBuffer, uint32_t dictCapacity,
+                                   const void* samples, const uint32_t* sampleSizes, size_t nbSamples,
+                                   zstdb200_train_params* params /* NULL = defaults; k and d chosen are written back */);
+
 /* Pinned host memory for src/dst buffers (lets the batch calls DMA straight from/to caller memory). */
 void* zstdb200_host_alloc(size_t bytes);
 void zstdb200_host_free(void* p);

@@ -56,7 +56,22 @@ ABI = {
                                                         _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p,
                                                         _c.POINTER(_c.c_float), _c.c_int]),
     "zstdb200_encode_kernel_name": (_c.c_char_p, [_c.c_int]),
+    "zstdb200_train_dictionary": (_c.c_uint32, [_c.c_void_p, _c.c_void_p, _c.c_uint32, _c.c_void_p, _u32p, _c.c_size_t, _c.c_void_p]),
 }
+
+
+class TrainParams(_c.Structure):
+    """zstdb200_train_params (include/zstdb200.h); zero fields take the library's defaults."""
+    _fields_ = [("k", _c.c_uint32), ("d", _c.c_uint32), ("f", _c.c_uint32), ("accel", _c.c_uint32), ("split_percent", _c.c_uint32),
+                ("level", _c.c_int), ("dict_id", _c.c_uint32)]
+
+
+class TrainError(RuntimeError):
+    """zstdb200_train_dictionary returned an error code (.code, in the library's encoding)."""
+
+    def __init__(self, code, message):
+        super().__init__(message)
+        self.code = code
 
 _lib = None
 
@@ -180,6 +195,23 @@ class Context:
         rc = self._lib.zstdb200_load_dictionary(self._h, d if d else None, len(d))
         if rc != 0:
             raise RuntimeError("zstdb200_load_dictionary failed: " + self.last_error())
+
+    def train_dictionary(self, samples, capacity, **params):
+        """Builds a dictionary of at most `capacity` bytes from the sample messages (a list of bytes-like objects) on the
+        context's first device; params are the fields of zstdb200_train_params (k, d, f, accel, split_percent, level, dict_id).
+        Returns the dictionary bytes; the k and d used are in self.last_train_params.  Raises TrainError on an error result."""
+        p = TrainParams(**{k: int(v) for k, v in params.items()})
+        views = [_as_u8(s) for s in samples]
+        blob = np.concatenate(views) if views else np.zeros(0, dtype=np.uint8)
+        blob = np.ascontiguousarray(blob, dtype=np.uint8)
+        sizes = np.array([v.size for v in views], dtype=np.uint32)
+        out = np.zeros(max(int(capacity), 1), dtype=np.uint8)
+        r = int(self._lib.zstdb200_train_dictionary(self._h, out.ctypes.data, int(capacity), blob.ctypes.data if blob.size else None,
+                                                    sizes.ctypes.data_as(_u32p), len(views), _c.byref(p)))
+        if is_error(r):
+            raise TrainError(r, f"zstdb200_train_dictionary failed: {error_name(r)} {self.last_error()}".rstrip())
+        self.last_train_params = p
+        return out[:r].tobytes()
 
     def decompress_batch(self, srcs, dsts):
         """Decodes srcs[i] into the writable buffer dsts[i]; returns np.uint32 result codes (reference convention)."""
@@ -361,3 +393,8 @@ class ZStdCompress:
     @staticmethod
     def CompressBatchUsingDict(srcs, dsts, level=3, checksum=True, ctx=None):
         return (ctx or default_context()).compress_batch_using_dict(srcs, dsts, level, checksum)
+
+
+def train_dictionary(samples, capacity, ctx=None, **params):
+    """Context.train_dictionary on `ctx` (default: the module's context)."""
+    return (ctx or default_context()).train_dictionary(samples, capacity, **params)

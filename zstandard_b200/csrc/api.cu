@@ -22,6 +22,7 @@
 
 #include "../../include/zstdb200.h"
 #include "decode_kernels.cuh"
+#include "dict_train.cuh"
 #include "encode_kernels.cuh"
 #include "zb_encode.cuh"
 
@@ -780,6 +781,23 @@ int zstdb200_compress_batch_device_timed(zstdb200_ctx* ctx, int device_index, in
   return 0;
 }
 const char* zstdb200_encode_kernel_name(int k) { return (k >= 0 && k < ENCODE_KERNELS) ? kEncodeKernelNames[k] : ""; }
+
+uint32_t zstdb200_train_dictionary(zstdb200_ctx* ctx, void* dictBuffer, uint32_t dictCapacity, const void* samples,
+                                   const uint32_t* sampleSizes, size_t nbSamples, zstdb200_train_params* params) {
+  if (!ctx) return zerr(ZE_GENERIC);
+  ctx->err.clear();
+  if (!dictBuffer || (nbSamples && !sampleSizes)) { ctx->err = "null argument"; return zerr(ZE_GENERIC); }
+  if (nbSamples > 0xFFFFFFFFull) { ctx->err = "too many samples"; return zerr(ZE_GENERIC); }
+  zstdb200_train_params p{};
+  if (params) p = *params;
+  Device& d = ctx->dev[0];
+  if (cudaSetDevice(d.id) != cudaSuccess) { ctx->err = "cudaSetDevice failed"; return zerr(ZE_GENERIC); }
+  DtDevice dv{d.stream[0], &d.enc, d.d_dst, ctx->srcCap, d.d_result, d.h_result, d.d_desc, d.h_desc, ctx->maxBatch, ctx->maxItems, 0};
+  const u32 r = dt_train_run(dv, (u8*)dictBuffer, dictCapacity, (const u8*)samples, sampleSizes, nbSamples, p, ctx->err);
+  ctx->launches += dv.launches;
+  if (!is_err(r) && params) { params->k = p.k; params->d = p.d; }
+  return r;
+}
 
 void* zstdb200_host_alloc(size_t bytes) { void* p = nullptr; return cudaMallocHost(&p, bytes ? bytes : 1) == cudaSuccess ? p : nullptr; }
 void zstdb200_host_free(void* p) { if (p) cudaFreeHost(p); }

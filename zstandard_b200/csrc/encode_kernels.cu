@@ -712,10 +712,8 @@ static cudaError_t encode_lazy_alloc(EncodeScratch& s) {
 
 const char* const kEncodeKernelNames[ENCODE_KERNELS] = {"k_enc_match", "k_enc_entropy", "k_enc_xxh"};
 
-cudaError_t encode_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, int* launches, cudaEvent_t* marks) {
-  if (a.n == 0) return cudaSuccess;
-  cudaError_t e = encode_lazy_alloc(s);
-  if (e != cudaSuccess) return e;
+// The match stage of one launch (k_enc_match): table sizes, grid and table placement.  marks: as for encode_launch.
+static void match_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, cudaEvent_t* marks) {
   // match stage: table sizes per level (u16 entries)
   const bool dfast = a.level >= 3;
   static const int envLog = getenv("ZSTDB200_ENC_HLOG") ? atoi(getenv("ZSTDB200_ENC_HLOG")) : 0;       // tuning aids
@@ -754,6 +752,14 @@ cudaError_t encode_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st
     if (dfast) k_enc_match<true, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
     else k_enc_match<false, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
   }
+}
+
+cudaError_t encode_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, int* launches, cudaEvent_t* marks) {
+  if (a.n == 0) return cudaSuccess;
+  cudaError_t e = encode_lazy_alloc(s);
+  if (e != cudaSuccess) return e;
+  match_launch(a, s, st, marks);
+  const bool exclusive = a.stream_slot == ENC_EXCLUSIVE;
   const u32 slot0 = exclusive ? 0 : (a.stream_slot % ENC_STREAM_PARTS) * kSlotsPerPart;
   const u32 maxSlots = exclusive ? s.entWarps : kSlotsPerPart;
   const u32 slots = a.n < maxSlots ? a.n : maxSlots;
@@ -764,6 +770,41 @@ cudaError_t encode_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st
   if (launches) *launches += 2;
   if (a.checksum) { k_enc_xxh<<<(a.n * 4 + 127) / 128, 128, 0, st>>>(a); if (launches) *launches += 1; }
   if (marks) cudaEventRecord(marks[3], st);
+  return cudaGetLastError();
+}
+
+// ---- statistics of the match stage (dictionary training, zb_dict_train.cuh) ----------------------------------------------
+// One warp per item, first block only: its literal bytes and the LL / ML / OF codes of its sequences, counted in shared memory
+// and added to st[0..DT_STAT_WORDS) (lit[256], ll[36], ml[53], of[32]: the layout of DtStats).
+__global__ void __launch_bounds__(256) k_enc_stats(EncodeArgs a, EncodeScratch sc, u32* st) {
+  __shared__ u32 h[DT_STAT_WORDS];
+  for (u32 i = threadIdx.x; i < DT_STAT_WORDS; i += blockDim.x) h[i] = 0;
+  __syncthreads();
+  u32* const hl = h; u32* const hll = h + 256; u32* const hml = hll + MaxLL + 1; u32* const hof = hml + MaxML + 1;
+  const u32 lane = threadIdx.x & 31, nw = gridDim.x * (blockDim.x >> 5);
+  for (u32 f = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); f < a.n; f += nw) {
+    const BlockMeta m = meta_base(a, sc, f)[0];
+    const u8* lits = lit_base(a, sc, f);
+    for (u32 i = lane; i < m.nlits; i += 32) atomicAdd(&hl[lits[i]], 1u);
+    SeqStore q; q.seqs = seq_base(a, sc, f); q.n = m.nseq; q.cap = kBlockSeqCap; q.lits = nullptr; q.nlits = 0;
+    for (u32 i = lane; i < m.nseq; i += 32) {
+      u32 ll, ob, mlm3; seq_get(q, i, ll, ob, mlm3);
+      atomicAdd(&hll[ll_code(ll)], 1u); atomicAdd(&hml[ml_code(mlm3)], 1u); atomicAdd(&hof[highbit(ob)], 1u);
+    }
+  }
+  __syncthreads();
+  for (u32 i = threadIdx.x; i < DT_STAT_WORDS; i += blockDim.x) if (h[i]) atomicAdd(&st[i], h[i]);
+}
+
+cudaError_t encode_match_stats(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, u32* stats, int* launches) {
+  if (a.n == 0) return cudaSuccess;
+  if (a.max_src_size > BLOCKSIZE_MAX || !a.dict) return cudaErrorInvalidValue;
+  cudaError_t e = encode_lazy_alloc(s);
+  if (e != cudaSuccess) return e;
+  match_launch(a, s, st, nullptr);
+  u32 grid = (a.n + 7) / 8; if (grid > (u32)s.sms * 8) grid = (u32)s.sms * 8;
+  k_enc_stats<<<grid, 256, 0, st>>>(a, s, stats);
+  if (launches) *launches += 2;
   return cudaGetLastError();
 }
 

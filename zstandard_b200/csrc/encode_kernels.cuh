@@ -47,5 +47,9 @@ void encode_free(EncodeScratch& s);
 #define ENCODE_KERNELS 3
 extern const char* const kEncodeKernelNames[ENCODE_KERNELS];
 cudaError_t encode_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, int* launches, cudaEvent_t* marks = nullptr);
+// Dictionary training: the match stage alone over items of at most one block (a.max_src_size <= 128 KiB) against a.dict, then
+// the histograms of its literals and sequence codes added to stats[0..DT_STAT_WORDS) (zb_dict_train.cuh DtStats)
+#define DT_STAT_WORDS (256 + 36 + 53 + 32)
+cudaError_t encode_match_stats(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, u32* stats, int* launches);
 
 }  // namespace zb
