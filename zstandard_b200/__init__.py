@@ -173,6 +173,17 @@ class Context:
     def last_error(self):
         return self._lib.zstdb200_last_error(self._h).decode()
 
+    def _check(self, name, rc):
+        if rc != 0:
+            raise RuntimeError(name + " failed: " + self.last_error())
+
+    def _timed(self, name, kernel_name, *args):
+        """Runs the *_timed entry point `name` -> {kernel name: ms}."""
+        ms = (_c.c_float * 8)()
+        self._check(name, getattr(self._lib, name)(self._h, *args, ms, 8))
+        names = [kernel_name(k).decode() for k in range(8)]
+        return {n: ms[k] for k, n in enumerate(names) if n}
+
     # ---- host-pointer batches -------------------------------------------------------------------
     def _batch(self, fn, pre, srcs, dsts):
         n = len(srcs)
@@ -192,9 +203,7 @@ class Context:
         """ZSTD_decompress_usingDict (ZStdDecompress.cs:2162-2167, :2366-2475): later decompress calls start every data frame
         from this dictionary, and the *_using_dict compress calls compress against it; None / b"" removes it."""
         d = bytes(dictionary) if dictionary else b""
-        rc = self._lib.zstdb200_load_dictionary(self._h, d if d else None, len(d))
-        if rc != 0:
-            raise RuntimeError("zstdb200_load_dictionary failed: " + self.last_error())
+        self._check("zstdb200_load_dictionary", self._lib.zstdb200_load_dictionary(self._h, d if d else None, len(d)))
 
     def train_dictionary(self, samples, capacity, **params):
         """Builds a dictionary of at most `capacity` bytes from the sample messages (a list of bytes-like objects) on the
@@ -226,54 +235,30 @@ class Context:
 
     # ---- device-pointer batches (raw addresses, e.g. torch .data_ptr()) -----------------------
     def decompress_batch_device(self, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0, device_index=0):
-        rc = self._lib.zstdb200_decompress_batch_device(self._h, device_index, src_base, src_off, src_size, dst_base, dst_off, dst_cap,
-                                                        result, n, stream)
-        if rc != 0:
-            raise RuntimeError("zstdb200_decompress_batch_device failed: " + self.last_error())
+        self._check("zstdb200_decompress_batch_device", self._lib.zstdb200_decompress_batch_device(
+            self._h, device_index, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream))
 
     def decompress_batch_device_timed(self, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0, device_index=0):
         """-> {kernel name: ms} for one synchronised run of the device pipeline."""
-        ms = (_c.c_float * 8)()
-        rc = self._lib.zstdb200_decompress_batch_device_timed(self._h, device_index, src_base, src_off, src_size, dst_base, dst_off,
-                                                              dst_cap, result, n, stream, ms, 8)
-        if rc != 0:
-            raise RuntimeError("zstdb200_decompress_batch_device_timed failed: " + self.last_error())
-        out = {}
-        for k in range(8):
-            name = self._lib.zstdb200_decode_kernel_name(k).decode()
-            if name:
-                out[name] = ms[k]
-        return out
+        return self._timed("zstdb200_decompress_batch_device_timed", self._lib.zstdb200_decode_kernel_name, device_index, src_base,
+                           src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream)
 
     def compress_batch_device(self, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0,
                               device_index=0):
-        rc = self._lib.zstdb200_compress_batch_device(self._h, device_index, int(level), 1 if checksum else 0, src_base, src_off, src_size,
-                                                      dst_base, dst_off, dst_cap, result, n, stream)
-        if rc != 0:
-            raise RuntimeError("zstdb200_compress_batch_device failed: " + self.last_error())
+        self._check("zstdb200_compress_batch_device", self._lib.zstdb200_compress_batch_device(
+            self._h, device_index, int(level), 1 if checksum else 0, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream))
 
     def compress_batch_device_using_dict(self, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n,
                                          stream=0, device_index=0):
         """compress_batch_device with the dictionary of load_dictionary (raises when none is loaded)."""
-        rc = self._lib.zstdb200_compress_batch_device_using_dict(self._h, device_index, int(level), 1 if checksum else 0, src_base, src_off,
-                                                                 src_size, dst_base, dst_off, dst_cap, result, n, stream)
-        if rc != 0:
-            raise RuntimeError("zstdb200_compress_batch_device_using_dict failed: " + self.last_error())
+        self._check("zstdb200_compress_batch_device_using_dict", self._lib.zstdb200_compress_batch_device_using_dict(
+            self._h, device_index, int(level), 1 if checksum else 0, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream))
 
     def compress_batch_device_timed(self, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0,
                                     device_index=0):
         """-> {kernel name: ms} for one synchronised run of the device pipeline."""
-        ms = (_c.c_float * 8)()
-        rc = self._lib.zstdb200_compress_batch_device_timed(self._h, device_index, int(level), 1 if checksum else 0, src_base, src_off,
-                                                            src_size, dst_base, dst_off, dst_cap, result, n, stream, ms, 8)
-        if rc != 0:
-            raise RuntimeError("zstdb200_compress_batch_device_timed failed: " + self.last_error())
-        out = {}
-        for k in range(8):
-            name = self._lib.zstdb200_encode_kernel_name(k).decode()
-            if name:
-                out[name] = ms[k]
-        return out
+        return self._timed("zstdb200_compress_batch_device_timed", self._lib.zstdb200_encode_kernel_name, device_index, int(level),
+                           1 if checksum else 0, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream)
 
 
 _default_ctx = None

@@ -15,7 +15,6 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
-#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -24,6 +23,7 @@
 #include "decode_kernels.cuh"
 #include "dict_train.cuh"
 #include "encode_kernels.cuh"
+#include "host_plan.h"
 #include "zb_encode.cuh"
 
 using namespace zb;
@@ -32,9 +32,6 @@ namespace {
 
 constexpr int NSTREAMS = 8;
 static_assert(NSTREAMS <= ENC_STREAM_PARTS, "one encoder slot partition per stream");
-constexpr size_t SLICE_BYTES_DEFAULT = 32u << 20;   // uncompressed bytes per slice (several slices per stream per GiB)
-constexpr size_t MIN_SLICE_ITEMS_DECODE = 1024;      // and at least this many frames (decode kernels: one frame-time per launch)
-constexpr size_t MIN_SLICE_ITEMS_ENCODE = 512;       // the match kernel fills the GPU with 2-4 thousand frames: start early
 
 // tuning aids (not part of the ABI): ZSTDB200_STREAMS = streams actually used (1..NSTREAMS), ZSTDB200_SLICE_MB
 int env_int(const char* name, int dflt, int lo, int hi) {
@@ -65,7 +62,6 @@ struct Device {
   // pinned host memory
   u8 *h_src = nullptr, *h_dst = nullptr;
   u8* h_desc = nullptr;
-  u64 *h_srcOff = nullptr, *h_dstOff = nullptr; u32 *h_srcSize = nullptr, *h_dstCap = nullptr;   // views into h_desc for the current sub-batch
   u32 *h_result = nullptr, *h_more = nullptr;
 };
 
@@ -86,18 +82,19 @@ template <int N> struct EventSet {
   cudaEvent_t ev[N] = {};
   ~EventSet() { for (auto e : ev) if (e) cudaEventDestroy(e); }
   cudaError_t create() { for (auto& e : ev) { cudaError_t r = cudaEventCreate(&e); if (r != cudaSuccess) return r; } return cudaSuccess; }
+  // waits for the last event, then ms[k] = time from event k to event k + 1 (at most max of them)
+  cudaError_t read(float* ms, int max) {
+    cudaError_t e = cudaEventSynchronize(ev[N - 1]);
+    for (int k = 0; e == cudaSuccess && k < N - 1 && k < max; k++) e = cudaEventElapsedTime(&ms[k], ev[k], ev[k + 1]);
+    return e;
+  }
 };
 
-#define CK(call)                                                                                   \
-  do {                                                                                             \
-    cudaError_t e_ = (call);                                                                       \
-    if (e_ != cudaSuccess) {                                                                       \
-      char b_[512]; snprintf(b_, sizeof b_, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_), __FILE__, __LINE__); \
-      ctx->err = b_; return 1;                                                                     \
-    }                                                                                              \
-  } while (0)
-
-size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+// CUDA errors of the entry points (ctx->err, return 1) and of the steps of a sub-batch (returned as text)
+#define CK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { char b_[512]; snprintf(b_, sizeof b_, "%s failed: %s (%s:%d)", \
+                      #call, cudaGetErrorString(e_), __FILE__, __LINE__); ctx->err = b_; return 1; } } while (0)
+#define SB_CK(call, what) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return std::string(what) + ": " + cudaGetErrorString(e_); } while (0)
+#define SB_TRY(step) do { std::string r_ = (step); if (!r_.empty()) return r_; } while (0)
 
 int alloc_device(zstdb200_ctx* ctx, Device& d) {
   CK(cudaSetDevice(d.id));
@@ -122,7 +119,6 @@ int alloc_device(zstdb200_ctx* ctx, Device& d) {
   CK(cudaMalloc(&d.d_hufFull, d.hufFullBytes * NSTREAMS));
   CK(cudaMallocHost(&d.h_src, ctx->srcCap + 256)); CK(cudaMallocHost(&d.h_dst, ctx->srcCap + 256));
   CK(cudaMallocHost(&d.h_desc, items * 24 + 64));
-  CK(decode_configure());
   cudaError_t ee = encode_alloc(d.enc, ctx->maxBatch, items);
   if (ee != cudaSuccess) { ctx->err = std::string("encoder arena allocation failed: ") + cudaGetErrorString(ee); return 1; }
   return 0;
@@ -141,8 +137,6 @@ void free_device(Device& d) {
   if (d.descEv) cudaEventDestroy(d.descEv);
   for (auto& ev : d.sliceEv) cudaEventDestroy(ev);
 }
-
-struct Range { size_t lo, hi; };
 
 // true when the driver can DMA the range directly (cudaMallocHost / cudaHostRegister memory).  A managed caller's
 // `fixed`-pinned byte[] (ZStdDecompress.cs:2182-2186) is pinned for the GC only: pageable for CUDA.
@@ -188,48 +182,16 @@ bool host_item_content_size(const u8* src, u32 size, u64* total) {
   }
 }
 
-// Greedy split of [0, n) into consecutive sub-batches that respect the per-device arena limits.
-template <class FI, class FO>
-std::vector<Range> make_subbatches(size_t n, size_t maxIn, size_t maxOut, size_t maxItems, FI inBytes, FO outBytes, bool* tooBig) {
-  std::vector<Range> r; size_t lo = 0; *tooBig = false;
-  while (lo < n) {
-    size_t in = 0, out = 0, hi = lo;
-    while (hi < n && hi - lo < maxItems) {
-      size_t a = align_up(inBytes(hi), 16), b = align_up(outBytes(hi), 16);   // exactly what run_subbatch lays out
-      if (in + a > maxIn || out + b > maxOut) break;
-      in += a; out += b; hi++;
-    }
-    if (hi == lo) { *tooBig = true; return r; }   // a single item exceeds the arena
-    r.push_back({lo, hi}); lo = hi;
-  }
-  return r;
-}
-
 enum class Op { Decompress, Compress };
 
-// Switches a launch to the block-parallel path for multi-block frames (zb_blocks.cuh); ZSTDB200_PAR=0 keeps every frame
-// on the frame-serial kernels (A/B measurements).  Also hands every launch its per-stream scratch: slot = the stream slot
-// the launch runs on (its eight counters, its Huffman full-table region); the item lists are indexed by item_base, so
-// slices of one sub-batch that run concurrently use disjoint ranges of them.
-void with_units(Device& d, DecodeArgs& a, u32 slot, size_t ctx_items) {
-  static const bool on = env_int("ZSTDB200_PAR", 1, 0, 1) != 0;
-  static const u32 seqAMax = (u32)env_int("ZSTDB200_SEQ_A_MAX", 512, 0, 0x7FFFFFFF), seqBMax = (u32)env_int("ZSTDB200_SEQ_B_MAX", 2048, 0, 0x7FFFFFFF);
-  a.seq_a_max = seqAMax; a.seq_b_max = seqBMax;
-  a.huf_full = (u16*)(d.d_hufFull + d.hufFullBytes * slot);       // (every launch: the Huffman kernels' full-table scratch and the counters of this stream)
-  a.cnt = d.d_cnt + 8 * slot; a.par_list = d.d_parList; a.list_stride = (u32)(ctx_items + 1);
-  if (!on) return;
-  a.units = d.d_units;
-}
-
-// Items that hold more than one data frame (DecompressMultiFrame, ZStdDecompress.cs:2096-2160): after the first pass
-// the execute stage has counted them in *more; every further pass decodes the next data frame of each of them.
-// Synchronises `st` once per pass (the count has to reach the host).  `a` covers the same items as the first pass.
-cudaError_t decode_more_passes(Device& d, DecodeArgs a, u32 slot, cudaStream_t st, int* launches) {
+// Items that hold several data frames (DecompressMultiFrame, ZStdDecompress.cs:2096-2160): each pass from a.pass on decodes
+// the next data frame of every item and counts in *a.more (slot `slot`) the items with another; passes run until none has.
+// `st` is synchronised once per pass (the count has to reach the host).  marks: as for decode_launch, first pass only.
+cudaError_t decode_passes(Device& d, DecodeArgs a, u32 slot, cudaStream_t st, int* launches, cudaEvent_t* marks = nullptr) {
   cudaError_t e;
-  while (true) {
-    a.pass++; a.more = d.d_more + slot;
+  for (;; a.pass++, marks = nullptr) {
     if ((e = cudaMemsetAsync(a.more, 0, 4, st)) != cudaSuccess) return e;
-    if ((e = decode_launch(a, st, launches)) != cudaSuccess) return e;
+    if ((e = decode_launch(a, st, launches, marks)) != cudaSuccess) return e;
     if ((e = cudaMemcpyAsync(d.h_more + slot, a.more, 4, cudaMemcpyDeviceToHost, st)) != cudaSuccess) return e;
     if ((e = cudaStreamSynchronize(st)) != cudaSuccess) return e;
     if (d.h_more[slot] == 0) return cudaSuccess;
@@ -246,176 +208,152 @@ struct Job {
   bool useDict;        // compress with the context's dictionary (the *_using_dict calls)
 };
 
-// The encoder's dictionary on device d (zstdb200_load_dictionary put it on every device of the context)
-void set_dict(const zstdb200_ctx* ctx, const Device& d, EncodeArgs& a) {
-  const EncDict* h = reinterpret_cast<const EncDict*>(ctx->encDict.data());
-  a.dict = reinterpret_cast<const EncDict*>(d.d_encDict); a.dict_id = h->dictID; a.dict_err = h->err;
+// The arguments of one decode launch over n items, numbered from item_base in the arenas, on stream slot `slot` (its counters
+// and Huffman full-table region).  The item lists are indexed by item_base, so slices of one sub-batch that run concurrently
+// use disjoint ranges of them.  ZSTDB200_PAR=0 keeps every frame on the frame-serial kernels (A/B measurements).
+DecodeArgs decode_args(const zstdb200_ctx* ctx, const Device& d, const Items& it, size_t n, u32 item_base, u32 slot) {
+  static const bool par = env_int("ZSTDB200_PAR", 1, 0, 1) != 0;
+  static const u32 seqAMax = (u32)env_int("ZSTDB200_SEQ_A_MAX", 512, 0, 0x7FFFFFFF), seqBMax = (u32)env_int("ZSTDB200_SEQ_B_MAX", 2048, 0, 0x7FFFFFFF);
+  DecodeArgs a{};
+  a.src_base = it.src; a.src_off = it.srcOff; a.src_size = it.srcSize;
+  a.dst_base = it.dst; a.dst_off = it.dstOff; a.dst_cap = it.dstCap; a.result = it.result;
+  a.n = (u32)n; a.item_base = item_base; a.info = d.d_info + item_base; a.lit_arena = d.d_lit; a.seq_arena = d.d_seq;
+  a.dict = d.dictOn ? d.d_dictState : nullptr; a.dict_bytes = d.d_dict; a.pass = 0; a.more = d.d_more + slot;
+  a.units = par ? d.d_units : nullptr; a.par_list = d.d_parList; a.list_stride = (u32)(ctx->maxItems + 1); a.cnt = d.d_cnt + 8 * slot;
+  a.seq_a_max = seqAMax; a.seq_b_max = seqBMax; a.huf_full = (u16*)(d.d_hufFull + d.hufFullBytes * slot);
+  return a;
 }
 
-// One sub-batch [lo, hi) on one device: slices over NSTREAMS streams, direct DMA where the layout allows.
-// Returns "" or an error description.
-std::string run_subbatch(zstdb200_ctx* ctx, Device& d, const Job& j, size_t lo, size_t hi, uint64_t* launches) {
-  const size_t m = hi - lo;
-  auto fail = [&](const char* what, cudaError_t e) { return std::string(what) + ": " + cudaGetErrorString(e); };
-  // ---- layout analysis ----
-  bool srcDirect = true, dstDirect = true;
-  for (size_t k = 0; k + 1 < m && (srcDirect || dstDirect); k++) {
-    const size_t i = lo + k;
-    const u8 *s0 = (const u8*)j.src[i], *s1 = (const u8*)j.src[i + 1];
-    if (!(s1 >= s0 + j.srcSize[i] && s1 <= s0 + j.srcSize[i] + 64)) srcDirect = false;
-    const u8 *d0 = (const u8*)j.dst[i], *d1 = (const u8*)j.dst[i + 1];
-    if (d1 != d0 + j.dstCap[i] || j.effCap[i] != j.dstCap[i]) dstDirect = false;
-  }
-  if (j.effCap[hi - 1] != j.dstCap[hi - 1]) dstDirect = false;
-  const u8* srcBase = (const u8*)j.src[lo]; u8* dstBase = (u8*)j.dst[lo];
-  // pageable caller memory goes through the pinned staging with parallel host copies (a pageable cudaMemcpyAsync
-  // is a synchronous, single-threaded bounce inside the driver)
-  if (srcDirect && !is_dma_able(srcBase)) srcDirect = false;
-  if (dstDirect && !is_dma_able(dstBase)) dstDirect = false;
-  if (srcDirect) {
-    const size_t span = (size_t)((const u8*)j.src[hi - 1] - srcBase) + j.srcSize[hi - 1];
-    const size_t lim = j.op == Op::Decompress ? ctx->srcCap : ctx->dstSpan;
-    if (span > lim || !srcBase) srcDirect = false;
-  }
-  if (dstDirect) {
-    const size_t span = (size_t)((u8*)j.dst[hi - 1] - dstBase) + j.effCap[hi - 1];
-    const size_t lim = j.op == Op::Decompress ? ctx->dstSpan : ctx->srcCap;
-    if (span > lim || !dstBase) dstDirect = false;
-  }
-  // ---- descriptors (device offsets), packed for this m ----
-  d.h_srcOff = (u64*)d.h_desc; d.h_dstOff = d.h_srcOff + m; d.h_srcSize = (u32*)(d.h_dstOff + m); d.h_dstCap = d.h_srcSize + m;
-  u64* const d_srcOff = (u64*)d.d_desc; u64* const d_dstOff = d_srcOff + m; u32* const d_srcSize = (u32*)(d_dstOff + m); u32* const d_dstCap = d_srcSize + m;
-  size_t in = 0, out = 0;
-  for (size_t k = 0; k < m; k++) {
-    const size_t i = lo + k;
-    d.h_srcSize[k] = j.srcSize[i]; d.h_dstCap[k] = j.effCap[i];
-    d.h_srcOff[k] = srcDirect ? (u64)((const u8*)j.src[i] - srcBase) : in;
-    d.h_dstOff[k] = dstDirect ? (u64)((u8*)j.dst[i] - dstBase) : out;
-    in += align_up(j.srcSize[i], 16); out += align_up(j.effCap[i], 16);
-  }
-  // ---- slices ----
-  static const int nStreams = env_int("ZSTDB200_STREAMS", NSTREAMS, 1, NSTREAMS);
-  static const size_t SLICE_BYTES = (size_t)env_int("ZSTDB200_SLICE_MB", (int)(SLICE_BYTES_DEFAULT >> 20), 1, 4096) << 20;
+// One sub-batch [lo, hi) on one device and its plan (host_plan.h): direct DMA where the caller's layout allows, the
+// descriptors, the slices.  The steps return "" or an error description.
+struct SubBatch {
+  zstdb200_ctx* ctx; Device& d; const Job& j;
+  size_t lo, m; bool decode, srcDirect, dstDirect, eager;
+  const u8* srcBase; u8* dstBase;
+  DescView h;                    // the descriptors (device offsets) in the pinned staging
+  Items dev;                     // the items on the device
   std::vector<Range> slices;
-  {
-    size_t a = 0;
-    while (a < m) {
-      size_t b = a, bytes = 0;
-      // a slice is >= SLICE_BYTES and >= MIN_SLICE_ITEMS frames: the kernels take one frame-time however few frames
-      // they are given, so slices of a few large frames would serialise on that latency
-      static const int envMin = env_int("ZSTDB200_MIN_SLICE_ITEMS", 0, 0, 1 << 30);
-      const size_t minItems = envMin ? (size_t)envMin : (j.op == Op::Decompress ? MIN_SLICE_ITEMS_DECODE : MIN_SLICE_ITEMS_ENCODE);
-      // The first slices are smaller: output can only start to leave once a slice's kernels are done (one frame-time
-      // however small the slice), and the D2H engine then has to be fed without a gap while the big slices finish.
-      const size_t k = slices.size(), shrink = j.op == Op::Decompress ? (k < 2 ? 4 : (k < 4 ? 2 : 1)) : 1;
-      const size_t wantItems = std::max<size_t>(1, minItems / shrink), wantBytes = SLICE_BYTES / shrink;
-      while (b < m && (b - a < wantItems || bytes + std::max(d.h_dstCap[b], d.h_srcSize[b]) <= wantBytes)) { bytes += std::max(d.h_dstCap[b], d.h_srcSize[b]); b++; }
-      slices.push_back({a, b}); a = b;
+
+  SubBatch(zstdb200_ctx* c, Device& dv, const Job& jb, size_t lo_, size_t hi)
+      : ctx(c), d(dv), j(jb), lo(lo_), m(hi - lo_), decode(jb.op == Op::Decompress),
+        srcBase((const u8*)jb.src[lo_]), dstBase((u8*)jb.dst[lo_]), h(dv.h_desc, hi - lo_) {
+    // pageable caller memory goes through the pinned staging with parallel host copies (a pageable cudaMemcpyAsync
+    // is a synchronous, single-threaded bounce inside the driver)
+    const size_t inLim = decode ? ctx->srcCap : ctx->dstSpan, outLim = decode ? ctx->dstSpan : ctx->srcCap;
+    srcDirect = back_to_back(j.src + lo, j.srcSize + lo, m, 64, inLim) && is_dma_able(srcBase);
+    dstDirect = std::equal(j.effCap + lo, j.effCap + hi, j.dstCap + lo) && back_to_back(j.dst + lo, j.dstCap + lo, m, 0, outLim) &&
+                is_dma_able(dstBase);
+    size_t in = 0, out = 0;
+    for (size_t k = 0; k < m; k++) {
+      const size_t i = lo + k;
+      h.srcSize[k] = j.srcSize[i]; h.dstCap[k] = j.effCap[i];
+      h.srcOff[k] = srcDirect ? (u64)((const u8*)j.src[i] - srcBase) : in;
+      h.dstOff[k] = dstDirect ? (u64)((u8*)j.dst[i] - dstBase) : out;
+      in += align_up(j.srcSize[i], 16); out += align_up(j.effCap[i], 16);
     }
+    dev = DescView(d.d_desc, m).items(d.d_src, d.d_dst, d.d_result);
+    static const size_t sliceBytes = (size_t)env_int("ZSTDB200_SLICE_MB", (int)(SLICE_BYTES_DEFAULT >> 20), 1, 4096) << 20;
+    slices = plan_slices(h.srcSize, h.dstCap, m, decode, sliceBytes);
+    eager = !dstDirect && decode && slices.size() > 1;
   }
-  cudaError_t e;
+
   // Small copies cost the copy engines about as much as a megabyte each, and they queue between the slices'
   // payload copies: descriptors go up once per sub-batch, results and counters come back once at its end.
-  {
+  std::string start() {
     cudaStream_t s0 = d.stream[0];
-    e = cudaMemsetAsync(d.d_more, 0, NSTREAMS * 4, s0); if (e) return fail("memset", e);
-    e = cudaMemcpyAsync(d.d_desc, d.h_desc, m * 24, cudaMemcpyHostToDevice, s0); if (e) return fail("H2D desc", e);
+    SB_CK(cudaMemsetAsync(d.d_more, 0, NSTREAMS * 4, s0), "memset");
+    SB_CK(cudaMemcpyAsync(d.d_desc, d.h_desc, DescView::bytes(m), cudaMemcpyHostToDevice, s0), "H2D desc");
     if (slices.size() > 1) {
-      e = cudaEventRecord(d.descEv, s0); if (e) return fail("event", e);
-      for (int k = 1; k < NSTREAMS; k++) { e = cudaStreamWaitEvent(d.stream[k], d.descEv, 0); if (e) return fail("event wait", e); }
+      SB_CK(cudaEventRecord(d.descEv, s0), "event");
+      for (int k = 1; k < NSTREAMS; k++) SB_CK(cudaStreamWaitEvent(d.stream[k], d.descEv, 0), "event wait");
     }
+    if (eager) while (d.sliceEv.size() < slices.size()) { cudaEvent_t ev; SB_CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming), "event create"); d.sliceEv.push_back(ev); }
+    return "";
   }
-  static const bool trace = getenv("ZSTDB200_TRACE") != nullptr;   // per-slice timeline on stderr (tuning aid)
-  const bool eager = !dstDirect && j.op == Op::Decompress && slices.size() > 1;
-  if (eager) while (d.sliceEv.size() < slices.size()) { cudaEvent_t ev; e = cudaEventCreateWithFlags(&ev, cudaEventDisableTiming); if (e) return fail("event create", e); d.sliceEv.push_back(ev); }
-  std::vector<cudaEvent_t> tev;
-  if (trace) { tev.resize(1 + 3 * slices.size()); for (auto& x : tev) cudaEventCreate(&x); cudaEventRecord(tev[0], d.stream[0]); }
-  for (size_t s = 0; s < slices.size(); s++) {
-    const size_t a = slices[s].lo, b = slices[s].hi, cnt = b - a;
-    cudaStream_t st = d.stream[s % nStreams];
-    // input bytes of the slice
-    const size_t inLo = d.h_srcOff[a], inHi = d.h_srcOff[b - 1] + d.h_srcSize[b - 1];
-    if (srcDirect) {
-      if (inHi > inLo) { e = cudaMemcpyAsync(d.d_src + inLo, srcBase + inLo, inHi - inLo, cudaMemcpyHostToDevice, st); if (e) return fail("H2D src", e); }
-    } else {
-      parallel_for(b - a, inHi - inLo, [&](size_t x, size_t y) {
-        for (size_t k = a + x; k < a + y; k++) if (d.h_srcSize[k]) memcpy(d.h_src + d.h_srcOff[k], j.src[lo + k], d.h_srcSize[k]);
-      });
-      if (inHi > inLo) { e = cudaMemcpyAsync(d.d_src + inLo, d.h_src + inLo, inHi - inLo, cudaMemcpyHostToDevice, st); if (e) return fail("H2D src", e); }
-    }
-    if (trace) cudaEventRecord(tev[1 + 3 * s], st);
+
+  std::string stage_in(size_t a, size_t b, cudaStream_t st) {
+    const size_t inLo = h.srcOff[a], inHi = h.srcOff[b - 1] + h.srcSize[b - 1];
+    if (!srcDirect) parallel_for(b - a, inHi - inLo, [&](size_t x, size_t y) {
+      for (size_t k = a + x; k < a + y; k++) if (h.srcSize[k]) memcpy(d.h_src + h.srcOff[k], j.src[lo + k], h.srcSize[k]);
+    });
+    if (inHi > inLo) SB_CK(cudaMemcpyAsync(d.d_src + inLo, (srcDirect ? srcBase : d.h_src) + inLo, inHi - inLo, cudaMemcpyHostToDevice, st), "H2D src");
+    return "";
+  }
+
+  std::string launch(size_t a, size_t b, u32 slot, cudaStream_t st, uint64_t* launches) {
     int nl = 0;
-    if (j.op == Op::Decompress) {
-      DecodeArgs ar{d.d_src, d_srcOff + a, d_srcSize + a, d.d_dst, d_dstOff + a, d_dstCap + a, d.d_result + a, (u32)cnt, (u32)a,
-                    d.d_info + a, d.d_lit, d.d_seq, d.dictOn ? d.d_dictState : nullptr, d.d_dict, 0, d.d_more + (s % nStreams)};
-      with_units(d, ar, (u32)(s % nStreams), ctx->maxItems);
-      e = decode_launch(ar, st, &nl);
-    } else {
-      EncodeArgs ar{d.d_src, d_srcOff + a, d_srcSize + a, d.d_dst, d_dstOff + a, d_dstCap + a, d.d_result + a, (u32)cnt, (u32)a,
-                    j.level, j.checksum, j.maxSrc, (u32)(s % nStreams)};
-      if (j.useDict) set_dict(ctx, d, ar);
-      e = encode_launch(ar, d.enc, st, &nl);
-    }
+    const cudaError_t e = decode ? decode_launch(decode_args(ctx, d, dev.from(a), b - a, (u32)a, slot), st, &nl)
+                                 : encode_launch(encode_args(dev.from(a), b - a, (u32)a, j.level, j.checksum, j.maxSrc, slot,
+                                                             j.useDict ? d.d_encDict : nullptr, &ctx->encDict), d.enc, st, &nl);
     *launches += nl;
-    if (e) return fail("kernel launch", e);
-    if (trace) cudaEventRecord(tev[2 + 3 * s], st);
-    const size_t outLo = d.h_dstOff[a], outHi = d.h_dstOff[b - 1] + d.h_dstCap[b - 1];
-    if (outHi > outLo) {
-      u8* hostDst = dstDirect ? dstBase + outLo : d.h_dst + outLo;
-      e = cudaMemcpyAsync(hostDst, d.d_dst + outLo, outHi - outLo, cudaMemcpyDeviceToHost, st); if (e) return fail("D2H dst", e);
-    }
-    if (trace) cudaEventRecord(tev[3 + 3 * s], st);
-    if (eager) { e = cudaEventRecord(d.sliceEv[s], st); if (e) return fail("event", e); }
+    SB_CK(e, "kernel launch");
+    return "";
   }
-  // Pageable destinations of a decode: scatter every slice out of the pinned staging as soon as its copy has landed,
-  // while the later slices are still in flight (the whole capacity of each item is copied: the result codes only arrive
-  // at the end; bytes past result[i] are unspecified, include/zstdb200.h).
-  if (eager)
-    for (size_t s = 0; s < slices.size(); s++) {
-      e = cudaEventSynchronize(d.sliceEv[s]); if (e) return fail("event sync", e);
+
+  std::string stage_out(size_t a, size_t b, cudaStream_t st) {
+    const size_t outLo = h.dstOff[a], outHi = h.dstOff[b - 1] + h.dstCap[b - 1];
+    if (outHi > outLo) SB_CK(cudaMemcpyAsync((dstDirect ? dstBase : d.h_dst) + outLo, d.d_dst + outLo, outHi - outLo, cudaMemcpyDeviceToHost, st), "D2H dst");
+    return "";
+  }
+
+  std::string finish(uint64_t* launches) {
+    // Pageable destinations of a decode: scatter every slice out of the pinned staging as soon as its copy has landed,
+    // while the later slices are still in flight (the whole capacity of each item is copied: the result codes only arrive
+    // at the end; bytes past result[i] are unspecified, include/zstdb200.h).
+    for (size_t s = 0; eager && s < slices.size(); s++) {
+      SB_CK(cudaEventSynchronize(d.sliceEv[s]), "event sync");
       const size_t a = slices[s].lo, b = slices[s].hi;
-      parallel_for(b - a, d.h_dstOff[b - 1] + d.h_dstCap[b - 1] - d.h_dstOff[a], [&](size_t x, size_t y) {
-        for (size_t k = a + x; k < a + y; k++) if (d.h_dstCap[k]) memcpy(j.dst[lo + k], d.h_dst + d.h_dstOff[k], d.h_dstCap[k]);
+      parallel_for(b - a, h.dstOff[b - 1] + h.dstCap[b - 1] - h.dstOff[a], [&](size_t x, size_t y) {
+        for (size_t k = a + x; k < a + y; k++) if (h.dstCap[k]) memcpy(j.dst[lo + k], d.h_dst + h.dstOff[k], h.dstCap[k]);
       });
     }
-  // a single slice ran on stream 0 alone: its results ride the same stream and one synchronisation ends the call
-  if (slices.size() > 1) for (auto& st : d.stream) { e = cudaStreamSynchronize(st); if (e) return fail("stream sync", e); }
-  if (trace) {
-    if (slices.size() == 1) cudaStreamSynchronize(d.stream[0]);
-    for (size_t s = 0; s < slices.size(); s++) {
-      float t1 = 0, t2 = 0, t3 = 0;
-      cudaEventElapsedTime(&t1, tev[0], tev[1 + 3 * s]); cudaEventElapsedTime(&t2, tev[0], tev[2 + 3 * s]); cudaEventElapsedTime(&t3, tev[0], tev[3 + 3 * s]);
-      fprintf(stderr, "[zstdb200] slice %2zu items %6zu: h2d done %7.3f  kernels done %7.3f  d2h done %7.3f ms\n", s, slices[s].hi - slices[s].lo, t1, t2, t3);
+    // a single slice ran on stream 0 alone: its results ride the same stream and one synchronisation ends the call
+    if (slices.size() > 1) for (auto& st : d.stream) SB_CK(cudaStreamSynchronize(st), "stream sync");
+    SB_CK(cudaMemcpyAsync(d.h_more, d.d_more, (NSTREAMS + m) * 4, cudaMemcpyDeviceToHost, d.stream[0]), "D2H results");
+    SB_CK(cudaStreamSynchronize(d.stream[0]), "stream sync");
+    u32 anyMore = 0;
+    for (int k = 0; k < NSTREAMS; k++) anyMore |= d.h_more[k];
+    if (decode && anyMore) {
+      // rare path: some items hold several data frames.  Everything is still resident: decode the remaining frames
+      // pass by pass over the whole sub-batch, then fetch results and output again.
+      cudaStream_t st = d.stream[0]; int nl = 0;
+      DecodeArgs a = decode_args(ctx, d, dev, m, 0, 0); a.pass = 1;
+      const cudaError_t e = decode_passes(d, a, 0, st, &nl);
+      *launches += nl;
+      SB_CK(e, "multi-frame passes");
+      SB_CK(cudaMemcpyAsync(d.h_result, d.d_result, m * 4, cudaMemcpyDeviceToHost, st), "D2H result");
+      SB_TRY(stage_out(0, m, st));
+      SB_CK(cudaStreamSynchronize(st), "stream sync");
     }
-    for (auto& x : tev) cudaEventDestroy(x);
+    for (size_t k = 0; k < m; k++) j.result[lo + k] = d.h_result[k];
+    // staged output not scattered yet (compress: frames are much smaller than their capacity; single-slice calls; items
+    // that needed further passes): copy what was produced; on error the reference leaves dst partially written, we copy nothing
+    if (!dstDirect && (!eager || anyMore)) parallel_for(m, h.dstOff[m - 1] + h.dstCap[m - 1], [&](size_t x, size_t y) {
+      for (size_t k = x; k < y; k++) {
+        const size_t i = lo + k; const u32 r = d.h_result[k];
+        if (!is_err(r) && r) memcpy(j.dst[i], d.h_dst + h.dstOff[k], std::min<u32>(r, j.dstCap[i]));
+      }
+    });
+    return "";
   }
-  e = cudaMemcpyAsync(d.h_more, d.d_more, (NSTREAMS + m) * 4, cudaMemcpyDeviceToHost, d.stream[0]); if (e) return fail("D2H results", e);
-  e = cudaStreamSynchronize(d.stream[0]); if (e) return fail("stream sync", e);
-  u32 anyMore = 0;
-  for (int k = 0; k < NSTREAMS; k++) anyMore |= d.h_more[k];
-  if (j.op == Op::Decompress && anyMore) {
-    // rare path: some items hold several data frames.  Everything is still resident: decode the remaining frames
-    // pass by pass over the whole sub-batch, then fetch results and output again.
-    cudaStream_t st = d.stream[0]; int nl = 0;
-    DecodeArgs ar{d.d_src, d_srcOff, d_srcSize, d.d_dst, d_dstOff, d_dstCap, d.d_result, (u32)m, 0, d.d_info, d.d_lit, d.d_seq, d.dictOn ? d.d_dictState : nullptr, d.d_dict, 0, nullptr};
-    with_units(d, ar, 0, ctx->maxItems);
-    e = decode_more_passes(d, ar, 0, st, &nl); *launches += nl;
-    if (e) return fail("multi-frame passes", e);
-    e = cudaMemcpyAsync(d.h_result, d.d_result, m * 4, cudaMemcpyDeviceToHost, st); if (e) return fail("D2H result", e);
-    const size_t outLo = d.h_dstOff[0], outHi = d.h_dstOff[m - 1] + d.h_dstCap[m - 1];
-    if (outHi > outLo) { e = cudaMemcpyAsync(dstDirect ? dstBase + outLo : d.h_dst + outLo, d.d_dst + outLo, outHi - outLo, cudaMemcpyDeviceToHost, st); if (e) return fail("D2H dst", e); }
-    e = cudaStreamSynchronize(st); if (e) return fail("stream sync", e);
+};
+
+// Descriptors up in one copy, then stage in / launch / stage out per slice, the slices dealt round-robin to the streams, then
+// finish.
+std::string run_subbatch(zstdb200_ctx* ctx, Device& d, const Job& j, size_t lo, size_t hi, uint64_t* launches) {
+  static const int nStreams = env_int("ZSTDB200_STREAMS", NSTREAMS, 1, NSTREAMS);
+  SubBatch sb(ctx, d, j, lo, hi);
+  SB_TRY(sb.start());
+  for (size_t s = 0; s < sb.slices.size(); s++) {
+    const size_t a = sb.slices[s].lo, b = sb.slices[s].hi;
+    const u32 slot = (u32)(s % nStreams);
+    cudaStream_t st = d.stream[slot];
+    SB_TRY(sb.stage_in(a, b, st));
+    SB_TRY(sb.launch(a, b, slot, st, launches));
+    SB_TRY(sb.stage_out(a, b, st));
+    if (sb.eager) SB_CK(cudaEventRecord(d.sliceEv[s], st), "event");
   }
-  for (size_t k = 0; k < m; k++) j.result[lo + k] = d.h_result[k];
-  // staged output not scattered yet (compress: frames are much smaller than their capacity; single-slice calls; items
-  // that needed further passes): copy what was produced; on error the reference leaves dst partially written, we copy nothing
-  if (!dstDirect && (!eager || anyMore)) parallel_for(m, d.h_dstOff[m - 1] + d.h_dstCap[m - 1], [&](size_t x, size_t y) {
-    for (size_t k = x; k < y; k++) {
-      const size_t i = lo + k; const u32 r = d.h_result[k];
-      if (!is_err(r) && r) memcpy(j.dst[i], d.h_dst + d.h_dstOff[k], std::min<u32>(r, j.dstCap[i]));
-    }
-  });
-  return "";
+  return sb.finish(launches);
 }
 
 int run_host_batch(zstdb200_ctx* ctx, const Job& j0, size_t n, bool clamp = true) {
@@ -454,24 +392,7 @@ int run_host_batch(zstdb200_ctx* ctx, const Job& j0, size_t n, bool clamp = true
   if (tooBig) { ctx->err = "an item is larger than the context's max_batch_bytes"; return 1; }
   // a single sub-batch on a multi-GPU context is re-cut so that every device gets a share
   const size_t nd = ctx->dev.size();
-  if (nd > 1 && subs.size() < nd) {
-    std::vector<Range> cut;
-    for (auto& r : subs) {
-      // equal shares of bytes (in + out), not of items: a raw-block frame costs a copy, a text frame a full decode
-      const size_t parts = std::min(nd, r.hi - r.lo);
-      uint64_t total = 0;
-      for (size_t i = r.lo; i < r.hi; i++) total += (uint64_t)j.srcSize[i] + j.effCap[i] + 1;
-      size_t lo = r.lo; uint64_t acc = 0;
-      for (size_t p = 0; p < parts; p++) {
-        size_t hi = lo;
-        const uint64_t want = total * (p + 1) / parts;
-        while (hi < r.hi && (acc < want || hi == lo) && (r.hi - hi) > (parts - 1 - p)) { acc += (uint64_t)j.srcSize[hi] + j.effCap[hi] + 1; hi++; }
-        if (p + 1 == parts) hi = r.hi;
-        cut.push_back({lo, hi}); lo = hi;
-      }
-    }
-    subs.swap(cut);
-  }
+  subs = split_over_devices(std::move(subs), nd, [&](size_t i) { return (uint64_t)j.srcSize[i] + j.effCap[i] + 1; });
   std::vector<std::string> errs(nd);
   std::vector<uint64_t> launches(nd, 0);
   auto worker = [&](size_t di) {
@@ -501,6 +422,31 @@ int run_host_batch(zstdb200_ctx* ctx, const Job& j0, size_t n, bool clamp = true
     for (size_t k = 0; k < m; k++) j.result[again[k]] = r2[k];
   }
   return 0;
+}
+
+// The checks every device-pointer entry point starts with (compress: the level and a loaded dictionary too); then the device
+// is selected.  *st: the caller's stream, or the device's first one.
+int device_call(zstdb200_ctx* ctx, Op op, int device_index, size_t n, int level, bool useDict, void* stream, Device** d, cudaStream_t* st) {
+  if (!ctx) return 1;
+  ctx->err.clear();
+  if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
+  if (op == Op::Compress && (level < 1 || level > 3)) { ctx->err = "level must be 1..3"; return 1; }
+  if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
+  if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
+  *d = &ctx->dev[device_index];
+  CK(cudaSetDevice((*d)->id));
+  *st = stream ? (cudaStream_t)stream : (*d)->stream[0];
+  return 0;
+}
+
+// One item through a batch call.  A null array is an empty one (the C# shim passes null for byte[0]).
+template <class F>
+uint32_t one_item(void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize, F batch) {
+  static unsigned char dummy[16];
+  if (!src) { src = dummy; srcSize = 0; }
+  if (!dst) { dst = dummy; dstCapacity = 0; }
+  uint32_t r = zerr(ZE_GENERIC);
+  return batch(&src, &srcSize, &dst, &dstCapacity, &r) ? zerr(ZE_GENERIC) : r;
 }
 
 }  // namespace
@@ -575,13 +521,9 @@ int zstdb200_load_dictionary(zstdb200_ctx* ctx, const void* dict, uint32_t dictS
   // every device gets a copy of the block
   ctx->encDict.clear();
   if (dict && dictSize) {
-    std::vector<u8> bytes((const u8*)dict, (const u8*)dict + dictSize); bytes.resize((size_t)dictSize + 64, 0);
-    std::unique_ptr<DictState> ds(new DictState());
-    HufBuildWk wk; HufFseScratch fs; u8 slot[260]; s16 norm[64]; u16 next[64];
-    dict_load(bytes.data(), dictSize, *ds, wk, fs, slot, norm, next);
-    ctx->encDict.assign((enc_dict_bytes(ds->err ? 0 : ds->contentSize) + 15) / 16, uint4{});
-    std::vector<u8> tableSymbol(512);
-    enc_dict_prepare(bytes.data(), dictSize, *ds, reinterpret_cast<EncDict*>(ctx->encDict.data()), wk, fs, slot, tableSymbol.data());
+    DictState ds{};
+    dict_load_host((const u8*)dict, dictSize, ds);
+    ctx->encDict = enc_dict_block((const u8*)dict, dictSize, ds);
   }
   for (auto& d : ctx->dev) {
     CK(cudaSetDevice(d.id));
@@ -614,27 +556,21 @@ int zstdb200_decompress_batch(zstdb200_ctx* ctx, const void* const* src, const u
 }
 
 uint32_t zstdb200_decompress(zstdb200_ctx* ctx, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize) {
-  uint32_t r = zerr(ZE_GENERIC);
-  const void* s = src; void* d = dst;
-  static unsigned char dummy[16];
-  if (!d) { d = dummy; dstCapacity = 0; }        // a null array is an empty one (the C# shim passes null for byte[0])
-  if (!s) { s = dummy; srcSize = 0; }
-  if (zstdb200_decompress_batch(ctx, &s, &srcSize, &d, &dstCapacity, &r, 1)) return zerr(ZE_GENERIC);
-  return r;
+  return one_item(dst, dstCapacity, src, srcSize, [&](auto s, auto ss, auto d, auto dc, auto r) { return zstdb200_decompress_batch(ctx, s, ss, d, dc, r, 1); });
 }
 
 // Device-resident decode: one launch sequence over the whole batch on the caller's stream (slicing a resident batch
 // over several streams was measured slower: whole-batch kernels fill the GPU better).  The count of items that
 // hold a further data frame has to reach the host, so this entry point synchronises the stream once per pass.
-static int decode_device(zstdb200_ctx* ctx, Device& d, const DecodeArgs& a, cudaStream_t user, cudaEvent_t* marks) {
+static int decompress_device(zstdb200_ctx* ctx, int device_index, const void* src_base, const uint64_t* src_off, const uint32_t* src_size,
+                             void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream,
+                             EventSet<DECODE_KERNELS + 1>* es) {
+  Device* d; cudaStream_t st;
+  if (device_call(ctx, Op::Decompress, device_index, n, 0, false, stream, &d, &st)) return 1;
+  if (es) CK(es->create());
+  const DecodeArgs a = decode_args(ctx, *d, Items{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result}, n, 0, 0);
   int nl = 0;
-  DecodeArgs b = a; b.pass = 0; b.more = d.d_more;
-  with_units(d, b, 0, ctx->maxItems);
-  CK(cudaMemsetAsync(b.more, 0, 4, user));
-  CK(decode_launch(b, user, &nl, marks));
-  CK(cudaMemcpyAsync(d.h_more, b.more, 4, cudaMemcpyDeviceToHost, user));
-  CK(cudaStreamSynchronize(user));
-  if (d.h_more[0]) CK(decode_more_passes(d, b, 0, user, &nl));
+  CK(decode_passes(*d, a, 0, st, &nl, es ? es->ev : nullptr));
   ctx->launches += nl;
   return 0;
 }
@@ -642,14 +578,7 @@ static int decode_device(zstdb200_ctx* ctx, Device& d, const DecodeArgs& a, cuda
 int zstdb200_decompress_batch_device(zstdb200_ctx* ctx, int device_index, const void* src_base, const uint64_t* src_off,
                                      const uint32_t* src_size, void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap,
                                      uint32_t* result, size_t n, void* stream) {
-  if (!ctx) return 1;
-  ctx->err.clear();
-  if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
-  if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
-  Device& d = ctx->dev[device_index];
-  CK(cudaSetDevice(d.id));
-  DecodeArgs a{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result, (u32)n, 0, d.d_info, d.d_lit, d.d_seq, d.dictOn ? d.d_dictState : nullptr, d.d_dict, 0, nullptr};
-  return decode_device(ctx, d, a, stream ? (cudaStream_t)stream : d.stream[0], nullptr);
+  return decompress_device(ctx, device_index, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, nullptr);
 }
 
 // Same work as one launch sequence with CUDA events between the kernels: per-kernel device times for the
@@ -657,36 +586,14 @@ int zstdb200_decompress_batch_device(zstdb200_ctx* ctx, int device_index, const 
 int zstdb200_decompress_batch_device_timed(zstdb200_ctx* ctx, int device_index, const void* src_base, const uint64_t* src_off,
                                            const uint32_t* src_size, void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap,
                                            uint32_t* result, size_t n, void* stream, float* kernel_ms, int max_kernels) {
-  if (!ctx) return 1;
-  ctx->err.clear();
-  if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
-  if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
-  Device& d = ctx->dev[device_index];
-  CK(cudaSetDevice(d.id));
-  cudaStream_t st = stream ? (cudaStream_t)stream : d.stream[0];
-  EventSet<DECODE_KERNELS + 1> es; CK(es.create());
-  cudaEvent_t* ev = es.ev;
-  DecodeArgs a{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result, (u32)n, 0, d.d_info, d.d_lit, d.d_seq, d.dictOn ? d.d_dictState : nullptr, d.d_dict, 0, nullptr};
-  if (decode_device(ctx, d, a, st, ev)) return 1;
-  CK(cudaStreamSynchronize(st));
-  for (int k = 0; k < DECODE_KERNELS && k < max_kernels; k++) CK(cudaEventElapsedTime(&kernel_ms[k], ev[k], ev[k + 1]));
+  EventSet<DECODE_KERNELS + 1> es;
+  if (decompress_device(ctx, device_index, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, &es)) return 1;
+  CK(es.read(kernel_ms, max_kernels));
   return 0;
 }
 const char* zstdb200_decode_kernel_name(int k) { return (k >= 0 && k < DECODE_KERNELS) ? kDecodeKernelNames[k] : ""; }
 
 size_t zstdb200_compress_bound(size_t srcSize) { return encode_bound(srcSize); }
-
-// The device-pointer compress entry points learn the largest chunk of the call (it selects the match stage's table
-// sizes) by fetching the size array once: one small copy and one synchronisation of the stream.
-static int device_max_u32(zstdb200_ctx* ctx, Device& d, const uint32_t* d_vals, size_t n, cudaStream_t st, u32* out) {
-  *out = 0;
-  if (n == 0) return 0;
-  u32* h = (u32*)d.h_desc;
-  CK(cudaMemcpyAsync(h, d_vals, n * 4, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
-  for (size_t i = 0; i < n; i++) *out = std::max(*out, h[i]);
-  return 0;
-}
 
 // The compress entry points with and without the context's dictionary share these bodies (useDict).
 static int compress_batch(zstdb200_ctx* ctx, int level, int checksum, const void* const* src, const uint32_t* srcSize,
@@ -699,34 +606,24 @@ static int compress_batch(zstdb200_ctx* ctx, int level, int checksum, const void
   return run_host_batch(ctx, j, n);
 }
 
-static uint32_t compress_one(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize,
-                             bool useDict) {
-  uint32_t r = zerr(ZE_GENERIC);
-  const void* s = src; void* d = dst;
-  static unsigned char dummy[16];
-  if (!s) { s = dummy; srcSize = 0; }
-  if (!d) { d = dummy; dstCapacity = 0; }
-  if (compress_batch(ctx, level, checksum, &s, &srcSize, &d, &dstCapacity, &r, 1, useDict)) return zerr(ZE_GENERIC);
-  return r;
-}
-
-static int compress_batch_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
-                                 const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
-                                 const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream, bool useDict) {
-  if (!ctx) return 1;
-  ctx->err.clear();
-  if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
-  if (level < 1 || level > 3) { ctx->err = "level must be 1..3"; return 1; }
-  if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
-  if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
-  Device& d = ctx->dev[device_index];
-  CK(cudaSetDevice(d.id));
+static int compress_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base, const uint64_t* src_off,
+                           const uint32_t* src_size, void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap, uint32_t* result,
+                           size_t n, void* stream, bool useDict, EventSet<ENCODE_KERNELS + 1>* es) {
+  Device* d; cudaStream_t st;
+  if (device_call(ctx, Op::Compress, device_index, n, level, useDict, stream, &d, &st)) return 1;
+  if (es) CK(es->create());
+  // the largest chunk of the call selects the match stage's table sizes: the size array comes to the host once (one small
+  // copy and one synchronisation of the stream)
   u32 maxSrc = 0;
-  if (device_max_u32(ctx, d, src_size, n, stream ? (cudaStream_t)stream : d.stream[0], &maxSrc)) return 1;
-  EncodeArgs a{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result, (u32)n, 0, level, checksum, maxSrc, ENC_EXCLUSIVE};
-  if (useDict) set_dict(ctx, d, a);
+  if (n) {
+    CK(cudaMemcpyAsync(d->h_desc, src_size, n * 4, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    maxSrc = *std::max_element((const u32*)d->h_desc, (const u32*)d->h_desc + n);
+  }
+  const Items it{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result};
   int nl = 0;
-  CK(encode_launch(a, d.enc, stream ? (cudaStream_t)stream : d.stream[0], &nl));
+  CK(encode_launch(encode_args(it, n, 0, level, checksum, maxSrc, ENC_EXCLUSIVE, useDict ? d->d_encDict : nullptr, &ctx->encDict), d->enc,
+                   st, &nl, es ? es->ev : nullptr));
   ctx->launches += nl;
   return 0;
 }
@@ -740,44 +637,30 @@ int zstdb200_compress_batch_using_dict(zstdb200_ctx* ctx, int level, int checksu
   return compress_batch(ctx, level, checksum, src, srcSize, dst, dstCap, result, n, true);
 }
 uint32_t zstdb200_compress(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize) {
-  return compress_one(ctx, level, checksum, dst, dstCapacity, src, srcSize, false);
+  return one_item(dst, dstCapacity, src, srcSize, [&](auto s, auto ss, auto d, auto dc, auto r) { return compress_batch(ctx, level, checksum, s, ss, d, dc, r, 1, false); });
 }
 uint32_t zstdb200_compress_using_dict(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize) {
-  return compress_one(ctx, level, checksum, dst, dstCapacity, src, srcSize, true);
+  return one_item(dst, dstCapacity, src, srcSize, [&](auto s, auto ss, auto d, auto dc, auto r) { return compress_batch(ctx, level, checksum, s, ss, d, dc, r, 1, true); });
 }
 int zstdb200_compress_batch_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
                                    const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
                                    const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream) {
-  return compress_batch_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, false);
+  return compress_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, false, nullptr);
 }
 int zstdb200_compress_batch_device_using_dict(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
                                               const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
                                               const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream) {
-  return compress_batch_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, true);
+  return compress_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, true, nullptr);
 }
 
 // zstdb200_compress_batch_device with CUDA events between its kernels (see zstdb200_decompress_batch_device_timed).
 int zstdb200_compress_batch_device_timed(zstdb200_ctx* ctx, int device_index, int level, int checksum, const void* src_base,
                                          const uint64_t* src_off, const uint32_t* src_size, void* dst_base, const uint64_t* dst_off,
                                          const uint32_t* dst_cap, uint32_t* result, size_t n, void* stream, float* kernel_ms, int max_kernels) {
-  if (!ctx) return 1;
-  ctx->err.clear();
-  if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
-  if (level < 1 || level > 3) { ctx->err = "level must be 1..3"; return 1; }
-  if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
-  Device& d = ctx->dev[device_index];
-  CK(cudaSetDevice(d.id));
-  cudaStream_t st = stream ? (cudaStream_t)stream : d.stream[0];
-  EventSet<ENCODE_KERNELS + 1> es; CK(es.create());
-  cudaEvent_t* ev = es.ev;
-  u32 maxSrc = 0;
-  if (device_max_u32(ctx, d, src_size, n, st, &maxSrc)) return 1;
-  EncodeArgs a{(const u8*)src_base, src_off, src_size, (u8*)dst_base, dst_off, dst_cap, result, (u32)n, 0, level, checksum, maxSrc, ENC_EXCLUSIVE};
-  int nl = 0;
-  CK(encode_launch(a, d.enc, st, &nl, ev));
-  ctx->launches += nl;
-  CK(cudaStreamSynchronize(st));
-  for (int k = 0; k < ENCODE_KERNELS && k < max_kernels; k++) CK(cudaEventElapsedTime(&kernel_ms[k], ev[k], ev[k + 1]));
+  EventSet<ENCODE_KERNELS + 1> es;
+  if (compress_device(ctx, device_index, level, checksum, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream, false, &es))
+    return 1;
+  CK(es.read(kernel_ms, max_kernels));
   return 0;
 }
 const char* zstdb200_encode_kernel_name(int k) { return (k >= 0 && k < ENCODE_KERNELS) ? kEncodeKernelNames[k] : ""; }

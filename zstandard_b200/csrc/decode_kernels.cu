@@ -1209,10 +1209,9 @@ cudaError_t decode_configure() {
 
 const char* const kDecodeKernelNames[DECODE_KERNELS] = {"k_parse", "k_huf", "k_seq", "k_exec", "k_xxh"};
 
-// The pipeline in two halves (entropy stages, execute stages).  They were split to overlap slices on different
-// streams; that measured slower (the execute warps starve the lone FSE warps of an SM), so decode_launch runs both
-// on one stream.
-cudaError_t decode_launch_entropy(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks) {
+// The whole pipeline on one stream.  Running the entropy stages of one slice beside the execute stages of another on a
+// second stream measured slower (the execute warps starve the lone FSE warps of an SM).
+cudaError_t decode_launch(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks) {
   if (a.n == 0) return cudaSuccess;
   { cudaError_t e = cudaMemsetAsync(a.cnt, 0, 32, st); if (e != cudaSuccess) return e; }
   if (marks) cudaEventRecord(marks[0], st);
@@ -1229,10 +1228,7 @@ cudaError_t decode_launch_entropy(const DecodeArgs& a, cudaStream_t st, int* lau
   if (a.units) k_seq_blk<<<g_par_grid_seq, 32, sizeof(SeqSmem), st>>>(a);
   if (marks) cudaEventRecord(marks[3], st);
   if (launches) *launches += a.units ? 8 : 6;
-  return cudaGetLastError();
-}
-cudaError_t decode_launch_exec(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks) {
-  if (a.n == 0) return cudaSuccess;
+  { cudaError_t e = cudaGetLastError(); if (e != cudaSuccess) return e; }
   if (a.dict) k_exec<true><<<(a.n + (EXEC_THREADS / 32) - 1) / (EXEC_THREADS / 32), EXEC_THREADS, 0, st>>>(a);
   else k_exec<false><<<(a.n + (EXEC_THREADS / 32) - 1) / (EXEC_THREADS / 32), EXEC_THREADS, 0, st>>>(a);
   if (a.units) {
@@ -1248,11 +1244,6 @@ cudaError_t decode_launch_exec(const DecodeArgs& a, cudaStream_t st, int* launch
   if (marks) cudaEventRecord(marks[5], st);
   if (launches) *launches += a.units ? 6 : 2;
   return cudaGetLastError();
-}
-cudaError_t decode_launch(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks) {
-  cudaError_t e = decode_launch_entropy(a, st, launches, marks);
-  if (e != cudaSuccess) return e;
-  return decode_launch_exec(a, st, launches, marks);
 }
 
 }  // namespace zb

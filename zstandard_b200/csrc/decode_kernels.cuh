@@ -48,9 +48,6 @@ cudaError_t decode_configure();
 cudaError_t decode_load_dictionary(const u8* d_dict_bytes, u32 size, DictState* d_state, cudaStream_t st);
 // enqueues the whole decode pipeline for one batch on `st`; *launches += number of kernels launched
 cudaError_t decode_launch(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks = nullptr);
-// the two halves of decode_launch
-cudaError_t decode_launch_entropy(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks = nullptr);
-cudaError_t decode_launch_exec(const DecodeArgs& a, cudaStream_t st, int* launches, cudaEvent_t* marks = nullptr);
 // marks (optional): DECODE_KERNELS + 1 events recorded before the first kernel and after each kernel
 // (the block-parallel kernels k_huf_blk / k_seq_blk / k_exec_big run right after k_huf / k_seq / k_exec and are timed with them)
 #define DECODE_KERNELS 5

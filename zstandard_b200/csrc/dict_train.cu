@@ -163,8 +163,6 @@ struct DevBufs {
   }
 };
 
-size_t a16(size_t v) { return (v + 15) & ~(size_t)15; }
-
 }  // namespace
 
 #define DTCK(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { err = std::string(#call) + ": " + cudaGetErrorString(e_); return zerr(ZE_GENERIC); } } while (0)
@@ -236,15 +234,11 @@ u32 dt_train_run(DtDevice& dv, u8* dict, u32 capacity, const u8* samples, const 
 
   // encoder dictionaries: host preparation as in zstdb200_load_dictionary, one device block reused by every candidate
   u8* dEnc = nullptr; size_t encCap = 0;
-  HufBuildWk wk; HufFseScratch fs; u8 slot[260]; s16 norm[64]; u16 next[64];
-  std::vector<u8> tableSymbol(512);
   std::vector<uint4> enc;
   auto upload = [&](const u8* bytes, u32 size, bool raw) -> cudaError_t {
-    std::vector<u8> b(bytes, bytes + size); b.resize((size_t)size + 64, 0);
     DictState ds;
-    if (raw) dt_raw_dict_state(ds, size); else dict_load(b.data(), size, ds, wk, fs, slot, norm, next);
-    enc.assign((enc_dict_bytes(ds.err ? 0 : ds.contentSize) + 15) / 16, uint4{});
-    enc_dict_prepare(b.data(), size, ds, reinterpret_cast<EncDict*>(enc.data()), wk, fs, slot, tableSymbol.data());
+    if (raw) dt_raw_dict_state(ds, size); else dict_load_host(bytes, size, ds);
+    enc = enc_dict_block(bytes, size, ds);
     const size_t bytesNeeded = enc.size() * sizeof(uint4);
     if (bytesNeeded > encCap) { cudaError_t e = mem.get(&dEnc, bytesNeeded); if (e) return e; encCap = bytesNeeded; }
     cudaError_t e = cudaMemcpyAsync(dEnc, enc.data(), bytesNeeded, cudaMemcpyHostToDevice, st);
@@ -263,14 +257,13 @@ u32 dt_train_run(DtDevice& dv, u8* dict, u32 capacity, const u8* samples, const 
     }
     return true;
   };
-  u64* hSrcOff = (u64*)dv.h_desc;
   const u32 nFinal = (u32)((u64)nbTrain * dt_accel_finalize(accel) / 100);
   std::vector<std::pair<u32, u32>> finalSubs, testSubs;
   auto firstBlock = [&](u32 i) -> size_t { return std::min<u32>(sizes[i], BLOCKSIZE_MAX); };
   if (!cut(0, nFinal, firstBlock, [](u32) { return (size_t)0; }, finalSubs)) { err = "a sample does not fit max_batch_bytes"; return zerr(ZE_GENERIC); }
   u32 testMax = 0;
   for (u32 i = nbTrain; i < n; i++) testMax = std::max(testMax, sizes[i]);
-  if (!k0 && !cut(nbTrain, (u32)n, [&](u32 i) { return (size_t)sizes[i]; }, [&](u32 i) { return a16(encode_bound(sizes[i])); }, testSubs)) {
+  if (!k0 && !cut(nbTrain, (u32)n, [&](u32 i) { return (size_t)sizes[i]; }, [&](u32 i) { return align_up(encode_bound(sizes[i]), 16); }, testSubs)) {
     err = "a test sample is larger than the context's max_batch_bytes"; return zerr(ZE_GENERIC);
   }
   std::vector<u8> out(capacity), best;
@@ -282,15 +275,13 @@ u32 dt_train_run(DtDevice& dv, u8* dict, u32 capacity, const u8* samples, const 
     DTCK(cudaMemsetAsync(dStats, 0, sizeof(DtStats), st));
     for (auto& sb : finalSubs) {
       const u32 m = sb.second - sb.first;
-      u64* so = hSrcOff; u32* ss = (u32*)(so + m);
+      const DescView h(dv.h_desc, m);   // no destinations: dstOff / dstCap are left as they are and not read
       u32 mx = 0;
-      for (u32 q = 0; q < m; q++) { so[q] = off[sb.first + q] - off[sb.first]; ss[q] = (u32)firstBlock(sb.first + q); mx = std::max(mx, ss[q]); }
-      DTCK(cudaMemcpyAsync(dv.d_desc, dv.h_desc, (size_t)m * 12, cudaMemcpyHostToDevice, st));
-      EncodeArgs ea{dSamples + off[sb.first], (const u64*)dv.d_desc, (const u32*)(dv.d_desc + (size_t)m * 8), nullptr, nullptr, nullptr,
-                    nullptr, m, 0, level, 0, mx, ENC_EXCLUSIVE};
-      ea.dict = reinterpret_cast<const EncDict*>(dEnc);
+      for (u32 q = 0; q < m; q++) { h.srcOff[q] = off[sb.first + q] - off[sb.first]; h.srcSize[q] = (u32)firstBlock(sb.first + q); mx = std::max(mx, h.srcSize[q]); }
+      DTCK(cudaMemcpyAsync(dv.d_desc, dv.h_desc, DescView::bytes(m), cudaMemcpyHostToDevice, st));
+      const Items it = DescView(dv.d_desc, m).items(dSamples + off[sb.first], nullptr, nullptr);
       int nl = 0;
-      DTCK(encode_match_stats(ea, *dv.enc, st, dStats, &nl));
+      DTCK(encode_match_stats(encode_args(it, m, 0, level, 0, mx, ENC_EXCLUSIVE, dEnc, &enc), *dv.enc, st, dStats, &nl));
       dv.launches += nl;
       DTCK(cudaStreamSynchronize(st));   // the descriptors' pinned staging is rewritten by the next sub-batch
     }
@@ -306,20 +297,16 @@ u32 dt_train_run(DtDevice& dv, u8* dict, u32 capacity, const u8* samples, const 
       DTCK(upload(out.data(), size, false));
       for (auto& sb : testSubs) {
         const u32 m = sb.second - sb.first;
-        u64* so = hSrcOff; u64* dof = so + m; u32* ss = (u32*)(dof + m); u32* dc = ss + m;
+        const DescView h(dv.h_desc, m);
         size_t o = 0;
         for (u32 q = 0; q < m; q++) {
           const u32 i = sb.first + q;
-          so[q] = off[i] - off[sb.first]; ss[q] = sizes[i]; dc[q] = (u32)encode_bound(sizes[i]); dof[q] = o; o += a16(dc[q]);
+          h.srcOff[q] = off[i] - off[sb.first]; h.srcSize[q] = sizes[i]; h.dstCap[q] = (u32)encode_bound(sizes[i]); h.dstOff[q] = o; o += align_up(h.dstCap[q], 16);
         }
-        DTCK(cudaMemcpyAsync(dv.d_desc, dv.h_desc, (size_t)m * 24, cudaMemcpyHostToDevice, st));
-        EncodeArgs ea{dSamples + off[sb.first], (const u64*)dv.d_desc, (const u32*)(dv.d_desc + (size_t)m * 16), dv.d_dst,
-                      (const u64*)(dv.d_desc + (size_t)m * 8), (const u32*)(dv.d_desc + (size_t)m * 20), dv.d_result, m, 0, level, 0,
-                      testMax, ENC_EXCLUSIVE};
-        const EncDict* hed = reinterpret_cast<const EncDict*>(enc.data());
-        ea.dict = reinterpret_cast<const EncDict*>(dEnc); ea.dict_id = hed->dictID; ea.dict_err = hed->err;
+        DTCK(cudaMemcpyAsync(dv.d_desc, dv.h_desc, DescView::bytes(m), cudaMemcpyHostToDevice, st));
+        const Items it = DescView(dv.d_desc, m).items(dSamples + off[sb.first], dv.d_dst, dv.d_result);
         int nl = 0;
-        DTCK(encode_launch(ea, *dv.enc, st, &nl));
+        DTCK(encode_launch(encode_args(it, m, 0, level, 0, testMax, ENC_EXCLUSIVE, dEnc, &enc), *dv.enc, st, &nl));
         dv.launches += nl;
         DTCK(cudaMemcpyAsync(dv.h_result, dv.d_result, (size_t)m * 4, cudaMemcpyDeviceToHost, st));
         DTCK(cudaStreamSynchronize(st));

@@ -21,7 +21,6 @@
 #include "zb_encode.cuh"
 #include "xxh_device.cuh"
 #include <stdio.h>
-#include <stdlib.h>
 
 namespace zb {
 
@@ -665,6 +664,33 @@ __global__ void __launch_bounds__(128) k_enc_xxh(EncodeArgs a) {
   }
 }
 
+EncodeArgs encode_args(const Items& it, size_t n, u32 item_base, int level, int checksum, u32 max_src_size, u32 slot,
+                       const void* dict, const std::vector<uint4>* h_dict) {
+  EncodeArgs a{};
+  a.src_base = it.src; a.src_off = it.srcOff; a.src_size = it.srcSize;
+  a.dst_base = it.dst; a.dst_off = it.dstOff; a.dst_cap = it.dstCap; a.result = it.result;
+  a.n = (u32)n; a.item_base = item_base; a.level = level; a.checksum = checksum; a.max_src_size = max_src_size; a.stream_slot = slot;
+  if (dict) {
+    const EncDict* h = reinterpret_cast<const EncDict*>(h_dict->data());
+    a.dict = reinterpret_cast<const EncDict*>(dict); a.dict_id = h->dictID; a.dict_err = h->err;
+  }
+  return a;
+}
+
+void dict_load_host(const u8* dict, u32 size, DictState& ds) {
+  std::vector<u8> b(dict, dict + size); b.resize((size_t)size + 64, 0);   // the parser may read 64 bytes past the end
+  HufBuildWk wk; HufFseScratch fs; u8 slot[260]; s16 norm[64]; u16 next[64];
+  dict_load(b.data(), size, ds, wk, fs, slot, norm, next);
+}
+
+std::vector<uint4> enc_dict_block(const u8* dict, u32 size, const DictState& ds) {
+  std::vector<u8> b(dict, dict + size); b.resize((size_t)size + 64, 0);
+  std::vector<uint4> out((enc_dict_bytes(ds.err ? 0 : ds.contentSize) + 15) / 16, uint4{});
+  HufBuildWk wk; HufFseScratch fs; u8 slot[260]; std::vector<u8> tableSymbol(512);
+  enc_dict_prepare(b.data(), size, ds, reinterpret_cast<EncDict*>(out.data()), wk, fs, slot, tableSymbol.data());
+  return out;
+}
+
 size_t encode_bound(size_t srcSize) { return srcSize + (srcSize >> 8) + 32 + 3 * ((srcSize >> 17) + 1); }
 
 // Entropy-stage work areas ("slots", one per resident warp).  A launch that owns the context (device-pointer path)
@@ -716,32 +742,27 @@ const char* const kEncodeKernelNames[ENCODE_KERNELS] = {"k_enc_match", "k_enc_en
 static void match_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, cudaEvent_t* marks) {
   // match stage: table sizes per level (u16 entries)
   const bool dfast = a.level >= 3;
-  static const int envLog = getenv("ZSTDB200_ENC_HLOG") ? atoi(getenv("ZSTDB200_ENC_HLOG")) : 0;       // tuning aids
-  static const int envPerSm = getenv("ZSTDB200_ENC_PERSM") ? atoi(getenv("ZSTDB200_ENC_PERSM")) : 0;
   // level 1: 2^12 (8 KB), level 2: 2^13 (16 KB), level 3: 2^11 long + 2^12 short (12 KB); chunks above 128 KiB: enc_hlog_*.
   // The sizes date from the shared-memory placement (24 / 12 / 16 warps per SM) and are kept: the ratio band is tested
   // with them (lock-step emulation in tests/hostsim: tick records within -2.4 % of libzstd at 128 KiB chunks, log text
   // gains ratio with the smaller tables) and 32 warps' tables still mostly fit L1.
   const bool big = a.max_src_size > BLOCKSIZE_MAX;
-  const u32 hlogL = envLog ? (u32)envLog : enc_hlog_long(a.level, big), hlogS = envLog ? (u32)envLog - 1 : enc_hlog_short(a.level, big), mls = a.level <= 1 ? 6 : 5;
+  const u32 hlogL = enc_hlog_long(a.level, big), hlogS = enc_hlog_short(a.level, big), mls = a.level <= 1 ? 6 : 5;
   const size_t smem = ((size_t)(1u << hlogL) + (dfast ? (1u << hlogS) : 0)) * 2;
-  const u32 capSm = envPerSm ? (u32)envPerSm : 32;
-  u32 perSm = (u32)((220 * 1024) / (smem + 1024)); if (perSm > capSm) perSm = capSm;
+  u32 perSm = (u32)((220 * 1024) / (smem + 1024)); if (perSm > 32) perSm = 32;
   const u64 units = (u64)a.n * (a.max_src_size > BLOCKSIZE_MAX ? (a.max_src_size + BLOCKSIZE_MAX - 1) / BLOCKSIZE_MAX : 1);
   u32 grid = (u32)s.sms * perSm; if (grid > units) grid = (u32)units;
   const bool exclusive = a.stream_slot == ENC_EXCLUSIVE;
-  // Match tables in global scratch when the launch has the device to itself (ZSTDB200_ENC_GTAB=0: always in shared memory,
-  // for A/B runs).  Slices of a host batch run concurrently on several streams, and the entropy stage of one slice then
-  // shares SMs with the match stage of another: its 34 KB of shared memory per CTA shrink the L1 the tables would live in
-  // (measured: host-path level 1 19.1 -> 16.4 GB/s with global tables), so those launches keep their tables in shared memory.
-  static const bool envGtab = !getenv("ZSTDB200_ENC_GTAB") || atoi(getenv("ZSTDB200_ENC_GTAB")) != 0;
+  // Match tables in global scratch when the launch has the device to itself.  Slices of a host batch run concurrently on
+  // several streams, and the entropy stage of one slice then shares SMs with the match stage of another: its 34 KB of shared
+  // memory per CTA shrink the L1 the tables would live in (measured: host-path level 1 19.1 -> 16.4 GB/s with global tables),
+  // so those launches keep their tables in shared memory.
   u16* gtab = nullptr;
-  if (envGtab && exclusive && smem <= kGtabStride) {
-    const u32 wps = envPerSm ? (envPerSm < (int)kGtabWarpsPerSm ? (u32)envPerSm : kGtabWarpsPerSm) : kGtabWarpsPerSm;
+  if (exclusive && smem <= kGtabStride) {
     if (!s.gtab && cudaMalloc(&s.gtab, (size_t)s.sms * kGtabWarpsPerSm * kGtabStride) != cudaSuccess) {
       cudaGetLastError(); s.gtab = nullptr;                      // no room for the 113 MB: this launch keeps shared-memory tables
     }
-    if (s.gtab) { gtab = (u16*)s.gtab; grid = (u32)s.sms * wps; if (grid > units) grid = (u32)units; }
+    if (s.gtab) { gtab = (u16*)s.gtab; grid = (u32)s.sms * kGtabWarpsPerSm; if (grid > units) grid = (u32)units; }
   }
   if (marks) cudaEventRecord(marks[0], st);
   const size_t sm = gtab ? 0 : smem;

@@ -1,11 +1,14 @@
 // encode_kernels.cuh — launch interface of the encoder kernels (encode_kernels.cu).
 #pragma once
 #include <cuda_runtime.h>
+#include <vector>
+#include "host_plan.h"
 #include "zb_common.cuh"
 
 namespace zb {
 
 struct EncDict;
+struct DictState;
 
 // All pointers are device pointers.  Item i: src_base[src_off[i] .. +src_size[i]) -> one zstd frame written at
 // dst_base[dst_off[i] ..] (at most dst_cap[i] bytes); result[i] = frame size or an error code.
@@ -39,6 +42,15 @@ struct EncodeScratch {
   int sms = 148;
   u32 entWarps = 0;       // entropy-stage warps resident on the device at once (set with the arenas)
 };
+
+// The arguments of one launch over n items, numbered from item_base in the scratch, on stream slot `slot` (or ENC_EXCLUSIVE).
+// dict: a block of enc_dict_block on the device, h_dict its host copy (for the id and error the launch carries); null: none.
+EncodeArgs encode_args(const Items& it, size_t n, u32 item_base, int level, int checksum, u32 max_src_size, u32 slot,
+                       const void* dict = nullptr, const std::vector<uint4>* h_dict = nullptr);
+// dict_load on the host: what k_dict computes on the device (zb_format.cuh)
+void dict_load_host(const u8* dict, u32 size, DictState& ds);
+// The encoder's block of a dictionary (zb_encode.cuh EncDict, enc_dict_prepare) from its bytes and their DictState
+std::vector<uint4> enc_dict_block(const u8* dict, u32 size, const DictState& ds);
 
 size_t encode_bound(size_t srcSize);
 cudaError_t encode_alloc(EncodeScratch& s, size_t maxBatchBytes, size_t maxItems);   // records sizes; memory comes lazily
