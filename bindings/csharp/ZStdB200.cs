@@ -131,7 +131,8 @@ namespace EPAM.Deltix.ZStd
                 return Native.zstdb200_compress(Native.Ctx(), level, checksum ? 1 : 0, d, (uint)dst.Length, s, (uint)src.Length);
         }
 
-        // one frame per segment; levels 1-3 (fast / double-fast match finder), XXH64 content checksum on request
+        // one frame per segment; levels 1-3 (fast / double-fast match finder) or -7..-1 (libzstd's fast negative levels: faster,
+        // larger, literals stored raw), XXH64 content checksum on request
         public static void Compress(IReadOnlyList<ArraySegment<byte>> srcs, IReadOnlyList<ArraySegment<byte>> dsts, uint[] results, int level = 3, bool checksum = true)
         {
             IntPtr c = Native.Ctx();

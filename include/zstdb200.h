@@ -84,8 +84,10 @@ int zstdb200_decompress_batch_device(zstdb200_ctx* ctx, int device_index,
                                      uint32_t* result, size_t n, void* stream);
 
 /* Compression (no reference counterpart exists: epam/Zstandard ships no compressor, SURVEY.md §0 F1; the
- * signatures mirror the decompress side).  level 1..3; checksum != 0 appends the XXH64 content checksum.
- * Frames are standard zstd frames accepted by the reference decoder. */
+ * signatures mirror the decompress side).  level 1..3, or -7..-1: libzstd's fast negative levels
+ * (ZSTD_c_compressionLevel = -N, zstd --fast=N), faster and larger, with literals stored raw; any other level is a batch-level
+ * failure.  checksum != 0 appends the XXH64 content checksum.  Frames are standard zstd frames accepted by the reference
+ * decoder. */
 size_t zstdb200_compress_bound(size_t srcSize);
 uint32_t zstdb200_compress(zstdb200_ctx* ctx, int level, int checksum, void* dst, uint32_t dstCapacity, const void* src, uint32_t srcSize);
 int zstdb200_compress_batch(zstdb200_ctx* ctx, int level, int checksum,
@@ -101,8 +103,8 @@ int zstdb200_compress_batch_device(zstdb200_ctx* ctx, int device_index, int leve
                                    void* dst_base, const uint64_t* dst_off, const uint32_t* dst_cap,
                                    uint32_t* result, size_t n, void* stream);
 
-/* The same three calls with the context's dictionary (the one zstdb200_load_dictionary loaded; same arguments and contracts as
- * the call each mirrors).  Frames name the dictionary's id in their header (a raw-content dictionary has id 0 and none is
+/* The same three calls with the context's dictionary (the one zstdb200_load_dictionary loaded; same arguments, levels 1..3 and
+ * -7..-1, and contracts as the call each mirrors).  Frames name the dictionary's id in their header (a raw-content dictionary has id 0 and none is
  * written), match against its content and start from its repeat offsets; they decode with that dictionary
  * (zstdb200_decompress*, libzstd's ZSTD_decompress_usingDict).  With no dictionary loaded the call fails at batch level
  * (non-zero, or GENERIC for zstdb200_compress_using_dict; zstdb200_last_error says why); when the dictionary's entropy

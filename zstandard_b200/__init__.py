@@ -227,10 +227,12 @@ class Context:
         return self._batch(self._lib.zstdb200_decompress_batch, (), srcs, dsts)
 
     def compress_batch(self, srcs, dsts, level=3, checksum=True):
+        """One zstd frame of srcs[i] into the writable buffer dsts[i]; returns np.uint32 result codes.  level: 1..3, or -7..-1
+        (libzstd's fast negative levels: faster and larger, literals stored raw); any other level raises."""
         return self._batch(self._lib.zstdb200_compress_batch, (int(level), 1 if checksum else 0), srcs, dsts)
 
     def compress_batch_using_dict(self, srcs, dsts, level=3, checksum=True):
-        """compress_batch with the dictionary of load_dictionary (raises when none is loaded)."""
+        """compress_batch with the dictionary of load_dictionary (raises when none is loaded); the same levels."""
         return self._batch(self._lib.zstdb200_compress_batch_using_dict, (int(level), 1 if checksum else 0), srcs, dsts)
 
     # ---- device-pointer batches (raw addresses, e.g. torch .data_ptr()) -----------------------
@@ -358,6 +360,7 @@ class ZStdCompress:
 
     @staticmethod
     def Compress(dst, src, level=3, checksum=True):
+        """One frame into dst; the frame size or an error code (GENERIC for a level outside 1..3 and -7..-1)."""
         dv, sv = _as_u8(dst, writable=True), _as_u8(src)
         ctx = default_context()
         return int(load_library().zstdb200_compress(ctx.handle, int(level), 1 if checksum else 0, dv.ctypes.data if dv.size else None,

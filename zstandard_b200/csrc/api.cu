@@ -424,13 +424,17 @@ int run_host_batch(zstdb200_ctx* ctx, const Job& j0, size_t n, bool clamp = true
   return 0;
 }
 
+// Compression levels: 1..3, and -7..-1 (libzstd's fast negative levels, acceleration = -level)
+static bool level_ok(int level) { return (level >= 1 && level <= 3) || (level >= -7 && level <= -1); }
+static const char* const kLevelError = "level must be 1..3 or -7..-1";
+
 // The checks every device-pointer entry point starts with (compress: the level and a loaded dictionary too); then the device
 // is selected.  *st: the caller's stream, or the device's first one.
 int device_call(zstdb200_ctx* ctx, Op op, int device_index, size_t n, int level, bool useDict, void* stream, Device** d, cudaStream_t* st) {
   if (!ctx) return 1;
   ctx->err.clear();
   if (device_index < 0 || device_index >= (int)ctx->dev.size()) { ctx->err = "bad device_index"; return 1; }
-  if (op == Op::Compress && (level < 1 || level > 3)) { ctx->err = "level must be 1..3"; return 1; }
+  if (op == Op::Compress && !level_ok(level)) { ctx->err = kLevelError; return 1; }
   if (n > ctx->maxItems) { ctx->err = "n exceeds zstdb200_max_items"; return 1; }
   if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
   *d = &ctx->dev[device_index];
@@ -600,7 +604,7 @@ static int compress_batch(zstdb200_ctx* ctx, int level, int checksum, const void
                           void* const* dst, const uint32_t* dstCap, uint32_t* result, size_t n, bool useDict) {
   if (!ctx) return 1;
   ctx->err.clear();
-  if (level < 1 || level > 3) { ctx->err = "level must be 1..3"; return 1; }
+  if (!level_ok(level)) { ctx->err = kLevelError; return 1; }
   if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
   Job j{Op::Compress, level, checksum, src, srcSize, dst, dstCap, result, nullptr, 0, useDict};
   return run_host_batch(ctx, j, n);

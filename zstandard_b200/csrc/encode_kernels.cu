@@ -1,6 +1,6 @@
 // encode_kernels.cu — sm_100a kernels of the batched zstd frame encoder.
 //
-//   k_enc_match<DFAST, DICT>             (DICT: also against the context's dictionary, see the kernel)
+//   k_enc_match<DFAST, DICT, ACCEL>      (DICT: also against the context's dictionary; ACCEL: the negative levels; see the kernel)
 //                      : warp / block    match finder: 32 consecutive (or strided) positions per step, one per lane;
 //                                        position hash table(s) of u16 entries in per-warp global scratch (L1 / L2
 //                                        resident; 32 one-warp CTAs per SM) or, for the concurrent slices of a host
@@ -86,7 +86,9 @@ __device__ __forceinline__ u32 warp_extend_ref(const u8* src, const u8* ref, u32
 // lane whose position found no match in the chunk's own tables, in libzstd's dictMatchState order: chunk long, dictionary
 // long, chunk short, dictionary short.  A dictionary match ends at the end of the content, its offset reaches back over
 // the chunk into the content, and the first block starts from the dictionary's repeat offsets.
-template <bool DFAST, bool DICT>
+// ACCEL: a negative level, acceleration -a.level (never with DFAST).  The lanes probe libzstd's pairs of adjacent positions
+// with a stride of 1 + acceleration (zb_encode.cuh enc_probe_off), so a window covers 16 strides instead of 32 positions.
+template <bool DFAST, bool DICT, bool ACCEL>
 __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc, u32 hlogL, u32 hlogS, u32 mls, u16* gtab) {
   extern __shared__ __align__(16) u16 tabShared[];
   const u32 lane = threadIdx.x, warp = blockIdx.x, nWarps = gridDim.x;
@@ -157,9 +159,9 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
         // window's table lookups and candidate loads run speculatively behind it: one memory round trip instead of two.
         bool fresh = false;
         while (p0 < ilimit || (fresh && p0 == ilimit)) {
-          const u32 step = 1 + ((p0 - anchor) >> 8);                 // skim incompressible runs
+          const u32 step = (ACCEL ? 1u - (u32)a.level : 1u) + ((p0 - anchor) >> 8);   // skim incompressible runs
           if (lane < 4) prefetch_line(src + p0 + 384 + 128 * lane);   // the source streams in from HBM: keep ~4 lines ahead in L1
-          const u32 p = p0 + lane * step;
+          const u32 p = p0 + enc_probe_off(ACCEL, lane, step);
           const bool act = p < ilimit;
           u32 r2a = 0, r2b = 1;
           if (fresh && rep2 != 0 && (!DICT || rep2 <= p0)) { r2a = ldu32(src + p0); r2b = ldu32(src + p0 - rep2); }   // (without a
@@ -170,14 +172,14 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
           const unsigned mL = __match_any_sync(FULLMASK, hL);
           const unsigned lowL = mL & ((1u << lane) - 1);
           u32 candL; bool validL;
-          if (lowL) { candL = p0 + (31 - __clz(lowL)) * step; validL = act; } else validL = cand_from_entry(p, eL, candL) && act;
+          if (lowL) { candL = p0 + enc_probe_off(ACCEL, 31 - __clz(lowL), step); validL = act; } else validL = cand_from_entry(p, eL, candL) && act;
           u32 hS = 0, candS = 0; bool validS = false; unsigned mS = 0;
           if (DFAST) {
             hS = act ? hash64(v, hlogS, mls) : (0x80000000u | lane);
             const u32 eS = act ? tabS[hS] : 0;
             mS = __match_any_sync(FULLMASK, hS);
             const unsigned lowS = mS & ((1u << lane) - 1);
-            if (lowS) { candS = p0 + (31 - __clz(lowS)) * step; validS = act; } else validS = cand_from_entry(p, eS, candS) && act;
+            if (lowS) { candS = p0 + enc_probe_off(ACCEL, 31 - __clz(lowS), step); validS = act; } else validS = cand_from_entry(p, eS, candS) && act;
           }
           bool okL = false, okS = false;
           if (validL) okL = DFAST ? (ldu64(src + candL) == v) : (ldu32(src + candL) == (u32)v);
@@ -191,7 +193,8 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
             candDS = dtabS[hash64(v, ENC_DICT_HLOG, mls)];
             if (candDS != ENC_DICT_EMPTY) okDS = ldu32(dc + candDS) == (u32)v;
           }
-          const bool rok = act && rep1 != 0 && rep1 <= p && ldu32(src + p - rep1) == (u32)v;
+          // (ACCEL: the repeat offset is tried at the start of every probe pair but the first, libzstd's ip2)
+          const bool rok = act && (!ACCEL || (lane != 0 && !(lane & 1))) && rep1 != 0 && rep1 <= p && ldu32(src + p - rep1) == (u32)v;
           if (fresh) {
             fresh = false;
             if (r2a == r2b) {                                                      // uniform over the warp
@@ -211,17 +214,27 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
             }
           }
           const unsigned fRep = __ballot_sync(FULLMASK, rok);
-          const unsigned found = __ballot_sync(FULLMASK, okL | okS | okDL | okDS) | fRep;
+          const unsigned fTab = __ballot_sync(FULLMASK, okL | okS | okDL | okDS);
+          const unsigned found = fTab | fRep;
           if (!found) {                                                // no match in the window: enter every position, move on
             if (act && (mL >> lane) == 1) tabL[hL] = (u16)p;          // the last position of each hash group is the one kept
             if (DFAST && act && (mS >> lane) == 1) tabS[hS] = (u16)p;
             __syncwarp();
-            p0 += 32 * step; continue;
+            p0 += (ACCEL ? 16 : 32) * step; continue;
           }
-          u32 fl = (u32)__ffs(found) - 1;
-          // a repeat-offset match up to 3 positions further on beats a table match here (it is cheaper to code)
-          if (!((fRep >> fl) & 1)) { const unsigned nearRep = fRep & (0xEu << fl); if (nearRep) fl = (u32)__ffs(nearRep) - 1; }
-          u32 pos = p0 + fl * step;
+          u32 fl = (u32)__ffs(found) - 1, probe = 0;
+          if (ACCEL) {
+            // libzstd's order over the pairs: for pair k the repeat offset at the next pair's start (lane 2k + 2) first, then
+            // the table at lane 2k, then at 2k + 1.  probe: where libzstd's current0 is (the fill after the match).
+            const unsigned repPair = fRep >> 2;
+            const u32 b = (u32)__ffs(repPair | fTab) - 1;
+            fl = ((repPair >> b) & 1) ? b + 2 : b;
+            probe = p0 + enc_probe_off(true, b, step);
+          } else if (!((fRep >> fl) & 1)) {
+            // a repeat-offset match up to 3 positions further on beats a table match here (it is cheaper to code)
+            const unsigned nearRep = fRep & (0xEu << fl); if (nearRep) fl = (u32)__ffs(nearRep) - 1;
+          }
+          u32 pos = p0 + enc_probe_off(ACCEL, fl, step);
           // at the winning lane: repeat offset > long/main table > (dictionary long) > short table (> dictionary short)
           const u32 kind = rok ? 0 : (okL ? 1 : (DICT ? (okDL ? 3 : (okS ? 2 : 4)) : 2));
           const u32 kf = __shfl_sync(FULLMASK, kind, fl);
@@ -275,6 +288,10 @@ __global__ void __launch_bounds__(32) k_enc_match(EncodeArgs a, EncodeScratch sc
           nlits += ll; nseq++;
           anchor = pos + mlen; p0 = anchor;
           if (p0 <= ilimit) {
+            if (ACCEL) {              // libzstd's fill: the positions 2 past current0 (probe) and 2 before the match end
+              if (lane == 0) { tabL[hash64(ldu64(src + probe + 2), hlogL, mls)] = (u16)(probe + 2); tabL[hash64(ldu64(src + p0 - 2), hlogL, mls)] = (u16)(p0 - 2); }
+              __syncwarp();
+            }
             fresh = true;                                              // immediate-repeat test at the top of the next pass
           }
         }
@@ -331,8 +348,9 @@ __device__ __forceinline__ u32 wmax(u32 v) {
   return v;
 }
 
-// literals section; returns bytes written, 0 = no room (mirror of enc_literals; ed likewise: the dictionary for the first block)
-__device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWarp& w, u8* tmp, u32 lane, const EncDict* ed) {
+// literals section; returns bytes written, 0 = no room (mirror of enc_literals; ed likewise: the dictionary for the first block).
+// rawOnly (the negative levels): always raw, as libzstd's fast strategy with a non-zero targetLength
+__device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWarp& w, u8* tmp, u32 lane, const EncDict* ed, bool rawOnly) {
   const u32 rawLh = n < 32 ? 1 : (n < 4096 ? 2 : 3);
   auto raw = [&]() -> u32 {
     if (rawLh + n > cap) return 0;
@@ -344,7 +362,7 @@ __device__ u32 warp_enc_literals(u8* out, u32 cap, const u8* lits, u32 n, EntWar
     __syncwarp();
     return rawLh + n;
   };
-  if (n < 64) return raw();
+  if (n < 64 || rawOnly) return raw();
   for (u32 i = lane; i < 256; i += 32) w.hist[i] = 0;
   __syncwarp();
   for (u32 i = lane; i < n; i += 32) atomicAdd(&w.hist[lits[i]], 1u);
@@ -623,7 +641,7 @@ __global__ void __launch_bounds__(128) k_enc_entropy(EncodeArgs a, EncodeScratch
           if (room > avail) room = avail;
           u8* body = dst + op + 3;
           const EncDict* const edb = DICT && blk == 0 && a.dict->hasEntropy ? a.dict : nullptr;   // (as encode_frame_with)
-          const u32 l = warp_enc_literals(body, room, st.lits, st.nlits, w, tmp, lane, edb);
+          const u32 l = warp_enc_literals(body, room, st.lits, st.nlits, w, tmp, lane, edb, a.level < 0);
           if (l) {
             const u32 sq = warp_enc_sequences(body + l, room - l, st, codes, w, lut, a.level, lane, edb);
             if (sq && l + sq < bsize) { csize = l + sq; compressed = true; }
@@ -729,10 +747,12 @@ static cudaError_t encode_lazy_alloc(EncodeScratch& s) {
   if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_enc_entropy<false>, 128, 0) != cudaSuccess || nb < 1) nb = 4;
   s.entWarps = (u32)(s.sms * nb * 4);
   if (s.entWarps > kSlotsExclusive) s.entWarps = kSlotsExclusive;
-  cudaFuncSetAttribute(k_enc_match<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-  cudaFuncSetAttribute(k_enc_match<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-  cudaFuncSetAttribute(k_enc_match<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
-  cudaFuncSetAttribute(k_enc_match<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+  cudaFuncSetAttribute(k_enc_match<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(k_enc_match<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+  cudaFuncSetAttribute(k_enc_match<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(k_enc_match<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+  cudaFuncSetAttribute(k_enc_match<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
+  cudaFuncSetAttribute(k_enc_match<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024);
   return cudaSuccess;
 }
 
@@ -741,13 +761,14 @@ const char* const kEncodeKernelNames[ENCODE_KERNELS] = {"k_enc_match", "k_enc_en
 // The match stage of one launch (k_enc_match): table sizes, grid and table placement.  marks: as for encode_launch.
 static void match_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st, cudaEvent_t* marks) {
   // match stage: table sizes per level (u16 entries)
-  const bool dfast = a.level >= 3;
-  // level 1: 2^12 (8 KB), level 2: 2^13 (16 KB), level 3: 2^11 long + 2^12 short (12 KB); chunks above 128 KiB: enc_hlog_*.
+  const bool dfast = a.level >= 3, accel = a.level < 0;
+  // level 1 and the negative levels: 2^12 (8 KB), level 2: 2^13 (16 KB), level 3: 2^11 long + 2^12 short (12 KB); chunks
+  // above 128 KiB: enc_hlog_*.
   // The sizes date from the shared-memory placement (24 / 12 / 16 warps per SM) and are kept: the ratio band is tested
   // with them (lock-step emulation in tests/hostsim: tick records within -2.4 % of libzstd at 128 KiB chunks, log text
   // gains ratio with the smaller tables) and 32 warps' tables still mostly fit L1.
   const bool big = a.max_src_size > BLOCKSIZE_MAX;
-  const u32 hlogL = enc_hlog_long(a.level, big), hlogS = enc_hlog_short(a.level, big), mls = a.level <= 1 ? 6 : 5;
+  const u32 hlogL = enc_hlog_long(a.level, big), hlogS = enc_hlog_short(a.level, big), mls = enc_mls(a.level);
   const size_t smem = ((size_t)(1u << hlogL) + (dfast ? (1u << hlogS) : 0)) * 2;
   u32 perSm = (u32)((220 * 1024) / (smem + 1024)); if (perSm > 32) perSm = 32;
   const u64 units = (u64)a.n * (a.max_src_size > BLOCKSIZE_MAX ? (a.max_src_size + BLOCKSIZE_MAX - 1) / BLOCKSIZE_MAX : 1);
@@ -767,11 +788,13 @@ static void match_launch(const EncodeArgs& a, EncodeScratch& s, cudaStream_t st,
   if (marks) cudaEventRecord(marks[0], st);
   const size_t sm = gtab ? 0 : smem;
   if (a.dict) {
-    if (dfast) k_enc_match<true, true><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
-    else k_enc_match<false, true><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    if (dfast) k_enc_match<true, true, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    else if (accel) k_enc_match<false, true, true><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    else k_enc_match<false, true, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
   } else {
-    if (dfast) k_enc_match<true, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
-    else k_enc_match<false, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    if (dfast) k_enc_match<true, false, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    else if (accel) k_enc_match<false, false, true><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
+    else k_enc_match<false, false, false><<<grid, 32, sm, st>>>(a, s, hlogL, hlogS, mls, gtab);
   }
 }
 

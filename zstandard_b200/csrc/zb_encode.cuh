@@ -1,4 +1,4 @@
-// zb_encode.cuh — per-thread body of the GPU zstd frame encoder (levels 1-3).
+// zb_encode.cuh — per-thread body of the GPU zstd frame encoder (levels 1-3 and -7..-1).
 //
 // The reference repository ships no compressor (SURVEY.md §0 F1): what binds this code is the reference
 // *decoder's* accept set — every structure written here is one that csharp/src/ZStdDecompress.cs,
@@ -252,8 +252,16 @@ struct HufEnc { HufCode code[256]; u8 weight[256]; u32 maxSym; u32 tableLog; };
 // libzstd (tick records, level 1 at 256 KiB: -3.7 %, level 3 at 1 MiB: -4.1 %).  Level 1 then takes 2^13 entries (-2.0 %),
 // level 3 a short table of 2^13 beside a long one of 2^12 (-0.7 % / -2.4 %; 24 KB, which still leaves 9 one-warp CTAs per
 // SM: a GiB of 1 MiB chunks is 1 024 chunks and must not need a second wave).
+// The negative (fast) levels take level 1's sizes: 2^12 entries as libzstd's hashLog 12 up to 128 KiB, 2^13 above.
 ZB_HD u32 enc_hlog_long(int level, bool big) { return big ? (level >= 3 ? 12 : 13) : (level == 2 ? 13 : (level >= 3 ? 11 : 12)); }
 ZB_HD u32 enc_hlog_short(int /*level*/, bool big) { return big ? 13 : 12; }
+// Bytes the match stage's (short) hash covers: libzstd's minMatch, 6 at level 1, 5 at the negative levels (the ratio sweep
+// of profiles/fast_levels_mls_sweep.jsonl) and at levels 2 and 3.
+ZB_HD u32 enc_mls(int level) { return level == 1 ? 6 : 5; }
+// Offset from the window start of the position lane l probes.  Levels 1-3: l * step.  Negative levels (accel): libzstd's fast
+// loop, pairs of adjacent positions every `step` bytes, so lanes 2k and 2k + 1 probe k * step and k * step + 1; step starts at
+// 1 + acceleration, which at acceleration 1 is every position.
+ZB_HD u32 enc_probe_off(bool accel, u32 l, u32 step) { return accel ? (l >> 1) * step + (l & 1) : l * step; }
 
 struct HufBuildScratch { u32 nodeCount[512]; u16 parent[512]; u16 order[256]; u8 depth[512]; };
 
