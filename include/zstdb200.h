@@ -142,6 +142,72 @@ uint32_t zstdb200_train_dictionary(zstdb200_ctx* ctx, void* dictBuffer, uint32_t
                                    const void* samples, const uint32_t* sampleSizes, size_t nbSamples,
                                    zstdb200_train_params* params /* NULL = defaults; k and d chosen are written back */);
 
+/* Seekable archives (no reference counterpart; zstd's seekable format, contrib/seekable_format/
+ * zstd_seekable_compression_format.md in the zstd repository).  An archive is independent zstd frames back to back from
+ * byte 0, followed by a skippable frame (magic 0x184D2A5E) holding the seek table: per frame its Compressed_Size,
+ * Decompressed_Size and, when the descriptor's bit 7 is set, the low 32 bits of the XXH64 of its content; then
+ * Number_Of_Frames, the descriptor byte and 0x8F92EAB1.  Any zstd decoder reads such an archive (concatenated frames, the
+ * table skipped), zstdb200_decompress included; the calls below decode any byte range of it with the frames that cover the
+ * range as items of one batch. */
+typedef struct {
+  uint64_t content_size;        /* sum of Decompressed_Size */
+  uint64_t data_size;           /* bytes of the data frames (the archive without its seek table) */
+  uint32_t n_frames;
+  uint32_t checksums;           /* checksum flag of the descriptor */
+  uint32_t max_frame_content, max_frame_compressed;
+} zstdb200_seekable_info;
+
+/* Host-only: reads the footer and the table of the archive src[0..srcSize).  Returns 0, or an error code (nothing else is
+ * written): srcSize_wrong (shorter than 17 bytes; the table is longer than the archive), prefix_unknown (footer magic;
+ * skippable magic), corruption_detected (a reserved descriptor bit 6..2 set; Frame_Size does not match the frame count and
+ * entry size; the Compressed_Size values do not add up to exactly the bytes before the table).  Bits 1..0 are ignored. */
+uint32_t zstdb200_seekable_info_get(const void* src, uint64_t srcSize, zstdb200_seekable_info* info);
+
+/* Largest archive zstdb200_compress_seekable* writes for srcSize bytes in frames of frameSize (0 for frameSize 0). */
+uint64_t zstdb200_seekable_bound(uint64_t srcSize, uint32_t frameSize);
+
+/* Compresses src[0..srcSize) into one archive at dst and stores its size in *dstSize.  Frame i holds bytes
+ * [i * frameSize, min((i + 1) * frameSize, srcSize)) and is byte for byte what zstdb200_compress_batch writes for that chunk
+ * at the same level (1..3, -7..-1) and checksum.  checksum != 0: every frame carries its content checksum and the table the
+ * same 4 bytes, with the checksum flag set; checksum == 0: neither does.  srcSize == 0 gives the 17-byte table frame alone.
+ * Batch-level failures (non-zero, zstdb200_last_error), detected before any work starts: 1 <= frameSize <= max_batch_bytes
+ * does not hold, more frames than the table's 32-bit Frame_Size holds (357 913 940 with checksums, 536 870 910 without),
+ * dstCapacity < zstdb200_seekable_bound(srcSize, frameSize), a null pointer, a bad level.
+ * Host variant: any srcSize within that frame count, over the sub-batches and devices of zstdb200_compress_batch; each
+ * sub-batch's frames are packed on the device and cross PCIe once, back to back, into their final place (no per-frame
+ * spare capacity, no second pass over the output). */
+int zstdb200_compress_seekable(zstdb200_ctx* ctx, int level, int checksum, uint32_t frameSize,
+                               const void* src, uint64_t srcSize, void* dst, uint64_t dstCapacity, uint64_t* dstSize);
+/* Device variant: src, dst and dstSize are device pointers on device `devices[device_index]`.  Requires srcSize <=
+ * max_batch_bytes and a frame count <= zstdb200_max_items(ctx); the source is readable 8 bytes past its end.  The frames are
+ * encoded into the context's device staging, then packed with their table into dst (*dstSize is written on the device;
+ * 0 if a frame failed, which a capacity at the bound rules out).  The descriptors' upload synchronises `stream` once (as
+ * zstdb200_compress_batch_device does); everything else is enqueued on `stream` (NULL = the context's stream). */
+int zstdb200_compress_seekable_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, uint32_t frameSize,
+                                      const void* src, uint64_t srcSize, void* dst, uint64_t dstCapacity,
+                                      uint64_t* dstSize, void* stream);
+
+/* Decodes content bytes [offset, offset + length) of the archive src[0..srcSize) into dst[0..length); no byte of dst outside
+ * that range is written.  Only the frames that overlap the range are decoded, all as items of one batch (one launch
+ * sequence of the decode pipeline per arena-sized round, never one pass per frame).  Frames inside the range decode straight
+ * into dst; the first and last, when only part of them is in the range, decode into scratch and their in-range part is
+ * copied out.  *code: 0, or the first error in archive order — a table error (the codes of zstdb200_seekable_info_get);
+ * srcSize_wrong when the range ends past content_size (nothing is decoded); a frame's own decoder code; corruption_detected
+ * when a frame decodes to a size other than its Decompressed_Size; checksum_wrong when the table's checksum does not match
+ * (compared with the frame's own verified checksum when it has one, else with the XXH64 of its decoded bytes).  On an
+ * error code the range's bytes are unspecified.  Batch-level failure (non-zero): a selected frame larger than
+ * max_batch_bytes, a null pointer, a CUDA failure.  Host variant: host pointers; the plan runs through the host batch path
+ * (items are spans of the archive, checked on the device right after their decode). */
+int zstdb200_decompress_seekable(zstdb200_ctx* ctx, void* dst, uint64_t offset, uint64_t length,
+                                 const void* src, uint64_t srcSize, uint32_t* code);
+/* Device variant: dst, src and code are device pointers.  The footer and then the table are copied to the host (two small
+ * copies, two synchronisations of `stream`); after that the call only enqueues (a range whose frames exceed one descriptor
+ * upload of max_items frames waits for the previous upload's work once per further upload).  The queued work uses the
+ * context's staging and scratch on that device, so the next call on the context that needs them first waits for it; a
+ * caller never has to synchronise `stream` before making another call. */
+int zstdb200_decompress_seekable_device(zstdb200_ctx* ctx, int device_index, void* dst, uint64_t offset, uint64_t length,
+                                        const void* src, uint64_t srcSize, uint32_t* code, void* stream);
+
 /* Pinned host memory for src/dst buffers (lets the batch calls DMA straight from/to caller memory). */
 void* zstdb200_host_alloc(size_t bytes);
 void zstdb200_host_free(void* p);

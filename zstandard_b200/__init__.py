@@ -57,7 +57,30 @@ ABI = {
                                                         _c.POINTER(_c.c_float), _c.c_int]),
     "zstdb200_encode_kernel_name": (_c.c_char_p, [_c.c_int]),
     "zstdb200_train_dictionary": (_c.c_uint32, [_c.c_void_p, _c.c_void_p, _c.c_uint32, _c.c_void_p, _u32p, _c.c_size_t, _c.c_void_p]),
+    "zstdb200_seekable_info_get": (_c.c_uint32, [_c.c_void_p, _c.c_uint64, _c.c_void_p]),
+    "zstdb200_seekable_bound": (_c.c_uint64, [_c.c_uint64, _c.c_uint32]),
+    "zstdb200_compress_seekable": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_uint32, _c.c_void_p, _c.c_uint64, _c.c_void_p,
+                                              _c.c_uint64, _u64p]),
+    "zstdb200_compress_seekable_device": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_uint32, _c.c_void_p, _c.c_uint64,
+                                                     _c.c_void_p, _c.c_uint64, _c.c_void_p, _c.c_void_p]),
+    "zstdb200_decompress_seekable": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_uint64, _c.c_uint64, _c.c_void_p, _c.c_uint64, _u32p]),
+    "zstdb200_decompress_seekable_device": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_uint64, _c.c_uint64, _c.c_void_p,
+                                                       _c.c_uint64, _c.c_void_p, _c.c_void_p]),
 }
+
+
+class SeekableInfo(_c.Structure):
+    """zstdb200_seekable_info (include/zstdb200.h)."""
+    _fields_ = [("content_size", _c.c_uint64), ("data_size", _c.c_uint64), ("n_frames", _c.c_uint32), ("checksums", _c.c_uint32),
+                ("max_frame_content", _c.c_uint32), ("max_frame_compressed", _c.c_uint32)]
+
+
+class SeekableError(RuntimeError):
+    """A seekable archive's table or a frame of the decoded range failed (.code, in the library's encoding)."""
+
+    def __init__(self, code, message):
+        super().__init__(message)
+        self.code = code
 
 
 class TrainParams(_c.Structure):
@@ -234,6 +257,60 @@ class Context:
     def compress_batch_using_dict(self, srcs, dsts, level=3, checksum=True):
         """compress_batch with the dictionary of load_dictionary (raises when none is loaded); the same levels."""
         return self._batch(self._lib.zstdb200_compress_batch_using_dict, (int(level), 1 if checksum else 0), srcs, dsts)
+
+    # ---- seekable archives (zstd's seekable format) ----------------------------------------------
+    @staticmethod
+    def seekable_bound(size, frame_size):
+        """Largest archive compress_seekable writes for `size` bytes in frames of `frame_size`."""
+        return int(load_library().zstdb200_seekable_bound(int(size), int(frame_size)))
+
+    def compress_seekable(self, data, frame_size, level=3, checksum=True):
+        """One seekable archive of `data`: frames of `frame_size` bytes (each what compress_batch writes for its chunk) and
+        the seek table.  Returns bytes; raises on a batch-level failure."""
+        sv = _as_u8(data)
+        out = np.empty(max(self.seekable_bound(sv.size, frame_size), 1), dtype=np.uint8)
+        size = _c.c_uint64(0)
+        self._check("zstdb200_compress_seekable", self._lib.zstdb200_compress_seekable(
+            self._h, int(level), 1 if checksum else 0, int(frame_size), sv.ctypes.data if sv.size else None, sv.size, out.ctypes.data,
+            out.size, _c.byref(size)))
+        return out[:size.value].tobytes()
+
+    def seekable_info(self, archive):
+        """The archive's table summary (SeekableInfo); raises SeekableError on a malformed table."""
+        v = _as_u8(archive)
+        info = SeekableInfo()
+        r = int(self._lib.zstdb200_seekable_info_get(v.ctypes.data if v.size else None, v.size, _c.byref(info)))
+        if r:
+            raise SeekableError(r, "seekable table: " + error_name(r))
+        return info
+
+    def decompress_seekable(self, archive, offset=0, length=None, out=None):
+        """Content bytes [offset, offset + length) of the archive (length None: to the end).  Returns bytes, or fills the
+        writable buffer `out` of `length` bytes and returns it.  Raises SeekableError with the first error's code."""
+        v = _as_u8(archive)
+        if length is None:
+            length = max(int(self.seekable_info(v).content_size) - int(offset), 0)
+        dv = _as_u8(out, writable=True) if out is not None else np.empty(int(length), dtype=np.uint8)
+        if dv.size < length:
+            raise ValueError("out is smaller than length")
+        code = _c.c_uint32(0)
+        self._check("zstdb200_decompress_seekable", self._lib.zstdb200_decompress_seekable(
+            self._h, dv.ctypes.data if dv.size else None, int(offset), int(length), v.ctypes.data if v.size else None, v.size,
+            _c.byref(code)))
+        if code.value:
+            raise SeekableError(code.value, f"decompress_seekable: {error_name(code.value)}")
+        return out if out is not None else dv.tobytes()
+
+    def compress_seekable_device(self, level, checksum, frame_size, src, size, dst, capacity, dst_size, stream=0, device_index=0):
+        """Device pointers: src (size bytes, readable 8 bytes past the end) -> archive at dst; its size to the u64 at dst_size."""
+        self._check("zstdb200_compress_seekable_device", self._lib.zstdb200_compress_seekable_device(
+            self._h, device_index, int(level), 1 if checksum else 0, int(frame_size), src, int(size), dst, int(capacity), dst_size, stream))
+
+    def decompress_seekable_device(self, dst, offset, length, src, size, code, stream=0, device_index=0):
+        """Device pointers: content bytes [offset, offset + length) of the archive src (size bytes) to dst; the u32 at code gets 0
+        or the first error."""
+        self._check("zstdb200_decompress_seekable_device", self._lib.zstdb200_decompress_seekable_device(
+            self._h, device_index, dst, int(offset), int(length), src, int(size), code, stream))
 
     # ---- device-pointer batches (raw addresses, e.g. torch .data_ptr()) -----------------------
     def decompress_batch_device(self, src_base, src_off, src_size, dst_base, dst_off, dst_cap, result, n, stream=0, device_index=0):

@@ -6,7 +6,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libzstdb200.so")
-SOURCES = ["api.cu", "decode_kernels.cu", "encode_kernels.cu", "dict_train.cu"]
+SOURCES = ["api.cu", "decode_kernels.cu", "encode_kernels.cu", "dict_train.cu", "seekable_kernels.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC,-O2,-Wall", "-diag-suppress", "20091", "--cudart", "static",

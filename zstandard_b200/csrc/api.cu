@@ -15,6 +15,8 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <condition_variable>
+#include <mutex>
 #include <string>
 #include <thread>
 #include <vector>
@@ -24,6 +26,8 @@
 #include "dict_train.cuh"
 #include "encode_kernels.cuh"
 #include "host_plan.h"
+#include "seekable.h"
+#include "seekable_kernels.cuh"
 #include "zb_encode.cuh"
 
 using namespace zb;
@@ -45,6 +49,10 @@ struct Device {
   int id = 0;
   cudaStream_t stream[NSTREAMS] = {};
   cudaEvent_t descEv = nullptr;                 // descriptors of the current sub-batch are on the device
+  // Work that zstdb200_decompress_seekable_device left queued (it returns without synchronising) still reads the pinned
+  // h_desc / h_seek and the device's descriptors, arenas and scratch: every later call that writes them, from the CPU or on
+  // another stream, first waits for pendingEv (pending_wait).
+  cudaEvent_t pendingEv = nullptr; bool pending = false;
   std::vector<cudaEvent_t> sliceEv;             // "this slice's output is in the pinned staging" (grown on demand)
   // device memory
   u8 *d_src = nullptr, *d_dst = nullptr;       // staging for the host-pointer API
@@ -59,6 +67,7 @@ struct Device {
   u8* d_dict = nullptr; size_t dictCap = 0; DictState* d_dictState = nullptr; bool dictOn = false;   // zstdb200_load_dictionary
   u8* d_encDict = nullptr; size_t encDictCap = 0;   // the same dictionary prepared for the encoder (EncDict block, zb_encode.cuh)
   EncodeScratch enc;                            // encoder arenas (encode_kernels.cuh)
+  u8* d_seek = nullptr; u8* h_seek = nullptr;   // seekable archives (seek_scratch), allocated by their first call
   // pinned host memory
   u8 *h_src = nullptr, *h_dst = nullptr;
   u8* h_desc = nullptr;
@@ -100,6 +109,7 @@ int alloc_device(zstdb200_ctx* ctx, Device& d) {
   CK(cudaSetDevice(d.id));
   for (auto& s : d.stream) CK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
   CK(cudaEventCreateWithFlags(&d.descEv, cudaEventDisableTiming));
+  CK(cudaEventCreateWithFlags(&d.pendingEv, cudaEventDisableTiming));
   const size_t items = ctx->maxItems;
   // d_src / d_dst are the codec's input / output staging in both directions: compressed frames of a full batch can
   // be larger than the batch (compress bounds), so both buffers take the larger size
@@ -131,11 +141,20 @@ void free_device(Device& d) {
   cudaFree(d.d_info); cudaFree(d.d_lit); cudaFree(d.d_seq); cudaFree(d.d_more); cudaFreeHost(d.h_more);
   cudaFree(d.d_units); cudaFree(d.d_parList); cudaFree(d.d_cnt); cudaFree(d.d_hufFull);
   cudaFree(d.d_dict); cudaFree(d.d_dictState); cudaFree(d.d_encDict);
+  cudaFree(d.d_seek); cudaFreeHost(d.h_seek);
   encode_free(d.enc);
   cudaFreeHost(d.h_src); cudaFreeHost(d.h_dst); cudaFreeHost(d.h_desc);
   for (auto& s : d.stream) if (s) cudaStreamDestroy(s);
   if (d.descEv) cudaEventDestroy(d.descEv);
+  if (d.pendingEv) cudaEventDestroy(d.pendingEv);
   for (auto& ev : d.sliceEv) cudaEventDestroy(ev);
+}
+
+// Waits until no work a call left queued uses the device's staging and scratch (Device::pendingEv).
+cudaError_t pending_wait(Device& d) {
+  if (!d.pending) return cudaSuccess;
+  d.pending = false;
+  return cudaEventSynchronize(d.pendingEv);
 }
 
 // true when the driver can DMA the range directly (cudaMallocHost / cudaHostRegister memory).  A managed caller's
@@ -206,7 +225,53 @@ struct Job {
   const uint32_t* effCap;
   uint32_t maxSrc;     // largest srcSize of the call (compress: table sizes of the match stage)
   bool useDict;        // compress with the context's dictionary (the *_using_dict calls)
+  struct SeekJob* seek = nullptr;   // seekable archives (below); null for every other call
 };
+
+// Seekable archives (seekable.h) through the host batch path.
+struct SeekJob {
+  // compress: after its encode, each sub-batch packs its frames on the device (k_seek_pack).  Once its result codes are on the
+  // host it waits until the sub-batch before it has published where it ends (start[lo], lo: its first item), publishes its own
+  // end (start[lo + m]) and copies its span to out + start[lo]: every byte crosses PCIe once and lands in its final place, also
+  // when devices run concurrently.  ~0: not known yet.  A device that fails calls abort(), which releases every waiter.
+  u8* out = nullptr;
+  std::vector<u64> start;
+  std::mutex mu; std::condition_variable cv; bool aborted = false;
+  bool wait_start(size_t lo, u64* at) {
+    std::unique_lock<std::mutex> l(mu);
+    cv.wait(l, [&] { return aborted || start[lo] != ~0ull; });
+    *at = start[lo];
+    return !aborted;
+  }
+  void publish(size_t i, u64 v) { { std::lock_guard<std::mutex> l(mu); start[i] = v; } cv.notify_all(); }
+  void abort() { { std::lock_guard<std::mutex> l(mu); aborted = true; } cv.notify_all(); }
+  // decompress: each slice's frames are checked against their table entries right after their decode, while the bytes are on
+  // the device (k_seek_check); cksum[i] is the entry's checksum of item i, null when the table carries none
+  const u32* cksum = nullptr;
+};
+
+// The seekable calls' per-device scratch: d_seek = [offsets (maxItems + 2) x 8][cksum maxItems x 4][frame maxItems x 4]
+// [first 8][done 4]; h_seek (pinned) = [cksum maxItems x 4][frame maxItems x 4][footer 16]
+struct SeekScratch {
+  u64* offsets; u32* cksum; u32* frame; unsigned long long* first; u32* done;
+  u32* h_cksum; u32* h_frame; u8* h_footer;
+};
+size_t seek_device_bytes(size_t items) { return (items + 2) * 8 + items * 8 + 16; }
+SeekScratch seek_scratch(const zstdb200_ctx* ctx, const Device& d) {
+  const size_t items = ctx->maxItems;
+  SeekScratch s;
+  s.offsets = (u64*)d.d_seek; s.cksum = (u32*)(s.offsets + items + 2); s.frame = s.cksum + items;
+  s.first = (unsigned long long*)(s.frame + items); s.done = (u32*)(s.first + 1);
+  s.h_cksum = (u32*)d.h_seek; s.h_frame = s.h_cksum + items; s.h_footer = (u8*)(s.h_frame + items);
+  return s;
+}
+int seek_alloc(zstdb200_ctx* ctx, Device& d) {
+  if (d.d_seek) return 0;
+  CK(cudaSetDevice(d.id));
+  CK(cudaMalloc(&d.d_seek, seek_device_bytes(ctx->maxItems)));
+  CK(cudaMallocHost(&d.h_seek, ctx->maxItems * 8 + 16));
+  return 0;
+}
 
 // The arguments of one decode launch over n items, numbered from item_base in the arenas, on stream slot `slot` (its counters
 // and Huffman full-table region).  The item lists are indexed by item_base, so slices of one sub-batch that run concurrently
@@ -229,13 +294,14 @@ DecodeArgs decode_args(const zstdb200_ctx* ctx, const Device& d, const Items& it
 struct SubBatch {
   zstdb200_ctx* ctx; Device& d; const Job& j;
   size_t lo, m; bool decode, srcDirect, dstDirect, eager;
+  bool packed;                   // a seekable compress: no per-item output; the frames leave packed, once (pack / fetch_packed)
   const u8* srcBase; u8* dstBase;
   DescView h;                    // the descriptors (device offsets) in the pinned staging
   Items dev;                     // the items on the device
   std::vector<Range> slices;
 
   SubBatch(zstdb200_ctx* c, Device& dv, const Job& jb, size_t lo_, size_t hi)
-      : ctx(c), d(dv), j(jb), lo(lo_), m(hi - lo_), decode(jb.op == Op::Decompress),
+      : ctx(c), d(dv), j(jb), lo(lo_), m(hi - lo_), decode(jb.op == Op::Decompress), packed(jb.seek && !decode),
         srcBase((const u8*)jb.src[lo_]), dstBase((u8*)jb.dst[lo_]), h(dv.h_desc, hi - lo_) {
     // pageable caller memory goes through the pinned staging with parallel host copies (a pageable cudaMemcpyAsync
     // is a synchronous, single-threaded bounce inside the driver)
@@ -263,6 +329,11 @@ struct SubBatch {
     cudaStream_t s0 = d.stream[0];
     SB_CK(cudaMemsetAsync(d.d_more, 0, NSTREAMS * 4, s0), "memset");
     SB_CK(cudaMemcpyAsync(d.d_desc, d.h_desc, DescView::bytes(m), cudaMemcpyHostToDevice, s0), "H2D desc");
+    if (decode && j.seek && j.seek->cksum) {   // the table's checksums of the sub-batch's frames, for k_seek_check
+      const SeekScratch sc = seek_scratch(ctx, d);
+      memcpy(sc.h_cksum, j.seek->cksum + lo, m * 4);
+      SB_CK(cudaMemcpyAsync(sc.cksum, sc.h_cksum, m * 4, cudaMemcpyHostToDevice, s0), "H2D checksums");
+    }
     if (slices.size() > 1) {
       SB_CK(cudaEventRecord(d.descEv, s0), "event");
       for (int k = 1; k < NSTREAMS; k++) SB_CK(cudaStreamWaitEvent(d.stream[k], d.descEv, 0), "event wait");
@@ -282,11 +353,52 @@ struct SubBatch {
 
   std::string launch(size_t a, size_t b, u32 slot, cudaStream_t st, uint64_t* launches) {
     int nl = 0;
-    const cudaError_t e = decode ? decode_launch(decode_args(ctx, d, dev.from(a), b - a, (u32)a, slot), st, &nl)
-                                 : encode_launch(encode_args(dev.from(a), b - a, (u32)a, j.level, j.checksum, j.maxSrc, slot,
-                                                             j.useDict ? d.d_encDict : nullptr, &ctx->encDict), d.enc, st, &nl);
+    cudaError_t e;
+    if (decode) {
+      DecodeArgs da = decode_args(ctx, d, dev.from(a), b - a, (u32)a, slot);
+      if (j.seek) da.more = nullptr;   // a seek table entry is one frame: nothing behind it is decoded
+      e = decode_launch(da, st, &nl);
+      if (e == cudaSuccess && j.seek) {
+        const SeekScratch sc = seek_scratch(ctx, d);
+        e = seek_check({dev.from(a), da.info, (u32)(b - a), j.seek->cksum ? sc.cksum + a : nullptr, nullptr, nullptr, nullptr, 0, nullptr, 0},
+                       st, &nl);
+      }
+    } else {
+      e = encode_launch(encode_args(dev.from(a), b - a, (u32)a, j.level, j.checksum, j.maxSrc, slot, j.useDict ? d.d_encDict : nullptr,
+                                    &ctx->encDict), d.enc, st, &nl);
+    }
     *launches += nl;
     SB_CK(e, "kernel launch");
+    return "";
+  }
+
+  // Seekable compress: the sub-batch's frames, back to back from d_src[0] (the raw chunks there are no longer needed)
+  std::string pack(uint64_t* launches) {
+    int nl = 0;
+    const SeekScratch sc = seek_scratch(ctx, d);
+    const cudaError_t e = seek_pack({d.d_dst, dev.dstOff, dev.result, dev.srcSize, (u32)m, d.d_src, sc.offsets, nullptr, 0, j.checksum},
+                                    d.stream[0], &nl);
+    *launches += nl;
+    SB_CK(e, "pack launch");
+    return "";
+  }
+
+  // ... and their one copy to the host, at their final offset (SeekJob).  A failed frame packs nothing; the call then fails.
+  std::string fetch_packed() {
+    u64 total = 0, at;
+    bool failed = false;
+    for (size_t k = 0; k < m; k++) { failed |= is_err(d.h_result[k]); total += d.h_result[k]; }
+    if (!j.seek->wait_start(lo, &at)) return "";   // an earlier sub-batch's device failed: so does the call
+    j.seek->publish(lo + m, failed ? at : at + total);
+    if (failed) return "";
+    u8* to = j.seek->out + at;
+    const bool direct = is_dma_able(to);
+    if (total) SB_CK(cudaMemcpyAsync(direct ? to : d.h_dst, d.d_src, total, cudaMemcpyDeviceToHost, d.stream[0]), "D2H packed");
+    SB_CK(cudaStreamSynchronize(d.stream[0]), "stream sync");
+    if (!direct) parallel_for((total + (1u << 20) - 1) >> 20, total, [&](size_t x, size_t y) {
+      const size_t a = x << 20, b = std::min<size_t>(total, y << 20);
+      if (b > a) memcpy(to + a, d.h_dst + a, b - a);
+    });
     return "";
   }
 
@@ -309,6 +421,7 @@ struct SubBatch {
     }
     // a single slice ran on stream 0 alone: its results ride the same stream and one synchronisation ends the call
     if (slices.size() > 1) for (auto& st : d.stream) SB_CK(cudaStreamSynchronize(st), "stream sync");
+    if (packed) SB_TRY(pack(launches));
     SB_CK(cudaMemcpyAsync(d.h_more, d.d_more, (NSTREAMS + m) * 4, cudaMemcpyDeviceToHost, d.stream[0]), "D2H results");
     SB_CK(cudaStreamSynchronize(d.stream[0]), "stream sync");
     u32 anyMore = 0;
@@ -326,6 +439,7 @@ struct SubBatch {
       SB_CK(cudaStreamSynchronize(st), "stream sync");
     }
     for (size_t k = 0; k < m; k++) j.result[lo + k] = d.h_result[k];
+    if (packed) return fetch_packed();
     // staged output not scattered yet (compress: frames are much smaller than their capacity; single-slice calls; items
     // that needed further passes): copy what was produced; on error the reference leaves dst partially written, we copy nothing
     if (!dstDirect && (!eager || anyMore)) parallel_for(m, h.dstOff[m - 1] + h.dstCap[m - 1], [&](size_t x, size_t y) {
@@ -342,6 +456,7 @@ struct SubBatch {
 // finish.
 std::string run_subbatch(zstdb200_ctx* ctx, Device& d, const Job& j, size_t lo, size_t hi, uint64_t* launches) {
   static const int nStreams = env_int("ZSTDB200_STREAMS", NSTREAMS, 1, NSTREAMS);
+  SB_CK(pending_wait(d), "pending wait");
   SubBatch sb(ctx, d, j, lo, hi);
   SB_TRY(sb.start());
   for (size_t s = 0; s < sb.slices.size(); s++) {
@@ -350,7 +465,7 @@ std::string run_subbatch(zstdb200_ctx* ctx, Device& d, const Job& j, size_t lo, 
     cudaStream_t st = d.stream[slot];
     SB_TRY(sb.stage_in(a, b, st));
     SB_TRY(sb.launch(a, b, slot, st, launches));
-    SB_TRY(sb.stage_out(a, b, st));
+    if (!sb.packed) SB_TRY(sb.stage_out(a, b, st));
     if (sb.eager) SB_CK(cudaEventRecord(d.sliceEv[s], st), "event");
   }
   return sb.finish(launches);
@@ -398,11 +513,9 @@ int run_host_batch(zstdb200_ctx* ctx, const Job& j0, size_t n, bool clamp = true
   auto worker = [&](size_t di) {
     Device& d = ctx->dev[di];
     cudaError_t e = cudaSetDevice(d.id);
-    if (e != cudaSuccess) { errs[di] = std::string("cudaSetDevice: ") + cudaGetErrorString(e); return; }
-    for (size_t s = di; s < subs.size(); s += nd) {
-      errs[di] = run_subbatch(ctx, d, j, subs[s].lo, subs[s].hi, &launches[di]);
-      if (!errs[di].empty()) return;
-    }
+    if (e != cudaSuccess) errs[di] = std::string("cudaSetDevice: ") + cudaGetErrorString(e);
+    for (size_t s = di; errs[di].empty() && s < subs.size(); s += nd) errs[di] = run_subbatch(ctx, d, j, subs[s].lo, subs[s].hi, &launches[di]);
+    if (!errs[di].empty() && j.seek) j.seek->abort();   // other devices' sub-batches may wait for this one's place (SeekJob)
   };
   if (nd == 1 || subs.size() == 1) { for (size_t di = 0; di < nd; di++) worker(di); }
   else { std::vector<std::thread> th; for (size_t di = 0; di < nd; di++) th.emplace_back(worker, di); for (auto& t : th) t.join(); }
@@ -439,6 +552,7 @@ int device_call(zstdb200_ctx* ctx, Op op, int device_index, size_t n, int level,
   if (useDict && ctx->encDict.empty()) { ctx->err = "no dictionary loaded (zstdb200_load_dictionary)"; return 1; }
   *d = &ctx->dev[device_index];
   CK(cudaSetDevice((*d)->id));
+  CK(pending_wait(**d));
   *st = stream ? (cudaStream_t)stream : (*d)->stream[0];
   return 0;
 }
@@ -531,6 +645,7 @@ int zstdb200_load_dictionary(zstdb200_ctx* ctx, const void* dict, uint32_t dictS
   }
   for (auto& d : ctx->dev) {
     CK(cudaSetDevice(d.id));
+    CK(pending_wait(d));
     if (!dict || dictSize == 0) { d.dictOn = false; continue; }
     if (dictSize + 64 > d.dictCap) {
       cudaFree(d.d_dict); d.d_dict = nullptr; d.dictCap = 0;
@@ -679,11 +794,240 @@ uint32_t zstdb200_train_dictionary(zstdb200_ctx* ctx, void* dictBuffer, uint32_t
   if (params) p = *params;
   Device& d = ctx->dev[0];
   if (cudaSetDevice(d.id) != cudaSuccess) { ctx->err = "cudaSetDevice failed"; return zerr(ZE_GENERIC); }
+  if (pending_wait(d) != cudaSuccess) { ctx->err = "waiting for queued work failed"; return zerr(ZE_GENERIC); }
   DtDevice dv{d.stream[0], &d.enc, d.d_dst, ctx->srcCap, d.d_result, d.h_result, d.d_desc, d.h_desc, ctx->maxBatch, ctx->maxItems, 0};
   const u32 r = dt_train_run(dv, (u8*)dictBuffer, dictCapacity, (const u8*)samples, sampleSizes, nbSamples, p, ctx->err);
   ctx->launches += dv.launches;
   if (!is_err(r) && params) { params->k = p.k; params->d = p.d; }
   return r;
+}
+
+// ---- seekable archives (seekable.h, seekable_kernels.cu) ---------------------------------------------------------------
+
+uint32_t zstdb200_seekable_info_get(const void* src, uint64_t srcSize, zstdb200_seekable_info* info) {
+  seek::Table t;
+  const u32 r = seek::parse((const u8*)src, srcSize, &t);
+  if (r) return r;
+  if (info) *info = {t.contentSize, t.dataSize, t.n, t.ck ? 1u : 0u, t.maxContent, t.maxCompressed};
+  return 0;
+}
+
+uint64_t zstdb200_seekable_bound(uint64_t srcSize, uint32_t frameSize) {
+  if (frameSize == 0) return 0;
+  return seek::bound(srcSize, frameSize, [](uint64_t c) { return (uint64_t)encode_bound(c); });
+}
+
+}  // extern "C"
+
+namespace {
+
+// The argument checks both seekable compress calls share.
+int seek_compress_args(zstdb200_ctx* ctx, int checksum, uint32_t frameSize, const void* src, uint64_t srcSize, const void* dst,
+                       uint64_t dstCapacity, const void* dstSize) {
+  if ((!src && srcSize) || !dst || !dstSize) { ctx->err = "null argument"; return 1; }
+  if (frameSize == 0 || frameSize > ctx->maxBatch) { ctx->err = "frameSize must be 1..max_batch_bytes"; return 1; }
+  if (!seek::table_fits(seek::frame_count(srcSize, frameSize), checksum != 0)) {
+    ctx->err = "too many frames: the seek table's Frame_Size would not fit 32 bits"; return 1;
+  }
+  if (dstCapacity < zstdb200_seekable_bound(srcSize, frameSize)) { ctx->err = "dstCapacity is below zstdb200_seekable_bound"; return 1; }
+  return 0;
+}
+
+// A selected frame whose content does not fit one launch's arenas fails the call.
+int seek_frames_fit(zstdb200_ctx* ctx, const std::vector<seek::Piece>& pieces) {
+  for (auto& p : pieces)
+    if (p.dsize > ctx->maxBatch || p.csize > ctx->maxBatch) { ctx->err = "a frame is larger than the context's max_batch_bytes"; return 1; }
+  return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int zstdb200_compress_seekable(zstdb200_ctx* ctx, int level, int checksum, uint32_t frameSize, const void* src, uint64_t srcSize,
+                               void* dst, uint64_t dstCapacity, uint64_t* dstSize) {
+  if (!ctx) return 1;
+  ctx->err.clear();
+  if (!level_ok(level)) { ctx->err = kLevelError; return 1; }
+  if (seek_compress_args(ctx, checksum, frameSize, src, srcSize, dst, dstCapacity, dstSize)) return 1;
+  const size_t n = (size_t)seek::frame_count(srcSize, frameSize);
+  const u8* s = (const u8*)src; u8* out = (u8*)dst;
+  std::vector<const void*> srcs(n); std::vector<void*> dsts(n, nullptr);
+  std::vector<uint32_t> sizes(n), caps(n), res(n);
+  for (size_t i = 0; i < n; i++) {
+    srcs[i] = s + (u64)i * frameSize; sizes[i] = seek::frame_content(srcSize, frameSize, i);
+    caps[i] = (uint32_t)encode_bound(sizes[i]);
+  }
+  SeekJob sj; sj.out = out; sj.start.assign(n + 1, ~0ull); sj.start[0] = 0;
+  Job j{Op::Compress, level, checksum ? 1 : 0, srcs.data(), sizes.data(), dsts.data(), caps.data(), res.data(), nullptr, 0, false, &sj};
+  if (n) {
+    for (auto& d : ctx->dev) if (seek_alloc(ctx, d)) return 1;
+    if (run_host_batch(ctx, j, n)) return 1;
+  }
+  for (size_t i = 0; i < n; i++)
+    if (is_err(res[i])) { ctx->err = "frame " + std::to_string(i) + " failed to compress: error " + std::to_string(zerr(res[i])); return 1; }
+  // the frames are in place (SeekJob); the table from their sizes and each frame's own checksum
+  const u64 total = sj.start[n];
+  std::vector<uint32_t> cks(checksum ? n : 0);
+  for (size_t i = 0, pos = 0; i < n; pos += res[i], i++) if (checksum) cks[i] = seek::rd32(out + pos + res[i] - 4);
+  seek::write_table(out + total, n, res.data(), sizes.data(), cks.data(), checksum != 0);
+  *dstSize = total + seek::table_bytes(n, checksum != 0);
+  return 0;
+}
+
+// The frames are encoded into the context's staging (d_dst, 16-byte aligned slots of their compress bound), then packed into
+// dst with their table.  One synchronisation: the descriptors' upload (as compress_batch_device's size fetch).
+int zstdb200_compress_seekable_device(zstdb200_ctx* ctx, int device_index, int level, int checksum, uint32_t frameSize, const void* src,
+                                      uint64_t srcSize, void* dst, uint64_t dstCapacity, uint64_t* dstSize, void* stream) {
+  Device* d; cudaStream_t st;
+  if (!ctx) return 1;
+  const uint64_t nf = frameSize ? seek::frame_count(srcSize, frameSize) : 0;
+  if (device_call(ctx, Op::Compress, device_index, (size_t)std::min<uint64_t>(nf, ~(size_t)0), level, false, stream, &d, &st)) return 1;
+  if (seek_compress_args(ctx, checksum, frameSize, src, srcSize, dst, dstCapacity, dstSize)) return 1;
+  if (srcSize > ctx->maxBatch) { ctx->err = "srcSize exceeds max_batch_bytes"; return 1; }
+  if (seek_alloc(ctx, *d)) return 1;
+  const size_t n = (size_t)nf;
+  DescView h(d->h_desc, n);
+  u64 out = 0;
+  for (size_t i = 0; i < n; i++) {
+    h.srcOff[i] = (u64)i * frameSize; h.srcSize[i] = seek::frame_content(srcSize, frameSize, i);
+    h.dstCap[i] = (u32)encode_bound(h.srcSize[i]); h.dstOff[i] = out; out += align_up(h.dstCap[i], 16);
+  }
+  if (out > ctx->srcCap) { ctx->err = "the frames' compress bounds exceed the context's staging"; return 1; }
+  int nl = 0;
+  const DescView dv(d->d_desc, n);
+  if (n) {
+    CK(cudaMemcpyAsync(d->d_desc, d->h_desc, DescView::bytes(n), cudaMemcpyHostToDevice, st));
+    CK(cudaStreamSynchronize(st));   // h_desc is the context's: the copy must be done before the next call refills it
+    const Items it = dv.items((const u8*)src, d->d_dst, d->d_result);
+    CK(encode_launch(encode_args(it, n, 0, level, checksum ? 1 : 0, (u32)std::min<uint64_t>(frameSize, srcSize), ENC_EXCLUSIVE, nullptr,
+                                 &ctx->encDict), d->enc, st, &nl));
+  }
+  const SeekScratch sc = seek_scratch(ctx, *d);
+  CK(seek_pack({d->d_dst, dv.dstOff, d->d_result, dv.srcSize, (u32)n, (u8*)dst, sc.offsets, dstSize, 1, checksum ? 1 : 0}, st, &nl));
+  ctx->launches += nl;
+  return 0;
+}
+
+int zstdb200_decompress_seekable(zstdb200_ctx* ctx, void* dst, uint64_t offset, uint64_t length, const void* src, uint64_t srcSize,
+                                 uint32_t* code) {
+  if (!ctx) return 1;
+  ctx->err.clear();
+  if (!code || (!src && srcSize) || (!dst && length)) { ctx->err = "null argument"; return 1; }
+  seek::Table t; std::vector<seek::Piece> pieces;
+  u32 r = seek::parse((const u8*)src, srcSize, &t);
+  if (!r) r = seek::plan_range(t, offset, length, &pieces);
+  *code = r;
+  if (r || pieces.empty()) return 0;
+  if (seek_frames_fit(ctx, pieces)) return 1;
+  for (auto& d : ctx->dev) if (seek_alloc(ctx, d)) return 1;
+  // one item per frame: interior frames decode straight into dst, the edge frames into scratch
+  const size_t n = pieces.size();
+  std::vector<const void*> srcs(n); std::vector<void*> dsts(n); std::vector<uint32_t> sizes(n), caps(n), res(n), cks(n);
+  std::vector<std::vector<u8>> edge(n);
+  for (size_t k = 0; k < n; k++) {
+    const seek::Piece& p = pieces[k];
+    if (p.edge()) edge[k].resize(p.dsize);
+    srcs[k] = (const u8*)src + p.srcOff; sizes[k] = p.csize; caps[k] = p.dsize;
+    dsts[k] = p.edge() ? (void*)edge[k].data() : (void*)((u8*)dst + p.dstOff);
+    cks[k] = t.ck ? t.cksum[p.frame] : 0;
+  }
+  SeekJob sj; sj.cksum = t.ck ? cks.data() : nullptr;
+  Job j{Op::Decompress, 0, 0, srcs.data(), sizes.data(), dsts.data(), caps.data(), res.data(), nullptr, 0, false, &sj};
+  if (run_host_batch(ctx, j, n, false)) return 1;   // capacities are the entries' sizes: nothing to clamp
+  for (size_t k = 0; k < n; k++) if (is_err(res[k])) { *code = res[k]; return 0; }
+  for (size_t k = 0; k < n; k++) if (pieces[k].edge()) memcpy((u8*)dst + pieces[k].dstOff, edge[k].data() + pieces[k].skip, pieces[k].take);
+  return 0;
+}
+
+// Edge frames first, into the context's staging d_dst, then the others in archive order straight into dst; each group is one
+// launch sequence of the decode pipeline followed by k_seek_check.  The groups respect one launch's arenas and share one
+// descriptor upload while they fit max_items (otherwise the stream is synchronised before the pinned descriptors are refilled).
+int zstdb200_decompress_seekable_device(zstdb200_ctx* ctx, int device_index, void* dst, uint64_t offset, uint64_t length, const void* src,
+                                        uint64_t srcSize, uint32_t* code, void* stream) {
+  Device* d; cudaStream_t st;
+  if (device_call(ctx, Op::Decompress, device_index, 0, 0, false, stream, &d, &st)) return 1;
+  if (!code || (!src && srcSize) || (!dst && length)) { ctx->err = "null argument"; return 1; }
+  if (seek_alloc(ctx, *d)) return 1;
+  const SeekScratch sc = seek_scratch(ctx, *d);
+  const u8* s = (const u8*)src;
+  seek::Table t; std::vector<seek::Piece> pieces;
+  u32 r = srcSize < seek::MIN_ARCHIVE ? seek::ERR_srcSize_wrong : 0;
+  if (!r) {   // the footer, then the table: two small copies, two synchronisations
+    CK(cudaMemcpyAsync(sc.h_footer, s + srcSize - seek::FOOTER_BYTES, seek::FOOTER_BYTES, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    seek::Footer f;
+    r = seek::parse_footer(sc.h_footer, srcSize, &f);
+    if (!r) {
+      std::vector<u8> tab(f.tableBytes);
+      CK(cudaMemcpyAsync(tab.data(), s + srcSize - f.tableBytes, f.tableBytes, cudaMemcpyDeviceToHost, st));
+      CK(cudaStreamSynchronize(st));
+      r = seek::parse_table(tab.data(), srcSize, f, &t);
+    }
+  }
+  if (!r) r = seek::plan_range(t, offset, length, &pieces);
+  if (seek_frames_fit(ctx, pieces)) return 1;
+  std::vector<size_t> order;   // indices into pieces: edge frames, then the rest
+  for (size_t k = 0; k < pieces.size(); k++) if (pieces[k].edge()) order.push_back(k);
+  const size_t nEdge = order.size();
+  for (size_t k = 0; k < pieces.size(); k++) if (!pieces[k].edge()) order.push_back(k);
+  bool big = false;
+  auto bytes = [&](size_t x) { return (size_t)pieces[order[x]].dsize; };
+  std::vector<Range> groups = make_subbatches(nEdge, ~(size_t)0, std::min(ctx->srcCap, ctx->maxBatch), ctx->maxItems, bytes, bytes, &big);
+  std::vector<Range> inner = make_subbatches(order.size() - nEdge, ~(size_t)0, ctx->maxBatch, ctx->maxItems,
+                                             [&](size_t x) { return bytes(nEdge + x); }, [&](size_t x) { return bytes(nEdge + x); }, &big);
+  for (auto& g : inner) groups.push_back({nEdge + g.lo, nEdge + g.hi});
+  u32 blocks = 0;
+  for (auto& g : groups) blocks += seek_check_blocks((u32)(g.hi - g.lo));
+  CK(cudaMemsetAsync(sc.first, 0xFF, 8, st));
+  CK(cudaMemsetAsync(sc.done, 0, 4, st));
+  int nl = 0;
+  if (groups.empty()) {   // an error of the table or the range, or an empty range: only the code
+    CK(seek_check({Items{}, nullptr, 0, nullptr, nullptr, sc.first, sc.done, 1, code, r}, st, &nl));
+    CK(cudaEventRecord(d->pendingEv, st)); d->pending = true;
+    ctx->launches += nl;
+    return 0;
+  }
+  for (size_t g = 0; g < groups.size();) {
+    size_t g1 = g, m = 0;
+    while (g1 < groups.size() && m + (groups[g1].hi - groups[g1].lo) <= ctx->maxItems) m += groups[g1].hi - groups[g1].lo, g1++;
+    CK(pending_wait(*d));   // the previous groups' work still reads the pinned descriptors
+    DescView h(d->h_desc, m);
+    for (size_t x = g, k = 0; x < g1; x++) {
+      const bool isEdge = groups[x].lo < nEdge;
+      u64 edgeAt = 0;
+      const u64 base = isEdge ? 0 : pieces[order[groups[x].lo]].dstOff;
+      for (size_t y = groups[x].lo; y < groups[x].hi; y++, k++) {
+        const seek::Piece& p = pieces[order[y]];
+        h.srcOff[k] = p.srcOff; h.srcSize[k] = p.csize; h.dstCap[k] = p.dsize;
+        h.dstOff[k] = isEdge ? edgeAt : p.dstOff - base;
+        edgeAt += align_up(p.dsize, 16);
+        sc.h_frame[k] = p.frame; sc.h_cksum[k] = t.ck ? t.cksum[p.frame] : 0;
+      }
+    }
+    CK(cudaMemcpyAsync(d->d_desc, d->h_desc, DescView::bytes(m), cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(sc.frame, sc.h_frame, m * 4, cudaMemcpyHostToDevice, st));
+    if (t.ck) CK(cudaMemcpyAsync(sc.cksum, sc.h_cksum, m * 4, cudaMemcpyHostToDevice, st));
+    const DescView dv(d->d_desc, m);
+    for (size_t x = g, k0 = 0; x < g1; k0 += groups[x].hi - groups[x].lo, x++) {
+      const bool isEdge = groups[x].lo < nEdge;
+      const u32 n = (u32)(groups[x].hi - groups[x].lo);
+      u8* base = isEdge ? d->d_dst : (u8*)dst + pieces[order[groups[x].lo]].dstOff;
+      const Items it = dv.items(s, base, d->d_result).from(k0);
+      DecodeArgs a = decode_args(ctx, *d, it, n, 0, 0);
+      a.more = nullptr;   // a seek table entry is one frame
+      CK(decode_launch(a, st, &nl));
+      CK(seek_check({it, a.info, n, t.ck ? sc.cksum + k0 : nullptr, sc.frame + k0, sc.first, sc.done, blocks, code, 0}, st, &nl));
+      for (size_t k = k0; isEdge && k < k0 + n; k++) {
+        const seek::Piece& p = pieces[order[groups[x].lo + (k - k0)]];
+        CK(cudaMemcpyAsync((u8*)dst + p.dstOff, d->d_dst + h.dstOff[k] + p.skip, p.take, cudaMemcpyDeviceToDevice, st));
+      }
+    }
+    CK(cudaEventRecord(d->pendingEv, st)); d->pending = true;
+    g = g1;
+  }
+  ctx->launches += nl;
+  return 0;
 }
 
 void* zstdb200_host_alloc(size_t bytes) { void* p = nullptr; return cudaMallocHost(&p, bytes ? bytes : 1) == cudaSuccess ? p : nullptr; }
