@@ -275,8 +275,10 @@ __device__ __forceinline__ void seq_smem_init(SM& sm, u32 lane) {
 }
 
 // CLS: 0 = full-size tables (also every frame the smaller instantiations handed over), 1 = FI_SEQ_A, 2 = FI_SEQ_B
+// Shared memory bounds residency (6 / 3 / 2 CTAs per SM), not registers: with a minimum of one CTA per SM ptxas keeps the
+// table and ring addresses of the sequence loop in registers instead of spilling or recomputing them every sequence.
 template <int CLS, int CL, int CO, int CM>
-__global__ void __launch_bounds__(32) k_seq_t(DecodeArgs a) {
+__global__ void __launch_bounds__(32, 1) k_seq_t(DecodeArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   typedef SeqSmemT<CL, CO, CM> SM;
   SM& sm = *reinterpret_cast<SM*>(smem_raw);
@@ -750,7 +752,7 @@ __global__ void __launch_bounds__(32) k_huf_blk(DecodeArgs a) {
 }
 
 // k_seq_blk : k_seq's mapping (one unit per lane, tables bank-interleaved), persistent over the launch's units
-__global__ void __launch_bounds__(32) k_seq_blk(DecodeArgs a) {
+__global__ void __launch_bounds__(32, 1) k_seq_blk(DecodeArgs a) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   SeqSmem& sm = *reinterpret_cast<SeqSmem*>(smem_raw);
   const u32 lane = threadIdx.x;

@@ -99,12 +99,9 @@ struct UnitEmitter {
     rec_store(out + n, dpos, lpos | ((ml >> 15) << 18) | (ot << 21), ov, ll | (ml << 17));
     n++; dpos = sat_add32(dpos, ll + ml); lpos = sat_lpos(lpos, ll);
   }
-  ZB_HD void fast(u32 hi, u32 llSym, u32 ofBits, u32 iLL, u32 iML) {
-    const u32 llBits = iLL >> 24, mlBits = iML >> 24;
-    const u32 ofv = shr_c(hi, 32 - ofBits);
-    const u32 mlv = shr_c(hi << ofBits, 32 - mlBits);
-    const u32 llv = shr_c(hi << (ofBits + mlBits), 32 - llBits);
-    emit(ofBits, ofv, llSym, (iLL & 0xFFFFFF) + llv, (iML & 0xFFFFFF) + mlv);
+  ZB_HD void fast(u32 hi, u32 llSym, u32 mlSym, u32 ofBits, u32 mlBits, u32 llBits) {
+    const u32 ofv = take_bits(hi, ofBits), mlv = take_bits(hi, mlBits), llv = take_bits(hi, llBits);
+    emit(ofBits, ofv, llSym, (llInfo[llSym] & 0xFFFFFF) + llv, (mlInfo[mlSym] & 0xFFFFFF) + mlv);
   }
   ZB_HD void values(u32 ofv, u32 mlv, u32 llv, u32 llSym, u32 mlSym, u32 ofBits) {
     emit(ofBits, ofv, llSym, (llInfo[llSym] & 0xFFFFFF) + llv, (mlInfo[mlSym] & 0xFFFFFF) + mlv);
@@ -207,7 +204,7 @@ ZB_HD void seq_decode_unit(const u8* src, const BlockUnit& u, const BlockUnit* f
   u32 nbSeq, modes, hdr;
   read_seq_count(sp, ssz, &nbSeq, &modes, &hdr);
   if (!nbSeq) return;
-  for (int k = 0; k < 3; k++) { T.cur[k] = T.space[k]; T.curStride[k] = T.stride; T.log[k] = 0; }
+  for (int k = 0; k < 3; k++) T.log[k] = 0;
   const int kinds[3] = {KIND_LL, KIND_OF, KIND_ML};
   const u32 modeOf[3] = {(modes >> 4) & 3, (modes >> 2) & 3, modes & 3};
   u32 e = 0;
@@ -215,7 +212,7 @@ ZB_HD void seq_decode_unit(const u8* src, const BlockUnit& u, const BlockUnit* f
     const int kind = kinds[k]; u32 used = 0, lg = 0; bool isDef = false;
     if (modeOf[k] == 3) continue;
     e = read_seq_table(modeOf[k], kind, sp + hdr, ssz - hdr, T.space[kind], T.stride, &lg, &isDef, true, &used, norm, symbolNext);
-    if (!e) { hdr += used; T.log[kind] = lg; if (isDef) { T.cur[kind] = T.defs[kind]; T.curStride[kind] = 1; } }
+    if (!e) { hdr += used; T.log[kind] = lg; if (isDef) seq_use_default(T, kind); }
   }
   for (int k = 0; k < 3 && !e; k++) {                                              // inherited tables: rebuilt from their definer
     const int kind = kinds[k];
@@ -230,7 +227,7 @@ ZB_HD void seq_decode_unit(const u8* src, const BlockUnit& u, const BlockUnit* f
       const u8* desc; u32 descSize, mode, used = 0, lg = 0; bool isDef = false;
       if (!unit_locate_table(src + d.body, d.csize, kind, norm, &desc, &descSize, &mode)) { e = ZE_corruption_detected; break; }
       e = read_seq_table(mode, kind, desc, descSize, T.space[kind], T.stride, &lg, &isDef, true, &used, norm, symbolNext);
-      if (!e) { T.log[kind] = lg; if (isDef) { T.cur[kind] = T.defs[kind]; T.curStride[kind] = 1; } }
+      if (!e) { T.log[kind] = lg; if (isDef) seq_use_default(T, kind); }
     }
   }
   if (e) { em.fail(0, ZE_corruption_detected); return; }

@@ -96,7 +96,7 @@ ZB_HD u64 ld64(const u8* p) { return (u64)ld32(p) | ((u64)ld32(p + 4) << 32); }
 
 ZB_HD u32 highbit(u32 v) {   // floor(log2(v)), v != 0 (csharp/src/BitStream.cs:205-215)
 #if defined(__CUDA_ARCH__)
-  return 31 - __clz(v);
+  u32 r; asm("bfind.u32 %0, %1;" : "=r"(r) : "r"(v)); return r;   // one FLO; 31 - __clz(v) leaves two subtractions behind
 #else
   return 31 - __builtin_clz(v);
 #endif
@@ -115,6 +115,13 @@ ZB_HD u32 fshl(u32 lo, u32 hi, u32 s) {   // high 32 bits of (hi:lo) << (s & 31)
 #else
   s &= 31; return s ? (hi << s) | (lo >> (32 - s)) : hi;
 #endif
+}
+// the top n bits of w (n < 32), and w moves past them: one 32 x 32 -> 64-bit multiplication by 2^n (an FMA-pipe
+// IMAD.WIDE) in place of a subtraction and two shifts on the ALU pipe
+ZB_HD u32 take_bits(u32& w, u32 n) {
+  const u64 p = (u64)w * (1u << n);
+  w = (u32)p;
+  return (u32)(p >> 32);
 }
 ZB_HD u32 shr_c(u32 x, u32 n) {   // x >> n with n clamped to 32 (so n == 32 yields 0), as PTX shr.b32 defines it
 #if defined(__CUDA_ARCH__)

@@ -45,11 +45,16 @@ ZB_HD u64 seq_capacity(u64 cap) { return 2 * (cap / 3) + 24; }
 
 struct SeqTableSet {
   u32 cap[3] = {9, 9, 9};   // table log each space can hold (KIND_LL, KIND_OF, KIND_ML); smaller in the kernels for frames of few sequences
-  u16* space[3];            // lane-private cells for LL, OF, ML (index with *stride)
+  u16* space[3];            // lane-private cells for LL, OF, ML (index with *stride): the tables in force
   u32 stride;
-  const u16* defs[3];       // predefined tables, stride 1
-  const u16* cur[3]; u32 curStride[3]; u32 log[3];
+  const u16* defs[3];       // predefined tables, stride 1: a block that selects one gets a copy in its space (seq_use_default)
+  u32 log[3];
 };
+// Every table the sequence loop reads sits in the lane's space, so that a cell's address is the state times one stride
+// (a shift on the device) whichever mode a block chose.  The predefined logs (6 / 5 / 6) fit every class's space.
+ZB_HD void seq_use_default(SeqTableSet& T, int kind) {
+  for (u32 u = 0; u < (1u << T.log[kind]); u++) T.space[kind][u * T.stride] = T.defs[kind][u];
+}
 
 struct SeqFrameOut {
   u32 err_block, err_code, err_index;
@@ -159,13 +164,10 @@ struct SeqEmitter {
     n++; dpos = sat_add32(dpos, ll + ml); lpos = sat_lpos(lpos, ll);
   }
   // a sequence of the fast path: hi = 32 stream bits whose top bits are its value bits (fewer than 32 of them), in the
-  // reference's read order offset, matchLength, litLength (:1504, :1534, :1542); iLL / iML = the symbols' info words
-  ZB_HD void fast(u32 hi, u32 llSym, u32 ofBits, u32 iLL, u32 iML) {
-    const u32 llBits = iLL >> 24, mlBits = iML >> 24;
-    const u32 ofv = shr_c(hi, 32 - ofBits);
-    const u32 mlv = shr_c(hi << ofBits, 32 - mlBits);
-    const u32 llv = shr_c(hi << (ofBits + mlBits), 32 - llBits);
-    emit(ofBits, ofv, llSym, (iLL & 0xFFFFFF) + llv, (iML & 0xFFFFFF) + mlv);
+  // reference's read order offset, matchLength, litLength (:1504, :1534, :1542)
+  ZB_HD void fast(u32 hi, u32 llSym, u32 mlSym, u32 ofBits, u32 mlBits, u32 llBits) {
+    const u32 ofv = take_bits(hi, ofBits), mlv = take_bits(hi, mlBits), llv = take_bits(hi, llBits);
+    emit(ofBits, ofv, llSym, (llInfo[llSym] & 0xFFFFFF) + llv, (mlInfo[mlSym] & 0xFFFFFF) + mlv);
   }
   // a sequence whose value bits the chain half had to extract itself (stream tail, >= 32 value bits, over-reads)
   ZB_HD void values(u32 ofv, u32 mlv, u32 llv, u32 llSym, u32 mlSym, u32 ofBits) {
@@ -190,7 +192,7 @@ struct SeqEmitter {
   ZB_HD void fail(u32 blk, u32 code) { if (dead) return; res.err_block = blk; res.err_code = code; res.err_index = 0xFFFFFFFFu; dead = true; }
 };
 
-// The bitstream of one compressed block: nbSeq sequences out of bits[0..nbytes) with the tables in force (T.cur, T.log)
+// The bitstream of one compressed block: nbSeq sequences out of bits[0..nbytes) with the tables in force (T.space, T.log)
 // go to `sink` (block_begin ... block_end).  Returns true when the frame cannot go on (the stream failed or the sink has
 // stopped).  blk = the block's index for the sink's error record.
 template <class Sink>
@@ -201,7 +203,7 @@ ZB_HD bool seq_decode_bitstream(const u8* bits, u32 nbytes, u32 nbSeq, u64 windo
   bool longVariant = false;
   if (window > (1u << 24)) {
     const u32 lg = T.log[KIND_OF]; u32 total = 0;
-    for (u32 u = 0; u < (1u << lg); u++) total += (T.cur[KIND_OF][u * T.curStride[KIND_OF]] >> 10) > 22;
+    for (u32 u = 0; u < (1u << lg); u++) total += (T.space[KIND_OF][u * T.stride] >> 10) > 22;
     longVariant = (total << (8 - lg)) >= 20;
   }
   // ---- bitstream ----
@@ -211,35 +213,36 @@ ZB_HD bool seq_decode_bitstream(const u8* bits, u32 nbytes, u32 nbSeq, u64 windo
   if (!bc_init(c, bits, nbytes)) bad = true;                          // :1577 -> corruption_detected
   if (!bad) {
     i32 P = c.P;
-    const u16 *tLL = T.cur[KIND_LL], *tOF = T.cur[KIND_OF], *tML = T.cur[KIND_ML];
-    const u32 sLLs = T.curStride[KIND_LL], sOFs = T.curStride[KIND_OF], sMLs = T.curStride[KIND_ML];
+    const u16 *tLL = T.space[KIND_LL], *tOF = T.space[KIND_OF], *tML = T.space[KIND_ML];
+    const u32 S = T.stride;
     u32 stLL, stOF, stML;
     { u64 w = bc_window64(c, P); u32 lg = T.log[KIND_LL]; stLL = top_bits(w, lg); w <<= lg; P -= (i32)lg;
       lg = T.log[KIND_OF]; stOF = top_bits(w, lg); w <<= lg; P -= (i32)lg;
       lg = T.log[KIND_ML]; stML = top_bits(w, lg); P -= (i32)lg; }             // :1578-1580 (<= 26 bits)
     u32 i = 0;
     // ---- fast loop: >= 128 unread bits, so no over-read is possible (a sequence takes <= 89 bits); leaves to
-    //      the careful loop when a sequence carries >= 32 value bits (rare: very long lengths / offsets) ----
+    //      the careful loop when a sequence carries >= 32 value bits (rare: very long lengths / offsets).
+    //      The next states and cursor are computed ahead of that test, so that their dependent chain (cell -> extra-bit
+    //      counts -> state bits -> next cell) does not wait behind it; the sink then gets the sequence ----
     BitRing ring;
     if (nbSeq && P >= 128) ring_init(ring, ringMem, bits, nbytes);
     while (i < nbSeq && P >= 128) {
       u32 lo, hi;
       ring_window(ring, P, lo, hi);                                          // 64-bit window ending at P
-      const u32 yLL = tLL[stLL * sLLs], yOF = tOF[stOF * sOFs], yML = tML[stML * sMLs];
+      const u32 yLL = tLL[stLL * S], yOF = tOF[stOF * S], yML = tML[stML * S];
       const u32 llSym = yLL >> 10, mlSym = yML >> 10, ofBits = yOF >> 10;   // the offset code is its own extra-bit count
-      const u32 iLL = llInfo[llSym], iML = mlInfo[mlSym];
-      const u32 valBits = ofBits + (iML >> 24) + (iLL >> 24);
-      const u32 lLL = yLL & 0x3FF, lOF = yOF & 0x3FF, lML = yML & 0x3FF;
-      const u32 nLL = cell_nb(lLL), nML = cell_nb(lML), nOF = cell_nb(lOF);
+      const u32 llBits = llInfo[llSym] >> 24, mlBits = mlInfo[mlSym] >> 24;
+      const u32 valBits = ofBits + mlBits + llBits;
+      // state update LL, ML, OF (:1547-1550) from the 32 bits after the value bits; w * 2^n drops n of them
+      const u32 uLL = cell_unit(yLL), uML = cell_unit(yML), uOF = cell_unit(yOF), uLM = uLL * uML;
+      const u32 h2 = fshl(lo, hi, valBits);
+      const u32 nLL = cell_next(yLL, uLL, h2), nML = cell_next(yML, uML, h2 * uLL), nOF = cell_next(yOF, uOF, h2 * uLM);
+      const i32 Pn = P - (i32)(valBits + highbit(uLM * uOF));                // the units multiply to 2^(state bits)
       // the one rare exit of the loop: >= 32 value bits (they do not fit the word handed over) — nothing has been
       // committed yet, the careful loop redoes this sequence
       if (valBits >= 32) break;
-      sink.fast(hi, llSym, ofBits, iLL, iML);
-      const u32 h2 = fshl(lo, hi, valBits);                                  // the 32 bits after the value bits
-      stLL = cell_base(lLL) + shr_c(h2, 32 - nLL);                           // state update LL, ML, OF (:1547-1550)
-      stML = cell_base(lML) + shr_c(h2 << nLL, 32 - nML);
-      stOF = cell_base(lOF) + shr_c(h2 << (nLL + nML), 32 - nOF);
-      const i32 Pn = P - (i32)(valBits + nLL + nML + nOF);
+      sink.fast(hi, llSym, mlSym, ofBits, mlBits, llBits);
+      stLL = nLL; stML = nML; stOF = nOF;
       ring_advance(ring, Pn);
       P = Pn; i++;
     }
@@ -248,7 +251,7 @@ ZB_HD bool seq_decode_bitstream(const u8* bits, u32 nbytes, u32 nbSeq, u64 windo
     for (; i < nbSeq; i++) {
       if (P < 0) { bad = true; break; }                                      // loop test :1582 (overflow)
       const u64 w0 = bc_window64(c, P);
-      const u32 yLL = tLL[stLL * sLLs], yOF = tOF[stOF * sOFs], yML = tML[stML * sMLs];
+      const u32 yLL = tLL[stLL * S], yOF = tOF[stOF * S], yML = tML[stML * S];
       const u32 llSym = yLL >> 10, mlSym = yML >> 10, ofBits = yOF >> 10;
       const u32 llBits = llInfo[llSym] >> 24, mlBits = mlInfo[mlSym] >> 24;
       const u32 lLL = yLL & 0x3FF, lOF = yOF & 0x3FF, lML = yML & 0x3FF;
@@ -288,7 +291,7 @@ ZB_HD void seq_decode_frame(const u8* src, u32 size, u32 body_off, u64 window, S
                             const u32* llInfo, const u32* mlInfo, NormT norm, NextT symbolNext, u32* ringMem, const DictState* dict = nullptr) {
   u32 pos = body_off, blk = 0;
   bool haveRepeat = false;
-  for (int k = 0; k < 3; k++) { T.cur[k] = T.space[k]; T.curStride[k] = T.stride; T.log[k] = 0; }
+  for (int k = 0; k < 3; k++) T.log[k] = 0;
   if (dict && dict->hasEntropy) {
     for (int k = 0; k < 3; k++) {
       const u32 n = 1u << dict->log[k];
@@ -323,8 +326,7 @@ ZB_HD void seq_decode_frame(const u8* src, u32 size, u32 body_off, u64 window, S
             hdr += used;
             if (m != 3) {
               T.log[kind] = lg;
-              if (isDef) { T.cur[kind] = T.defs[kind]; T.curStride[kind] = 1; }
-              else { T.cur[kind] = T.space[kind]; T.curStride[kind] = T.stride; }
+              if (isDef) seq_use_default(T, kind);
             }
           }
         }

@@ -236,6 +236,18 @@ ZB_HD u32 cell_nb(u32 low10) {
 #endif
 }
 ZB_HD u32 cell_base(u32 low10) { return (low10 & (low10 - 1)) >> 1; }
+// The same decoding with a multiplication instead of a bit scan (the sequence loop's dependent chain): the low 10 bits
+// are 2 * base + 2^nb, so the cell's lowest set bit is unit = 2^nb, and the high word of w * unit is the top nb bits of w.
+// cell_next = the next state when w holds the state bits at its top.
+ZB_HD u32 cell_unit(u32 cell) { return cell & (0u - cell); }
+ZB_HD u32 cell_next(u32 cell, u32 unit, u32 w) {
+  const u32 base = ((cell & 0x3FF) ^ unit) >> 1;
+#if defined(__CUDA_ARCH__)
+  u32 r; asm("mad.hi.u32 %0, %1, %2, %3;" : "=r"(r) : "r"(w), "r"(unit), "r"(base)); return r;
+#else
+  return base + (u32)(((u64)w * unit) >> 32);
+#endif
+}
 
 // base / extra-bit tables: ZStdInternal.cs:158-180, ZStdDecompress.cs:1081-1107
 #if defined(__CUDACC__)
