@@ -7,7 +7,7 @@ import re
 import subprocess
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-PICK = ("LDG", "STG", "LDS", "STS", "ATOMS", "ATOMG", "RED", "LDGSTS", "UBLKCP", "UTMALDG", "UTMASTG", "SHFL", "VOTE", "MATCH", "REDUX", "LDL", "STL",
+PICK = ("LD", "ST", "LDG", "STG", "LDS", "STS", "ATOMS", "ATOMG", "RED", "LDGSTS", "UBLKCP", "UTMALDG", "UTMASTG", "SHFL", "VOTE", "MATCH", "REDUX", "LDL", "STL",
         "BAR", "WARPSYNC", "NANOSLEEP", "MEMBAR")
 
 

@@ -9,6 +9,7 @@
 #include "zb_decode.cuh"
 #include "decode_kernels.cuh"
 #include "xxh_device.cuh"
+#include "zb_exec_copy.cuh"
 #ifdef ZB_EXEC_DEBUG
 #include <stdio.h>
 #endif
@@ -347,12 +348,6 @@ __device__ __forceinline__ void warp_fill(u8* dst, u8 v, u32 n, u32 lane) {
   for (u32 i = body + lane; i < n; i += 32) dst[i] = v;
 }
 
-__device__ __forceinline__ u32 warp_incl_scan(u32 v, u32 lane) {
-#pragma unroll
-  for (int d = 1; d < 32; d <<= 1) { u32 t = __shfl_up_sync(0xFFFFFFFFu, v, d); if (lane >= (u32)d) v += t; }
-  return v;
-}
-
 // =================================================================================================
 // k_exec : one warp per frame
 // =================================================================================================
@@ -374,121 +369,6 @@ __device__ __forceinline__ u32 warp_upper_bound(u32 incl, u32 x) {
   return j;   // j + s - 1 <= 30 inside the loop and j <= 31 here: no lane index ever wraps
 }
 
-// Flattened copy of many short runs in units of one 4-byte-aligned destination word: run of lane j writes len_j
-// bytes at g + dpos_j, i.e. touches units_j = ((g + dpos_j) % 4 + len_j + 3) / 4 aligned words (the first and the
-// last possibly in part); uincl/uexcl are the inclusive/exclusive warp prefix sums of units_j.  One unit per
-// lane and row, U rows in flight per pass so that the U shuffle binary searches and the U loads overlap instead
-// of serialising on their latencies.  Source of run j: src + spos_j.  The source word is assembled from the (at
-// most two) aligned words that hold a byte the unit needs — nothing outside [source, source + len_j) rounded to
-// words is touched.  (Used for literal runs; the same scheme for matches measured slower than flat_copy_m4.)
-template <int U>
-__device__ __forceinline__ void flat_copy_w(u8* g, const u8* src, u32 totalUnits, u32 uincl, u32 uexcl, u32 dpos, u32 spos, u32 len, u32 lane) {
-  for (u32 t0 = 0; t0 < totalUnits; t0 += 32 * U) {
-    u32 t[U], j[U], dj[U], ej[U], sj[U], nj[U], v[U], lo[U], hi[U];
-#pragma unroll
-    for (int k = 0; k < U; k++) { t[k] = t0 + 32 * k + lane; j[k] = 0; }
-#pragma unroll
-    for (int s = 16; s >= 1; s >>= 1) {
-#pragma unroll
-      for (int k = 0; k < U; k++) { const u32 x = __shfl_sync(FULLMASK, uincl, j[k] + s - 1); if (x <= t[k]) j[k] += s; }
-    }
-#pragma unroll
-    for (int k = 0; k < U; k++) {
-      dj[k] = __shfl_sync(FULLMASK, dpos, j[k]); ej[k] = __shfl_sync(FULLMASK, uexcl, j[k]);
-      sj[k] = __shfl_sync(FULLMASK, spos, j[k]); nj[k] = __shfl_sync(FULLMASK, len, j[k]);
-    }
-#pragma unroll
-    for (int k = 0; k < U; k++) {
-      v[k] = 0; lo[k] = 0; hi[k] = 0;
-      if (t[k] < totalUnits) {
-        u8* const d0 = g + dj[k];                                         // first byte of the run
-        const u32 word = ((u32)(uintptr_t)d0 & 3) + 0;                    // its position within its aligned word
-        const i32 rel = (i32)(4 * (t[k] - ej[k])) - (i32)word;           // run-relative position of this unit's word (-3..)
-        lo[k] = rel < 0 ? (u32)-rel : 0;                                  // bytes [lo, hi) of the word belong to the run
-        const u32 left = nj[k] - (u32)(rel + (i32)lo[k]);
-        hi[k] = lo[k] + left < 4 ? lo[k] + left : 4;
-        const u8* sp = src + sj[k] + rel;                                 // source of the word's byte 0
-        const u32* w = (const u32*)((uintptr_t)sp & ~(uintptr_t)3); const u32 sb = (u32)(uintptr_t)sp & 3;
-        const u32 a0 = (sb + lo[k] < 4) ? w[0] : 0, a1 = (sb + hi[k] > 4) ? w[1] : 0;
-        v[k] = __funnelshift_r(a0, a1, sb * 8);
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < U; k++) if (t[k] < totalUnits) {
-      u8* d = (u8*)(((uintptr_t)(g + dj[k]) & ~(uintptr_t)3) + 4 * (size_t)(t[k] - ej[k]));
-      if (hi[k] - lo[k] == 4) *(u32*)d = v[k];
-      else {
-        if (lo[k] == 0) d[0] = (u8)v[k];
-        if (lo[k] <= 1 && hi[k] > 1) d[1] = (u8)(v[k] >> 8);
-        if (lo[k] <= 2 && hi[k] > 2) d[2] = (u8)(v[k] >> 16);
-        if (hi[k] == 4) d[3] = (u8)(v[k] >> 24);
-      }
-    }
-  }
-}
-// RLE literals: the same units, filled with one byte value
-template <int U>
-__device__ __forceinline__ void flat_fill_w(u8* g, u32 fillWord, u32 totalUnits, u32 uincl, u32 uexcl, u32 dpos, u32 len, u32 lane) {
-  for (u32 t0 = 0; t0 < totalUnits; t0 += 32 * U) {
-#pragma unroll
-    for (int k = 0; k < U; k++) {
-      const u32 t = t0 + 32 * k + lane; u32 j = 0;
-#pragma unroll
-      for (int s = 16; s >= 1; s >>= 1) { const u32 x = __shfl_sync(FULLMASK, uincl, j + s - 1); if (x <= t) j += s; }
-      const u32 dj = __shfl_sync(FULLMASK, dpos, j), ej = __shfl_sync(FULLMASK, uexcl, j), nj = __shfl_sync(FULLMASK, len, j);
-      if (t < totalUnits) {
-        u8* const d0 = g + dj;
-        const i32 rel = (i32)(4 * (t - ej)) - (i32)((u32)(uintptr_t)d0 & 3);
-        const u32 lo = rel < 0 ? (u32)-rel : 0, left = nj - (u32)(rel + (i32)lo), hi = lo + left < 4 ? lo + left : 4;
-        u8* d = (u8*)(((uintptr_t)d0 & ~(uintptr_t)3) + 4 * (size_t)(t - ej));
-        if (hi - lo == 4) *(u32*)d = fillWord;
-        else for (u32 b = lo; b < hi; b++) d[b] = (u8)fillWord;
-      }
-    }
-  }
-}
-// units of a run of len bytes starting at p (0 for an empty run)
-__device__ __forceinline__ u32 word_units(const u8* p, u32 len) { return len ? (((u32)(uintptr_t)p & 3) + len + 3) >> 2 : 0; }
-
-// Flattened copy of many short non-overlapping matches in units of 4 bytes: run of lane j has len_j bytes
-// (off_j >= len_j), i.e. (len_j + 3) / 4 units; unit u moves bytes [4u, min(4u + 4, len_j)) from g + mrel_j - off_j.
-// The source word is assembled from two aligned loads (bytes past the run's end are read and dropped).
-template <int U>
-__device__ __forceinline__ void flat_copy_m4(u8* g, u32 totalUnits, u32 uincl, u32 uexcl, u32 mrel, u32 off, u32 len, u32 lane) {
-  for (u32 t0 = 0; t0 < totalUnits; t0 += 32 * U) {
-    u32 t[U], j[U], dj[U], ej[U], oj[U], nj[U], v[U];
-#pragma unroll
-    for (int k = 0; k < U; k++) { t[k] = t0 + 32 * k + lane; j[k] = 0; }
-#pragma unroll
-    for (int s = 16; s >= 1; s >>= 1) {
-#pragma unroll
-      for (int k = 0; k < U; k++) { const u32 x = __shfl_sync(FULLMASK, uincl, j[k] + s - 1); if (x <= t[k]) j[k] += s; }
-    }
-#pragma unroll
-    for (int k = 0; k < U; k++) {
-      dj[k] = __shfl_sync(FULLMASK, mrel, j[k]); ej[k] = __shfl_sync(FULLMASK, uexcl, j[k]);
-      oj[k] = __shfl_sync(FULLMASK, off, j[k]); nj[k] = __shfl_sync(FULLMASK, len, j[k]);
-    }
-#pragma unroll
-    for (int k = 0; k < U; k++) {
-      v[k] = 0;
-      if (t[k] < totalUnits) {
-        const u8* sp = g + dj[k] + 4 * (t[k] - ej[k]) - (size_t)oj[k];
-        const u32* w = (const u32*)((uintptr_t)sp & ~(uintptr_t)3); const u32 sh = ((u32)(uintptr_t)sp & 3) * 8;
-        const u32 a0 = w[0], a1 = sh ? w[1] : 0;
-        v[k] = __funnelshift_r(a0, a1, sh);
-      }
-    }
-#pragma unroll
-    for (int k = 0; k < U; k++) if (t[k] < totalUnits) {
-      const u32 b0 = 4 * (t[k] - ej[k]); const u32 cnt = nj[k] - b0;   // >= 1
-      u8* d = g + dj[k] + b0;
-      if (cnt >= 4 && (((uintptr_t)d) & 3) == 0) *(u32*)d = v[k];
-      else { d[0] = (u8)v[k]; if (cnt > 1) d[1] = (u8)(v[k] >> 8); if (cnt > 2) d[2] = (u8)(v[k] >> 16); if (cnt > 3) d[3] = (u8)(v[k] >> 24); }
-    }
-  }
-}
-
 // one match copied by the whole warp; handles every offset/length relation (byte-serial semantics of :1319-1350)
 __device__ __forceinline__ void warp_match(u8* d, u32 off, u32 len, u32 lane) {
   const u8* s = d - off;
@@ -501,31 +381,60 @@ __device__ __forceinline__ void warp_match(u8* d, u32 off, u32 len, u32 lane) {
   for (u32 i = lane; i < len; i += 32) { d[i] = s[r]; r += stepm; if (r >= off) r -= off; }
 }
 
-// 16 CTAs of 4 warps per SM (32 registers, spills to local memory included): measured faster than fewer, fatter warps —
-// the kernel lives on occupancy (6 / 8 / 10 / 12 / 16 CTAs: 3.93 / 3.44 / 3.03 / 2.95 / 2.83 ms on the bench workload).
+// The per-frame state k_exec's group loop reads rarely or never, in one shared-memory slot per warp.  At 32 registers
+// it spilled to local memory when it lived in registers, and the spill loads sat in the dependency rounds.  The slot is
+// volatile so that the compiler reloads a field where it is used instead of keeping it in a register across the loop.
+// Every lane writes the same value to a field.  The running counters (pos, litRun, recRun, blk) are advanced from their
+// own old value, so each is rewritten only after a __syncwarp that follows every lane's read of the old value; the
+// per-block fields are rewritten only in the next compressed block, after the __syncwarp that ends this one.
+struct ExecCold {
+  const u8* src; u8* dst; const u8* litScratch; const SeqRec* recs; const u8* dictEnd;
+  const u8* lit;                                           // the current block's literals
+  u32 size, cap, recCap, pos, blk, litRun, recRun, dictContent;
+  u32 hufErrBlock, hufErrCode, seqErrBlock, seqErrCode, seqErrIndex, flags;
+  u32 litSize, outBytes, litBytes;                         // of the current block
+  u8 rleByte, isRle, dry, litEntropy;
+};
+static_assert(sizeof(ExecCold) < 128, "one small slot per warp");
+
+// 16 CTAs of 4 warps per SM (32 registers): measured faster than fewer, fatter warps — the kernel lives on occupancy
+// (6 / 8 / 10 / 12 / 16 CTAs: 3.93 / 3.44 / 3.03 / 2.95 / 2.83 ms on the bench workload).
 // DICT: the context has a dictionary (its content is the window's prefix); the common kernel carries none of that code
 template <bool DICT>
 __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
+  __shared__ ExecCold coldSlots[EXEC_THREADS / 32];
+  volatile ExecCold& c = coldSlots[threadIdx.x >> 5];
   const u32 lane = threadIdx.x & 31;
   const u32 f = (blockIdx.x * EXEC_THREADS + threadIdx.x) >> 5;
   if (f >= a.n) return;
-  FrameInfo fi = a.info[f];
-  if (fi.flags & (FI_DONE | FI_PAR)) return;
-  const u8* src = a.src_base + a.src_off[f]; const u32 size = a.src_size[f];
-  u8* dst = a.dst_base + frame_dst_off(a, f, fi); const u32 cap = frame_cap(a, f, fi);
-  const u8* litScratch = lit_region(a, f, fi);
-  const SeqRec* recs = seq_region(a, f, fi); const u32 recCap = (u32)seq_capacity(cap);
-  u32 pos = fi.body_off, blk = 0, op = 0, litRun = 0, recRun = 0;   // op <= cap < 2^32 throughout: checks are written against cap - op
-  bool litEntropy = false, dry = false; u32 err = 0;
-  // the dictionary's content is the window's prefix (RefDictContent :2366-2373): dictEnd[-k] is what offset (produced + k) reaches
-  const u32 dictContent = DICT ? a.dict->contentSize : 0;
-  const u8* const dictEnd = DICT ? a.dict_bytes + a.dict->contentOff + dictContent : nullptr;
-  if (DICT && a.dict->hasEntropy) litEntropy = true;                               // :2468
+  {
+    const FrameInfo fi = a.info[f];
+    if (fi.flags & (FI_DONE | FI_PAR)) return;
+    c.src = a.src_base + a.src_off[f]; c.size = a.src_size[f];
+    c.dst = a.dst_base + frame_dst_off(a, f, fi); c.cap = frame_cap(a, f, fi);
+    c.litScratch = lit_region(a, f, fi);
+    c.recs = seq_region(a, f, fi); c.recCap = (u32)seq_capacity(frame_cap(a, f, fi));
+    c.pos = fi.body_off; c.blk = 0; c.litRun = 0; c.recRun = 0;
+    c.hufErrBlock = fi.huf_err_block; c.hufErrCode = fi.huf_err_code;
+    c.seqErrBlock = fi.seq_err_block; c.seqErrCode = fi.seq_err_code; c.seqErrIndex = fi.seq_err_index; c.flags = fi.flags;
+    // the dictionary's content is the window's prefix (RefDictContent :2366-2373): dictEnd[-k] is what offset (produced + k) reaches
+    c.dictContent = DICT ? a.dict->contentSize : 0;
+    c.dictEnd = DICT ? a.dict_bytes + a.dict->contentOff + a.dict->contentSize : nullptr;
+    c.litEntropy = DICT && a.dict->hasEntropy;                                    // :2468
+    c.dry = 0;
+  }
+  u32 op = 0, err = 0;   // op <= cap < 2^32 throughout: checks are written against cap - op
   while (true) {
     BlockHdr bh;
-    err = read_block_hdr(src + pos, size - pos, bh);
+    u32 pos = c.pos;
+    const u8* const src = c.src;
+    err = read_block_hdr(src + pos, c.size - pos, bh);
     if (err) break;
     pos += 3;
+    __syncwarp();                                                                  // every lane has read the old cursor
+    c.pos = pos + bh.csize;                                                        // the next block
+    const u32 cap = c.cap;
+    u8* const dst = c.dst;
     if (bh.type == 0) {                                                            // raw, :662-667
       if (bh.csize > cap - op) { err = ZE_dstSize_tooSmall; break; }
       warp_copy(dst + op, src + pos, bh.csize, lane); op += bh.csize;
@@ -537,40 +446,43 @@ __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
       if (bsz >= BLOCKSIZE_MAX) { err = ZE_srcSize_wrong; break; }                 // :1880
       LitHdr lh; bool needs;
       u32 e = read_lit_hdr(bp, bsz, lh, &needs);
-      if (needs && !litEntropy) { err = ZE_dictionary_corrupted; break; }          // :696-697
+      if (needs && !c.litEntropy) { err = ZE_dictionary_corrupted; break; }        // :696-697
       if (e) { err = e; break; }
-      const u8* lit; u32 rleByte = 0; bool isRle = false;
+      const u8* lit; bool isRle = false;
       if (lh.type >= 2) {
-        if (fi.huf_err_block == blk) {
-          if (fi.huf_err_code != HUF_DRY) { err = fi.huf_err_code; break; }        // :742 (all Huffman failures -> corruption_detected)
-          dry = true;                                                              // literals were not stored: checks only, the block must fail
+        if (c.hufErrBlock == c.blk) {
+          if (c.hufErrCode != HUF_DRY) { err = c.hufErrCode; break; }              // :742 (all Huffman failures -> corruption_detected)
+          c.dry = 1;                                                               // literals were not stored: checks only, the block must fail
         }
-        litEntropy = true; lit = litScratch + litRun; litRun += lh.litSize;
+        const u32 litRun = c.litRun; lit = c.litScratch + litRun;
+        __syncwarp();
+        c.litEntropy = 1; c.litRun = litRun + lh.litSize;
       } else if (lh.type == 0) lit = bp + lh.lhSize;
-      else { lit = nullptr; isRle = true; rleByte = bp[lh.lhSize]; }
-      const u32 litSize = lh.litSize;
+      else { lit = nullptr; isRle = true; c.rleByte = bp[lh.lhSize]; }
+      c.lit = lit; c.isRle = isRle; c.litSize = lh.litSize;
       const u8* sp = bp + lh.consumed; const u32 ssz = bsz - lh.consumed;
       u32 nbSeq, modes, hdr;
       e = read_seq_count(sp, ssz, &nbSeq, &modes, &hdr);
       if (e) { err = e; break; }
-      if (fi.seq_err_block == blk && fi.seq_err_index == 0xFFFFFFFFu) { err = fi.seq_err_code; break; }
+      if (c.seqErrBlock == c.blk && c.seqErrIndex == 0xFFFFFFFFu) { err = c.seqErrCode; break; }
       u32 litPos = 0;
       if (nbSeq) {
         // the block's header record: how many records follow and what they produce (zb_decode.cuh)
         u32 nRecs = 0, outBytes = 0, litBytes = 0;
-        if (recRun < recCap) { const uint4 h = __ldg(reinterpret_cast<const uint4*>(recs + recRun)); nRecs = h.x; outBytes = h.y; litBytes = h.z; }
-        const uint4* rv = reinterpret_cast<const uint4*>(recs + recRun + 1);
+        if (c.recRun < c.recCap) { const uint4 h = __ldg(reinterpret_cast<const uint4*>(c.recs + c.recRun)); nRecs = h.x; outBytes = h.y; litBytes = h.z; }
+        c.outBytes = outBytes; c.litBytes = litBytes;
         const u32 blockBase = op;
         for (u32 g0 = 0; g0 < nRecs; g0 += 32) {
+          const uint4* const rv = reinterpret_cast<const uint4*>(c.recs + c.recRun + 1);
           const bool valid = g0 + lane < nRecs;
           const uint4 rec = valid ? __ldg(rv + g0 + lane) : make_uint4(0, 0, 0, 0);
           if (lane < 2 && g0 + 32 < nRecs) prefetch_line(rv + g0 + 32 + 16 * lane);   // next group's 512 bytes
           const u32 ll = valid ? (rec.w & 0x1FFFF) : 0, ml = valid ? ((rec.w >> 17) | (((rec.y >> 18) & 7) << 15)) : 0, off = rec.z, lpos = rec.y & 0x3FFFF;
           // checks in the reference's order (:1278, :1279, :1290-1294)
           const u64 start64 = (u64)blockBase + rec.x;
-          const bool e1 = valid && start64 + ll + ml > cap;
-          const bool e2 = valid && lpos + ll > litSize;
-          const bool e3 = valid && (u64)off > start64 + ll + dictContent;           // :1290-1294 (the prefix includes the dictionary)
+          const bool e1 = valid && start64 + ll + ml > c.cap;
+          const bool e2 = valid && lpos + ll > c.litSize;
+          const bool e3 = valid && (u64)off > start64 + ll + c.dictContent;         // :1290-1294 (the prefix includes the dictionary)
           const unsigned bad = __ballot_sync(FULLMASK, e1 | e2 | e3);
           if (bad) {
             const u32 first = (u32)__ffs(bad) - 1;
@@ -583,22 +495,22 @@ __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
           op = blockBase + base; litPos = lbase;
           const u32 excl = valid ? rec.x - base : 0, mrel = excl + ll, incl = valid ? mrel + ml : 0xFFFFFFFFu;   // lanes past the end never bound a search
           const u32 lsrc = lpos - lbase;                    // literal source position of this lane, relative to litPos
-          u8* const g = dst + op;
+          u8* const g = c.dst + op;
+          __builtin_assume(__isGlobal(g));                   // read back from the slot: keep global (not generic) addressing
+          const bool dry = c.dry;
           // ---- literals: short runs flattened over the lanes, long runs by the whole warp ----
           if (!dry) {
+            const bool grpRle = c.isRle; const u32 rleByte = c.rleByte;
             const bool bigL = ll >= 128;
             unsigned bigMask = __ballot_sync(FULLMASK, bigL);
             const u32 ls = bigL ? 0 : ll;
-            const u32 lu = word_units(g + excl, ls);
-            const u32 sincl = warp_incl_scan(lu, lane), sexcl = sincl - lu;
-            const u32 Ls = __shfl_sync(FULLMASK, sincl, 31);
-            if (isRle) { if (Ls) flat_fill_w<1>(g, rleByte * 0x01010101u, Ls, sincl, sexcl, excl, ls, lane); }
-            else if (Ls > 32) flat_copy_w<2>(g, lit + litPos, Ls, sincl, sexcl, excl, lsrc, ls, lane);
-            else if (Ls) flat_copy_w<1>(g, lit + litPos, Ls, sincl, sexcl, excl, lsrc, ls, lane);
+            const u8* const lit = c.lit + litPos;
+            __builtin_assume(grpRle || __isGlobal(lit));         // RLE blocks have no literal pointer
+            flat_literals(g, lit, grpRle, rleByte, excl, lsrc, ls, lane);
             while (bigMask) {
               const u32 j = (u32)__ffs(bigMask) - 1; bigMask &= bigMask - 1;
               const u32 dj = __shfl_sync(FULLMASK, excl, j), nj = __shfl_sync(FULLMASK, ll, j), lj = __shfl_sync(FULLMASK, lsrc, j);
-              if (isRle) warp_fill(g + dj, (u8)rleByte, nj, lane); else warp_copy(g + dj, lit + litPos + lj, nj, lane);
+              if (grpRle) warp_fill(g + dj, (u8)rleByte, nj, lane); else warp_copy(g + dj, lit + lj, nj, lane);
             }
           }
           __syncwarp();
@@ -624,11 +536,7 @@ __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
               const unsigned R = __ballot_sync(FULLMASK, ready);
               const bool inDict = DICT && off > blockBase + base + mrel;          // the source begins in the dictionary (:1290-1315)
               const bool plain = ready && off >= ml && ml < 128 && !inDict;
-              const u32 len = plain ? ml : 0, units = (len + 3) >> 2;
-              const u32 pincl = warp_incl_scan(units, lane), pexcl = pincl - units;
-              const u32 Tt = __shfl_sync(FULLMASK, pincl, 31);
-              if (Tt > 32) flat_copy_m4<2>(g, Tt, pincl, pexcl, mrel, off, len, lane);
-              else if (Tt) flat_copy_m4<1>(g, Tt, pincl, pexcl, mrel, off, len, lane);
+              flat_matches(g, mrel, off, plain ? ml : 0, lane);
               unsigned big = __ballot_sync(FULLMASK, ready && !plain);
               while (big) {
                 const u32 j = (u32)__ffs(big) - 1; big &= big - 1;
@@ -637,7 +545,7 @@ __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
                 if (DICT && oj > pj) {
                   // `back` bytes come from the end of the dictionary content, the rest continues at the frame's first byte
                   const u32 back = oj - pj, l1 = back < nj ? back : nj;
-                  warp_copy(g + mj, dictEnd - back, l1, lane);
+                  warp_copy(g + mj, c.dictEnd - back, l1, lane);
                   __syncwarp();
                   if (nj > l1) warp_match(g + mj + l1, pj + l1, nj - l1, lane);
                 } else warp_match(g + mj, oj, nj, lane);
@@ -648,25 +556,31 @@ __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
           }
         }
         if (err) break;
-        recRun += 1 + nRecs;
-        if (fi.seq_err_block == blk) { err = fi.seq_err_code; break; }             // :1594 after the decodable prefix
-        op = blockBase + outBytes; litPos = litBytes;
+        const u32 recRun = c.recRun;
+        __syncwarp();
+        c.recRun = recRun + 1 + nRecs;
+        if (c.seqErrBlock == c.blk) { err = c.seqErrCode; break; }                 // :1594 after the decodable prefix
+        op = blockBase + c.outBytes; litPos = c.litBytes;
       }
       // last literals (:1599-1605)
-      const u32 lastLL = litSize - litPos;
-      if (lastLL > cap - op || dry) { err = ZE_dstSize_tooSmall; break; }
-      if (isRle) warp_fill(dst + op, (u8)rleByte, lastLL, lane); else warp_copy(dst + op, lit + litPos, lastLL, lane);
+      const u32 lastLL = c.litSize - litPos;
+      if (lastLL > c.cap - op || c.dry) { err = ZE_dstSize_tooSmall; break; }
+      if (c.isRle) warp_fill(c.dst + op, (u8)c.rleByte, lastLL, lane); else warp_copy(c.dst + op, c.lit + litPos, lastLL, lane);
       op += lastLL;
       __syncwarp();
     }
-    pos += bh.csize; blk++;
+    const u32 blk = c.blk;
+    __syncwarp();
+    c.blk = blk + 1;
     if (bh.last) break;
   }
   // ---- frame epilogue (:2069-2085) and the multi-frame loop tail (:2111-2157) ----
+  const u8* const src = c.src; const u32 size = c.size, flags = c.flags;
+  u32 pos = c.pos;
   bool needXxh = false; u32 trailer = 0;
   if (!err) {
-    if ((fi.flags & FI_FCS_KNOWN) && op != fi.fcs) err = ZE_corruption_detected;
-    else if (fi.flags & FI_CHECKSUM) {
+    if ((flags & FI_FCS_KNOWN) && op != a.info[f].fcs) err = ZE_corruption_detected;
+    else if (flags & FI_CHECKSUM) {
       if (size - pos < 4) err = ZE_checksum_wrong; else { trailer = pos; pos += 4; needXxh = true; }
     }
   }
@@ -685,10 +599,10 @@ __global__ void __launch_bounds__(EXEC_THREADS, 16) k_exec(DecodeArgs a) {
     }
   }
   if (lane == 0) {
-    u32 res = err ? zerr(err) : (tailErr ? zerr(tailErr) : fi.out_base + (u32)op);
+    u32 res = err ? zerr(err) : (tailErr ? zerr(tailErr) : a.info[f].out_base + (u32)op);
     a.result[f] = res;                                                             // provisional while next_off != 0
     a.info[f].trailer_off = trailer; a.info[f].decoded = (u32)op; a.info[f].next_off = nextOff;
-    a.info[f].flags = fi.flags | (needXxh ? FI_NEED_XXH : 0);
+    a.info[f].flags = flags | (needXxh ? FI_NEED_XXH : 0);
     if (nextOff && a.more) atomicAdd(a.more, 1u);
   }
 }
@@ -991,12 +905,7 @@ __global__ void __launch_bounds__((W + (W == 4)) * 32, W == 4 ? 7 : 32 / W) k_ex
               const bool bigL = ll >= 128;
               unsigned bigMask = __ballot_sync(FULLMASK, bigL);
               const u32 ls = bigL ? 0 : ll;
-              const u32 lu = word_units(g + excl, ls);
-              const u32 sincl = warp_incl_scan(lu, lane), sexcl = sincl - lu;
-              const u32 Ls = __shfl_sync(FULLMASK, sincl, 31);
-              if (isRle) { if (Ls) flat_fill_w<1>(g, rleByte * 0x01010101u, Ls, sincl, sexcl, excl, ls, lane); }
-              else if (Ls > 32) flat_copy_w<2>(g, lit + lbase, Ls, sincl, sexcl, excl, lsrc, ls, lane);
-              else if (Ls) flat_copy_w<1>(g, lit + lbase, Ls, sincl, sexcl, excl, lsrc, ls, lane);
+              flat_literals(g, lit + lbase, isRle, rleByte, excl, lsrc, ls, lane);
               while (bigMask) {
                 const u32 j = (u32)__ffs(bigMask) - 1; bigMask &= bigMask - 1;
                 const u32 dj = __shfl_sync(FULLMASK, excl, j), nj = __shfl_sync(FULLMASK, ll, j), lj = __shfl_sync(FULLMASK, lsrc, j);
@@ -1038,11 +947,7 @@ __global__ void __launch_bounds__((W + (W == 4)) * 32, W == 4 ? 7 : 32 / W) k_ex
                 }
                 const bool inDict = DICT && off > gstart + mrel;
                 const bool plain = ready && off >= ml && ml < 128 && !inDict;
-                const u32 len = plain ? ml : 0, units4 = (len + 3) >> 2;
-                const u32 pincl = warp_incl_scan(units4, lane), pexcl = pincl - units4;
-                const u32 Tt = __shfl_sync(FULLMASK, pincl, 31);
-                if (Tt > 32) flat_copy_m4<2>(g, Tt, pincl, pexcl, mrel, off, len, lane);
-                else if (Tt) flat_copy_m4<1>(g, Tt, pincl, pexcl, mrel, off, len, lane);
+                flat_matches(g, mrel, off, plain ? ml : 0, lane);
                 unsigned big = __ballot_sync(FULLMASK, ready && !plain);
                 while (big) {
                   const u32 j = (u32)__ffs(big) - 1; big &= big - 1;
